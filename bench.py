@@ -15,6 +15,10 @@ used for the barriers and the max-over-ranks timing only ("scaling": "weak").
 
 `--impl reference` times the CPU restatement of the reference algorithm (oracle/, kind "port": the
 reference itself is Python + SciPy ARPACK and cannot travel to the GPU box) on a bounded sample.
+
+`--dump-outputs DIR` writes what the last timed step returned to its caller as DIR/<name>.npy: the eigenvalues (fp64),
+get_vals() (fp32) and the gradient to the quadratic vertex positions (fp32).  The input mesh is generated, not random, so
+two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -169,6 +173,38 @@ def dist_env():
     return rank, world, local
 
 
+DUMP_LIMIT = 64 * 10 ** 6       # bytes --dump-outputs writes in all
+
+
+def step_outputs(obj, vals, grad):
+    """What one step of the timed path hands its caller, copied to the host."""
+    return {"eigenvalues": obj.eigenvalues.detach().cpu().numpy(), "vals": vals.detach().cpu().numpy(),
+            "vertex_grad": grad.detach().cpu().numpy()}
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT):
+    """Writes every array as out_dir/<name>.npy.  Arrays of at most limit / 64 bytes are written whole.  If the larger ones do
+    not fit in the rest of the limit, each is cut to a fixed, seeded sample of its rows (the same rows for the same row count),
+    whose ids go to out_dir/<name>_rows.npy as float64."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    header = 256                                    # bytes of .npy header allowed per file
+    small = {k for k, a in arrays.items() if a.nbytes <= limit // 64}
+    large = [a for k, a in arrays.items() if k not in small]
+    room = limit - sum(arrays[k].nbytes + header for k in small) - 2 * header * len(large)
+    keep = 1.0
+    if sum(a.nbytes for a in large) > room:
+        keep = room / sum(a.nbytes + 8 * a.shape[0] for a in large)
+    for name, a in arrays.items():
+        if a.dtype not in (np.float32, np.float64):
+            raise TypeError(f"--dump-outputs: {name} is {a.dtype}, not float32 / float64")
+        if name not in small and keep < 1.0:
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], int(a.shape[0] * keep), replace=False))
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+
+
 # ----------------------------------------------------------------------------------------------
 # CPU arm: the oracle's restatement of the reference algorithm on the host cores
 # ----------------------------------------------------------------------------------------------
@@ -307,7 +343,7 @@ def run_rowpart(args):
         obj._warm = []
         obj._Kval = obj._Mblk = None
         stats, state["solver"] = eigen_decomposition_rowpart(obj, solver=state["solver"], keep=True)
-        vals = obj.get_vals()
+        vals = state["vals"] = obj.get_vals()
         leaf.grad = None
         (vals[:, 0] * (1.0 / obj.eigenvalues).float()).sum().backward()
         return stats
@@ -342,6 +378,7 @@ def run_rowpart(args):
     barrier()
     launches = int(lib.ds_launch_count() - launches0)
     sampler.stop_flag = True
+    outputs = step_outputs(obj, state["vals"], leaf.grad) if args.dump_outputs and rank == 0 else None
     each_ms = [a.elapsed_time(b) for a, b in zip([e0] + marks[:-1], marks)]
     tms = torch.tensor([e0.elapsed_time(e1)], device=dev, dtype=torch.float64)
     if world > 1:
@@ -384,6 +421,8 @@ def run_rowpart(args):
             "gpu_launches": launches, "clocks": sampler.summary(),
             "kernel_ms_per_step_rank0": {k: v["ms"] / 2 for k, v in prof_all.items()},
             "phase_wall_ms_rank0_synchronised": phases}
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     if rank == 0:
         print(json.dumps(line), flush=True)
     state["solver"].close()
@@ -404,7 +443,13 @@ def main():
     ap.add_argument("--mode", default="sweep", choices=["sweep", "rowpart"],
                     help="sweep: one independent mesh per GPU (weak scaling, the default and the driver's line); rowpart: ONE "
                          "mesh, eigen-solve row-partitioned over the GPUs (strong scaling)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs the native arm (the reference arm keeps no outputs)")
     if args.impl == "reference":
         run_reference_arm(args)
         return
@@ -497,6 +542,7 @@ def main():
     prof = pf.read()
     launches = int(lib.ds_launch_count() - launches0)
     sampler.stop_flag = True
+    outputs = step_outputs(obj, vals, grad) if args.dump_outputs and rank == 0 else None
     ms = e0.elapsed_time(e1)
     each_ms = [a.elapsed_time(b) for a, b in zip([e0] + marks[:-1], marks)]
     with native.prof() as pf_all:
@@ -514,7 +560,7 @@ def main():
 
     # ---- end to end through the public API from host buffers (a new model per step, as the sweeps build one
     # per candidate); one untimed pass first so that the caching allocator owns the blocks a second model needs
-    e2e_steps = max(2, args.steps)          # as many end-to-end steps as device-timed steps
+    e2e_steps = args.steps                  # as many end-to-end steps as device-timed steps
 
     def e2e_step():
         lf, ob = build(v_host, t_host)
@@ -653,6 +699,8 @@ def main():
             "fp64_peak_tflops": fp64_peak}
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         line["cpu_baseline"], _ = cpu_baseline(args.cpu_cube, steps=1, warmup=0, budget_s=120.0)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     if rank == 0:
         print(json.dumps(line), flush=True)
     if world > 1:

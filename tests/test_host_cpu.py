@@ -172,3 +172,31 @@ def test_bench_clock_sampler_summary():
     assert s.summary()["reasons"] == ["hw_slowdown", "sw_thermal_slowdown"] + ["sw_power_cap"]
     s.samples = []
     assert s.summary()["sm_mhz"] is None and s.summary()["reasons"] == []
+
+
+def test_bench_dump_outputs_bounded_and_seeded(tmp_path):
+    """bench.py --dump-outputs: arrays are written whole while they fit; above the limit the large ones are cut to the same
+    seeded row sample in every run, with the row ids beside them, and the files stay within the limit."""
+    import bench
+    rng = np.random.default_rng(1)
+    arrays = {"eigenvalues": rng.standard_normal(32), "vertex_grad": rng.standard_normal((5000, 3)).astype(np.float32)}
+    bench.dump_outputs(str(tmp_path / "whole"), arrays)
+    assert sorted(os.listdir(tmp_path / "whole")) == ["eigenvalues.npy", "vertex_grad.npy"]
+    for name, a in arrays.items():
+        b = np.load(tmp_path / "whole" / (name + ".npy"))
+        assert b.dtype == a.dtype and np.array_equal(a, b)
+    limit = 40000
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays, limit=limit)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["eigenvalues.npy", "vertex_grad.npy", "vertex_grad_rows.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= limit
+    for f in files:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b)
+    rows = np.load(tmp_path / "a" / "vertex_grad_rows.npy").astype(np.int64)
+    assert 1000 < rows.size < 5000 and np.all(np.diff(rows) > 0)
+    assert np.array_equal(np.load(tmp_path / "a" / "vertex_grad.npy"), arrays["vertex_grad"][rows])
+    assert np.array_equal(np.load(tmp_path / "a" / "eigenvalues.npy"), arrays["eigenvalues"])
+    with pytest.raises(TypeError):
+        bench.dump_outputs(str(tmp_path / "c"), {"tets": np.zeros((4, 4), dtype=np.int64)})
