@@ -50,6 +50,22 @@ int widen_f32(const float* src, int width, int64_t n, double* dst, int64_t ldd, 
 int colnorm2_f32(const float* V, int w, int64_t n, double* partial, int ctas, cudaStream_t st);
 int fill_random_f32(float* V, int64_t count, uint64_t seed, cudaStream_t st);
 
+// Morton codes of points (also used by the triangle-mesh BVH of sdf.cu).  ordered_key maps a float to a uint32 whose
+// unsigned order is the float order (atomicMin / atomicMax on keys give float bounds); key_to_float inverts it.
+__device__ __forceinline__ uint32_t ordered_key(float f) {
+    const uint32_t u = __float_as_uint(f + 0.0f);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float key_to_float(uint32_t k) {
+    return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
+}
+// mm[0..2] = min key per axis, mm[3..5] = max key per axis of coords [n x 3] (mm initialised to 0xffffffff / 0 by the
+// caller; any grid, grid-stride loop)
+__global__ void k_bbox(const float* __restrict__ coords, int64_t n, uint32_t* __restrict__ mm);
+// codes[i] = 30-bit Morton code of point i inside the box mm, iota[i] = i
+__global__ void k_morton_codes(const float* __restrict__ coords, int64_t n, const uint32_t* __restrict__ mm,
+                               uint32_t* __restrict__ codes, uint32_t* __restrict__ iota);
+
 // one level of the FP32 preconditioner: records + block-Jacobi inverse + spectral bound of invD A
 struct Level32 {
     const int32_t* brow = nullptr;           // row pointers in the level's own numbering

@@ -606,13 +606,6 @@ k_pack_k32(const int32_t* __restrict__ brow, const int32_t* __restrict__ bcol, i
 }
 
 // ---- Morton renumbering of the operator's rows (locality of the gathered X rows) ------------------
-__device__ __forceinline__ uint32_t ordered_key(float f) {
-    const uint32_t u = __float_as_uint(f + 0.0f);
-    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-__device__ __forceinline__ float key_to_float(uint32_t k) {
-    return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
-}
 // mm[0..2] = min key per axis, mm[3..5] = max key per axis (initialised to 0xffffffff / 0 by the caller)
 __global__ void k_bbox(const float* __restrict__ coords, int64_t n, uint32_t* __restrict__ mm) {
     uint32_t lo[3] = {0xffffffffu, 0xffffffffu, 0xffffffffu}, hi[3] = {0u, 0u, 0u};

@@ -1,0 +1,555 @@
+// Signed distance from query points to a triangle mesh: the open3d RaycastingScene sampling of apply_sdf(path) in the
+// reference (src/dmtet/geometry/dmtet_thickness.py:301-314; SURVEY.md section 8f-4).
+//
+// Contract (include/diffsound_sm100.h, ds_mesh_sdf):
+//   * |sdf(p)| = Euclidean distance from p to the closest point of the triangle set: closest point on each triangle by the
+//     vertex / edge / face region analysis (Ericson, Real-Time Collision Detection 5.1.5), evaluated in fp64 from the fp32
+//     inputs, rounded once to fp32.  Degenerate faces (zero cross product) are the union of their three edges.
+//   * sign: positive inside, negative outside, by the parity of ray crossings (face orientation does not matter), majority
+//     of three fixed rays that are not axis-aligned.  Ray / triangle: the watertight test of Woop, Benthin & Wald
+//     (JCGT 2(1), 2013) in fp32 with a per-edge fp64 recomputation when an edge function is exactly 0; a crossing through
+//     an edge or a vertex is assigned to exactly one triangle of a closed mesh by a top-left rule on the projected edge
+//     direction, taken in the triangle's counter-clockwise order so that the choice does not depend on face orientation.
+//     Degenerate faces and faces seen edge-on never count.  A point at distance 0 gives +0.
+//
+// BVH mode: Morton codes of the triangle centroids (k_bbox / k_morton_codes of precond32.cu), CUB radix sort, binary
+// radix tree (Karras, HPG 2012; equal codes ordered by index), boxes refit bottom-up with per-node arrival counters.
+// Each internal node stores the boxes of its two children.  Node boxes are padded by 2^-16 of the largest coordinate
+// magnitude of mesh and queries: that margin exceeds the fp32 rounding of the ray test's sheared coordinates and the fp64
+// rounding of the distances, so a box is never pruned while it holds a triangle the brute-force loop would count
+// (nearest: pruned only when its squared box distance is strictly greater than the best; rays: conservative slab test
+// of Ize 2013, t_max scaled by 1 + 2 gamma_3).  The minimum and the crossing counts then do not depend on the hierarchy
+// or on the visit order, and BVH and brute-force outputs are bitwise equal.  Queries run in Morton order of the points.
+// Per-triangle arithmetic uses explicit round-to-nearest intrinsics (no contraction into FMA), so both kernels evaluate
+// bit-identical per-triangle values.
+#include "common.cuh"
+#include "../../include/diffsound_sm100.h"
+#include "kernels.cuh"
+#include <cub/cub.cuh>
+#include <cfloat>
+#include <climits>
+
+namespace ds {
+
+namespace {
+
+constexpr int SDF_BLOCK = 64;      // query threads per CTA (the traversal stacks live in shared memory)
+constexpr int SDF_STACK = 64;      // > depth of a radix tree over 30-bit codes + 32-bit indices
+constexpr int SDF_TILE = 256;      // triangles per shared-memory tile of the brute-force kernel
+
+// three fixed ray directions, none axis-aligned, no two components equal in magnitude
+__constant__ float c_ray_dir[3][3] = {{0.3090f, 0.5878f, 0.7470f}, {-0.8024f, 0.2590f, 0.5375f}, {0.4531f, -0.8127f, -0.3664f}};
+
+// internal node: b[0..5] = lo xyz, hi xyz of child 0, b[6..11] of child 1; child >= 0 internal node, < 0 leaf ~index
+struct __align__(16) BvhNode {
+    float b[12];
+    int child[2];
+    int pad[2];
+};
+
+__device__ __forceinline__ double dsub(double a, double b) { return __dsub_rn(a, b); }
+__device__ __forceinline__ double dadd(double a, double b) { return __dadd_rn(a, b); }
+__device__ __forceinline__ double dmul(double a, double b) { return __dmul_rn(a, b); }
+
+struct D3 {
+    double x, y, z;
+};
+__device__ __forceinline__ D3 d3(float4 v) { return {(double)v.x, (double)v.y, (double)v.z}; }
+__device__ __forceinline__ D3 sub3(D3 a, D3 b) { return {dsub(a.x, b.x), dsub(a.y, b.y), dsub(a.z, b.z)}; }
+__device__ __forceinline__ double dot3(D3 a, D3 b) { return dadd(dadd(dmul(a.x, b.x), dmul(a.y, b.y)), dmul(a.z, b.z)); }
+__device__ __forceinline__ D3 axpy3(D3 a, double t, D3 d) { return {dadd(a.x, dmul(t, d.x)), dadd(a.y, dmul(t, d.y)), dadd(a.z, dmul(t, d.z))}; }
+__device__ __forceinline__ double dist2(D3 p, D3 q) { const D3 d = sub3(p, q); return dot3(d, d); }
+
+// squared distance from p to the segment [a, b] (a point when a == b)
+__device__ __forceinline__ double seg_d2(D3 p, D3 a, D3 b) {
+    const D3 ab = sub3(b, a);
+    const double l2 = dot3(ab, ab);
+    double t = l2 > 0.0 ? dot3(sub3(p, a), ab) / l2 : 0.0;
+    t = fmin(fmax(t, 0.0), 1.0);
+    return dist2(p, axpy3(a, t, ab));
+}
+
+// squared distance from p to triangle (A, B, C); A.w != 0 marks a degenerate face (its three edges)
+__device__ __forceinline__ double tri_d2(D3 p, float4 A4, float4 B4, float4 C4) {
+    const D3 a = d3(A4), b = d3(B4), c = d3(C4);
+    if (A4.w != 0.f) return fmin(fmin(seg_d2(p, a, b), seg_d2(p, b, c)), seg_d2(p, c, a));
+    const D3 ab = sub3(b, a), ac = sub3(c, a), ap = sub3(p, a);
+    const double d1 = dot3(ab, ap), d2 = dot3(ac, ap);
+    if (d1 <= 0.0 && d2 <= 0.0) return dist2(p, a);
+    const D3 bp = sub3(p, b);
+    const double d3_ = dot3(ab, bp), d4 = dot3(ac, bp);
+    if (d3_ >= 0.0 && d4 <= d3_) return dist2(p, b);
+    const double vc = dsub(dmul(d1, d4), dmul(d3_, d2));
+    if (vc <= 0.0 && d1 >= 0.0 && d3_ <= 0.0) return dist2(p, axpy3(a, d1 / dsub(d1, d3_), ab));
+    const D3 cp = sub3(p, c);
+    const double d5 = dot3(ab, cp), d6 = dot3(ac, cp);
+    if (d6 >= 0.0 && d5 <= d6) return dist2(p, c);
+    const double vb = dsub(dmul(d5, d2), dmul(d1, d6));
+    if (vb <= 0.0 && d2 >= 0.0 && d6 <= 0.0) return dist2(p, axpy3(a, d2 / dsub(d2, d6), ac));
+    const double va = dsub(dmul(d3_, d6), dmul(d5, d4));
+    const double e43 = dsub(d4, d3_), e56 = dsub(d5, d6);
+    if (va <= 0.0 && e43 >= 0.0 && e56 >= 0.0) return dist2(p, axpy3(b, e43 / dadd(e43, e56), sub3(c, b)));
+    const double den = dadd(dadd(va, vb), vc);
+    if (!(den > 0.0)) return fmin(fmin(seg_d2(p, a, b), seg_d2(p, b, c)), seg_d2(p, c, a));   // cancellation on a sliver
+    const double v = vb / den, w = vc / den;
+    return dist2(p, axpy3(axpy3(a, v, ab), w, ac));
+}
+
+// ray from o along c_ray_dir[r], in the sheared frame of Woop et al.: kz = dominant axis, S = shear
+struct Ray {
+    float o[3];
+    float Sx, Sy, Sz;
+    float inv[3];
+    int kx, ky, kz;
+};
+__device__ __forceinline__ float sel3(float4 v, int k) { return k == 0 ? v.x : (k == 1 ? v.y : v.z); }
+__device__ __forceinline__ float sel3(const float* v, int k) { return k == 0 ? v[0] : (k == 1 ? v[1] : v[2]); }
+
+__device__ __forceinline__ Ray make_ray(float px, float py, float pz, int r) {
+    Ray R;
+    R.o[0] = px; R.o[1] = py; R.o[2] = pz;
+    const float dx = c_ray_dir[r][0], dy = c_ray_dir[r][1], dz = c_ray_dir[r][2];
+    const float ax = fabsf(dx), ay = fabsf(dy), az = fabsf(dz);
+    R.kz = (ax >= ay && ax >= az) ? 0 : (ay >= az ? 1 : 2);
+    R.kx = R.kz == 2 ? 0 : R.kz + 1;
+    R.ky = R.kx == 2 ? 0 : R.kx + 1;
+    const float d[3] = {dx, dy, dz};
+    const float dkz = sel3(d, R.kz);
+    R.Sx = sel3(d, R.kx) / dkz;
+    R.Sy = sel3(d, R.ky) / dkz;
+    R.Sz = 1.0f / dkz;
+    R.inv[0] = 1.0f / dx; R.inv[1] = 1.0f / dy; R.inv[2] = 1.0f / dz;
+    return R;
+}
+
+struct P2 {
+    float x, y, z;
+};
+__device__ __forceinline__ P2 shear(const Ray& R, float4 V) {
+    const float vx = __fsub_rn(sel3(V, R.kx), sel3(R.o, R.kx));
+    const float vy = __fsub_rn(sel3(V, R.ky), sel3(R.o, R.ky));
+    const float vz = __fsub_rn(sel3(V, R.kz), sel3(R.o, R.kz));
+    return {__fsub_rn(vx, __fmul_rn(R.Sx, vz)), __fsub_rn(vy, __fmul_rn(R.Sy, vz)), __fmul_rn(R.Sz, vz)};
+}
+// 2-D edge function of the directed edge P -> Q at the origin (twice the signed area of O, P, Q); fp64 when the fp32
+// value is exactly 0.  A shared edge gets exactly negated values in its two triangles.
+__device__ __forceinline__ double edge_fn(P2 P, P2 Q) {
+    const float e = __fsub_rn(__fmul_rn(P.x, Q.y), __fmul_rn(P.y, Q.x));
+    if (e != 0.0f) return (double)e;
+    return dsub(dmul((double)P.x, (double)Q.y), dmul((double)P.y, (double)Q.x));
+}
+// a zero edge function counts as inside only for edges whose counter-clockwise direction is "top-left"
+__device__ __forceinline__ bool top_left(P2 P, P2 Q, bool ccw) {
+    const float dx = ccw ? __fsub_rn(Q.x, P.x) : __fsub_rn(P.x, Q.x);
+    const float dy = ccw ? __fsub_rn(Q.y, P.y) : __fsub_rn(P.y, Q.y);
+    return dy > 0.0f || (dy == 0.0f && dx < 0.0f);
+}
+
+// 1 when the ray crosses triangle (A, B, C) at t > 0
+__device__ __forceinline__ int ray_hit(const Ray& R, float4 A4, float4 B4, float4 C4) {
+    if (A4.w != 0.f) return 0;
+    const P2 A = shear(R, A4), B = shear(R, B4), C = shear(R, C4);
+    const double e0 = edge_fn(B, C), e1 = edge_fn(C, A), e2 = edge_fn(A, B);
+    if ((e0 < 0.0 || e1 < 0.0 || e2 < 0.0) && (e0 > 0.0 || e1 > 0.0 || e2 > 0.0)) return 0;
+    const double det = dadd(dadd(e0, e1), e2);
+    if (det == 0.0) return 0;
+    const bool ccw = det > 0.0;
+    if (e0 == 0.0 && !top_left(B, C, ccw)) return 0;
+    if (e1 == 0.0 && !top_left(C, A, ccw)) return 0;
+    if (e2 == 0.0 && !top_left(A, B, ccw)) return 0;
+    const double T = dadd(dadd(dmul(e0, (double)A.z), dmul(e1, (double)B.z)), dmul(e2, (double)C.z));
+    return (ccw ? T > 0.0 : T < 0.0) ? 1 : 0;
+}
+
+__device__ __forceinline__ double box_d2(double px, double py, double pz, const float* lo, const float* hi) {
+    const double dx = fmax(fmax((double)lo[0] - px, px - (double)hi[0]), 0.0);
+    const double dy = fmax(fmax((double)lo[1] - py, py - (double)hi[1]), 0.0);
+    const double dz = fmax(fmax((double)lo[2] - pz, pz - (double)hi[2]), 0.0);
+    return dx * dx + dy * dy + dz * dz;
+}
+__device__ __forceinline__ bool ray_box(const Ray& R, const float* lo, const float* hi) {
+    constexpr float gamma3 = 3.0f * FLT_EPSILON * 0.5f / (1.0f - 3.0f * FLT_EPSILON * 0.5f);
+    float tn = -FLT_MAX, tf = FLT_MAX;
+#pragma unroll
+    for (int d = 0; d < 3; ++d) {
+        const float t0 = (lo[d] - R.o[d]) * R.inv[d], t1 = (hi[d] - R.o[d]) * R.inv[d];
+        tn = fmaxf(tn, fminf(t0, t1));
+        tf = fminf(tf, fmaxf(t0, t1));
+    }
+    tf *= 1.0f + 2.0f * gamma3;
+    return tn <= tf && tf >= 0.0f;
+}
+
+__device__ __forceinline__ void load_node(const BvhNode* nodes, int n, float (&b)[12], int& c0, int& c1) {
+    const float4* q = reinterpret_cast<const float4*>(nodes + n);
+    const float4 v0 = __ldg(q), v1 = __ldg(q + 1), v2 = __ldg(q + 2);
+    const int4 v3 = __ldg(reinterpret_cast<const int4*>(q + 3));
+    b[0] = v0.x; b[1] = v0.y; b[2] = v0.z; b[3] = v0.w; b[4] = v1.x; b[5] = v1.y;
+    b[6] = v1.z; b[7] = v1.w; b[8] = v2.x; b[9] = v2.y; b[10] = v2.z; b[11] = v2.w;
+    c0 = v3.x;
+    c1 = v3.y;
+}
+
+// ---- validation ------------------------------------------------------------------------------------------------
+// bad[0] = first face with an index outside [0, V), bad[1] = first non-finite vertex, bad[2] = first non-finite point
+__global__ void k_sdf_validate(const float* __restrict__ verts, int64_t V, const int64_t* __restrict__ faces, int64_t F,
+                               const float* __restrict__ pts, int64_t P, unsigned long long* __restrict__ bad) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < 3 * F; i += stride) {
+        const int64_t v = faces[i];
+        if (v < 0 || v >= V) atomicMin(&bad[0], (unsigned long long)(i / 3));
+    }
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < 3 * V; i += stride)
+        if (!isfinite(verts[i])) atomicMin(&bad[1], (unsigned long long)(i / 3));
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < 3 * P; i += stride)
+        if (!isfinite(pts[i])) atomicMin(&bad[2], (unsigned long long)(i / 3));
+}
+
+// ---- build -----------------------------------------------------------------------------------------------------
+__global__ void k_sdf_centroids(const float* __restrict__ verts, const int64_t* __restrict__ faces, int64_t F,
+                                float* __restrict__ cent) {
+    const int64_t f = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (f >= F) return;
+    const int64_t a = faces[3 * f], b = faces[3 * f + 1], c = faces[3 * f + 2];
+#pragma unroll
+    for (int d = 0; d < 3; ++d) cent[3 * f + d] = (verts[3 * a + d] + verts[3 * b + d] + verts[3 * c + d]) * (1.0f / 3.0f);
+}
+
+// tri[3 i .. 3 i + 2] = corners of face order[i] (identity when order is NULL), sorted; A.w = 1 for a zero cross product
+__global__ void k_sdf_gather(const float* __restrict__ verts, const int64_t* __restrict__ faces,
+                             const uint32_t* __restrict__ order, int64_t F, float4* __restrict__ tri) {
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i >= F) return;
+    const int64_t f = order ? (int64_t)order[i] : i;
+    float4 v[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        const int64_t id = faces[3 * f + k];
+        v[k] = make_float4(verts[3 * id], verts[3 * id + 1], verts[3 * id + 2], 0.f);
+    }
+    // corners in lexicographic order: the per-triangle arithmetic then does not depend on how the face was written
+    // (orientation, first corner), so flipped or re-indexed meshes give bitwise equal results
+    auto cswap = [](float4& a, float4& b) {
+        const bool less = b.x < a.x || (b.x == a.x && (b.y < a.y || (b.y == a.y && b.z < a.z)));
+        if (less) { const float4 t = a; a = b; b = t; }
+    };
+    cswap(v[0], v[1]);
+    cswap(v[1], v[2]);
+    cswap(v[0], v[1]);
+    const D3 a = d3(v[0]), ab = sub3(d3(v[1]), a), ac = sub3(d3(v[2]), a);
+    const double nx = dsub(dmul(ab.y, ac.z), dmul(ab.z, ac.y));
+    const double ny = dsub(dmul(ab.z, ac.x), dmul(ab.x, ac.z));
+    const double nz = dsub(dmul(ab.x, ac.y), dmul(ab.y, ac.x));
+    v[0].w = (nx == 0.0 && ny == 0.0 && nz == 0.0) ? 1.f : 0.f;
+    tri[3 * i] = v[0];
+    tri[3 * i + 1] = v[1];
+    tri[3 * i + 2] = v[2];
+}
+
+__device__ __forceinline__ int delta(const uint32_t* __restrict__ codes, int n, int i, int j) {
+    if (j < 0 || j >= n) return -1;
+    const uint32_t a = codes[i], b = codes[j];
+    return a != b ? __clz(a ^ b) : 32 + __clz((uint32_t)(i ^ j));
+}
+
+// internal node i of the radix tree over n sorted codes (Karras 2012, algorithm 2); parent[] over node ids
+// (internal j -> j, leaf k -> n - 1 + k), parent[0] = -1
+__global__ void k_sdf_karras(const uint32_t* __restrict__ codes, int n, BvhNode* __restrict__ nodes, int* __restrict__ parent) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n - 1) return;
+    const int d = delta(codes, n, i, i + 1) - delta(codes, n, i, i - 1) >= 0 ? 1 : -1;
+    const int dmin = delta(codes, n, i, i - d);
+    int lmax = 2;
+    while (delta(codes, n, i, i + lmax * d) > dmin) lmax *= 2;
+    int l = 0;
+    for (int t = lmax / 2; t >= 1; t /= 2)
+        if (delta(codes, n, i, i + (l + t) * d) > dmin) l += t;
+    const int j = i + l * d;
+    const int dnode = delta(codes, n, i, j);
+    int s = 0, t = l;
+    do {
+        t = (t + 1) >> 1;
+        if (delta(codes, n, i, i + (s + t) * d) > dnode) s += t;
+    } while (t > 1);
+    const int gamma = i + s * d + min(d, 0);
+    const int left = min(i, j) == gamma ? ~gamma : gamma;
+    const int right = max(i, j) == gamma + 1 ? ~(gamma + 1) : gamma + 1;
+    nodes[i].child[0] = left;
+    nodes[i].child[1] = right;
+    parent[left < 0 ? n - 1 + ~left : left] = i;
+    parent[right < 0 ? n - 1 + ~right : right] = i;
+    if (i == 0) parent[0] = -1;
+}
+
+// bottom-up box refit: one thread per leaf; the second thread to reach a node continues with the union of its children
+__global__ void k_sdf_refit(const float4* __restrict__ tri, int n, BvhNode* nodes, const int* __restrict__ parent,
+                            int* __restrict__ arrived, const uint32_t* __restrict__ mm_v, const uint32_t* __restrict__ mm_p) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    float S = FLT_MIN;
+#pragma unroll
+    for (int d = 0; d < 6; ++d) S = fmaxf(S, fmaxf(fabsf(key_to_float(mm_v[d])), fabsf(key_to_float(mm_p[d]))));
+    const float pad = S * (1.0f / 65536.0f);
+    const float4 A = tri[3 * k], B = tri[3 * k + 1], C = tri[3 * k + 2];
+    float lo[3] = {fminf(fminf(A.x, B.x), C.x), fminf(fminf(A.y, B.y), C.y), fminf(fminf(A.z, B.z), C.z)};
+    float hi[3] = {fmaxf(fmaxf(A.x, B.x), C.x), fmaxf(fmaxf(A.y, B.y), C.y), fmaxf(fmaxf(A.z, B.z), C.z)};
+#pragma unroll
+    for (int d = 0; d < 3; ++d) {
+        lo[d] = __fsub_rd(lo[d], pad);
+        hi[d] = __fadd_ru(hi[d], pad);
+    }
+    int enc = ~k;
+    int p = parent[n - 1 + k];
+    while (p >= 0) {
+        const int slot = nodes[p].child[0] == enc ? 0 : 1;
+        volatile float* b = nodes[p].b;
+#pragma unroll
+        for (int d = 0; d < 3; ++d) {
+            b[6 * slot + d] = lo[d];
+            b[6 * slot + 3 + d] = hi[d];
+        }
+        __threadfence();
+        if (atomicAdd(&arrived[p], 1) == 0) return;
+        __threadfence();
+#pragma unroll
+        for (int d = 0; d < 3; ++d) {
+            lo[d] = fminf(b[d], b[6 + d]);
+            hi[d] = fmaxf(b[3 + d], b[9 + d]);
+        }
+        enc = p;
+        p = parent[p];
+    }
+}
+
+// ---- queries ---------------------------------------------------------------------------------------------------
+__device__ __forceinline__ float signed_out(double best, int votes) {
+    const float d = (float)sqrt(best);
+    return d == 0.0f ? 0.0f : (votes >= 2 ? d : -d);
+}
+
+__global__ void __launch_bounds__(SDF_BLOCK)
+k_sdf_query_bvh(const float4* __restrict__ tri, const BvhNode* __restrict__ nodes, int F, const float* __restrict__ pts,
+                const uint32_t* __restrict__ order, int64_t P, float* __restrict__ out) {
+    __shared__ int s_node[SDF_STACK][SDF_BLOCK];
+    __shared__ float s_d2[SDF_STACK][SDF_BLOCK];
+    const int64_t i = blockIdx.x * (int64_t)SDF_BLOCK + threadIdx.x;
+    if (i >= P) return;
+    const int tid = threadIdx.x;
+    const int64_t q = order[i];
+    const float px = pts[3 * q], py = pts[3 * q + 1], pz = pts[3 * q + 2];
+    const D3 p = {(double)px, (double)py, (double)pz};
+    float b[12];
+    int c[2];
+    // nearest triangle
+    double best = INFINITY;
+    if (F == 1) {
+        best = tri_d2(p, tri[0], tri[1], tri[2]);
+    } else {
+        int sp = 0, node = 0;
+        for (;;) {
+            load_node(nodes, node, b, c[0], c[1]);
+            double bd[2] = {box_d2(p.x, p.y, p.z, b, b + 3), box_d2(p.x, p.y, p.z, b + 6, b + 9)};
+            bool go[2] = {bd[0] <= best, bd[1] <= best};
+#pragma unroll
+            for (int s = 0; s < 2; ++s)
+                if (go[s] && c[s] < 0) {
+                    const int t = ~c[s];
+                    best = fmin(best, tri_d2(p, tri[3 * t], tri[3 * t + 1], tri[3 * t + 2]));
+                    go[s] = false;
+                }
+            if (go[0] && go[1]) {
+                const bool r_first = bd[1] < bd[0];      // nearer child first, the other one on the stack
+                s_node[sp][tid] = r_first ? c[0] : c[1];
+                s_d2[sp][tid] = __double2float_rd(r_first ? bd[0] : bd[1]);
+                ++sp;
+                node = r_first ? c[1] : c[0];
+                continue;
+            }
+            if (go[0] || go[1]) {
+                node = go[0] ? c[0] : c[1];
+                continue;
+            }
+            node = -1;
+            while (sp > 0) {
+                --sp;
+                if ((double)s_d2[sp][tid] <= best) {
+                    node = s_node[sp][tid];
+                    break;
+                }
+            }
+            if (node < 0) break;
+        }
+    }
+    // crossing parity of the three rays
+    int votes = 0;
+#pragma unroll 1
+    for (int r = 0; r < 3; ++r) {
+        const Ray R = make_ray(px, py, pz, r);
+        int cnt = 0;
+        if (F == 1) {
+            cnt = ray_hit(R, tri[0], tri[1], tri[2]);
+        } else {
+            int sp = 0, node = 0;
+            for (;;) {
+                load_node(nodes, node, b, c[0], c[1]);
+                bool go[2] = {ray_box(R, b, b + 3), ray_box(R, b + 6, b + 9)};
+#pragma unroll
+                for (int s = 0; s < 2; ++s)
+                    if (go[s] && c[s] < 0) {
+                        const int t = ~c[s];
+                        cnt += ray_hit(R, tri[3 * t], tri[3 * t + 1], tri[3 * t + 2]);
+                        go[s] = false;
+                    }
+                if (go[0] && go[1]) {
+                    s_node[sp++][tid] = c[1];
+                    node = c[0];
+                } else if (go[0] || go[1]) {
+                    node = go[0] ? c[0] : c[1];
+                } else if (sp > 0) {
+                    node = s_node[--sp][tid];
+                } else {
+                    break;
+                }
+            }
+        }
+        votes += cnt & 1;
+    }
+    out[q] = signed_out(best, votes);
+}
+
+// every point against every triangle (shared-memory tiles of SDF_TILE triangles): the reference for the BVH path
+__global__ void __launch_bounds__(SDF_BLOCK)
+k_sdf_query_brute(const float4* __restrict__ tri, int F, const float* __restrict__ pts, int64_t P, float* __restrict__ out) {
+    __shared__ float4 s_tri[3 * SDF_TILE];
+    const int64_t i = blockIdx.x * (int64_t)SDF_BLOCK + threadIdx.x;
+    const bool valid = i < P;
+    const float px = valid ? pts[3 * i] : 0.f, py = valid ? pts[3 * i + 1] : 0.f, pz = valid ? pts[3 * i + 2] : 0.f;
+    const D3 p = {(double)px, (double)py, (double)pz};
+    const Ray R0 = make_ray(px, py, pz, 0), R1 = make_ray(px, py, pz, 1), R2 = make_ray(px, py, pz, 2);
+    double best = INFINITY;
+    int c0 = 0, c1 = 0, c2 = 0;
+    for (int base = 0; base < F; base += SDF_TILE) {
+        const int nt = min(SDF_TILE, F - base);
+        __syncthreads();
+        for (int k = threadIdx.x; k < 3 * nt; k += SDF_BLOCK) s_tri[k] = tri[3 * (int64_t)base + k];
+        __syncthreads();
+        if (!valid) continue;
+#pragma unroll 1
+        for (int t = 0; t < nt; ++t) {
+            const float4 A = s_tri[3 * t], B = s_tri[3 * t + 1], C = s_tri[3 * t + 2];
+            best = fmin(best, tri_d2(p, A, B, C));
+            c0 += ray_hit(R0, A, B, C);
+            c1 += ray_hit(R1, A, B, C);
+            c2 += ray_hit(R2, A, B, C);
+        }
+    }
+    if (valid) out[i] = signed_out(best, (c0 & 1) + (c1 & 1) + (c2 & 1));
+}
+
+__global__ void k_sdf_init(uint32_t* __restrict__ mm, unsigned long long* __restrict__ bad) {
+    const int t = threadIdx.x;
+    if (t < 24) mm[t] = (t % 8) < 3 ? 0xffffffffu : 0u;
+    if (t < 3) bad[t] = ULLONG_MAX;
+}
+
+inline unsigned nblk(int64_t n, int b) { return (unsigned)ceil_div(n > 0 ? n : 1, b); }
+
+}  // namespace
+
+}  // namespace ds
+
+using namespace ds;
+
+extern "C" int ds_mesh_sdf(ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F,
+                           const float* points, int64_t P, int mode, float* sdf_out, void* stream) {
+    DS_REQUIRE(ws && tri_verts && faces, "ds_mesh_sdf: null argument");
+    DS_REQUIRE(V > 0 && F > 0, "ds_mesh_sdf: empty mesh (V = %lld, F = %lld)", (long long)V, (long long)F);
+    DS_REQUIRE(mode == 0 || mode == 1, "ds_mesh_sdf: unknown mode %d (0 = BVH, 1 = brute force)", mode);
+    DS_REQUIRE(P >= 0, "ds_mesh_sdf: negative point count");
+    DS_REQUIRE(F < ((int64_t)1 << 30) && P < ((int64_t)1 << 31) - SDF_BLOCK && V < ((int64_t)1 << 40),
+               "ds_mesh_sdf: too many faces or points");
+    if (P == 0) return DS_OK;
+    DS_REQUIRE(points && sdf_out, "ds_mesh_sdf: null argument");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t nmax = std::max(F, P);
+    size_t sort_tmp = 0;
+    DS_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, sort_tmp, (uint32_t*)nullptr, (uint32_t*)nullptr, (uint32_t*)nullptr,
+                                            (uint32_t*)nullptr, (int)nmax, 0, 30, st));
+    const size_t need = (size_t)F * (12 + 16 + 48 + 64 + 12) + (size_t)P * 16 + sort_tmp + (1 << 16);
+    DS_TRY(ws->arena.reserve(need, st));
+    Arena& a = ws->arena;
+    uint32_t* mm = a.take<uint32_t>(24);
+    unsigned long long* bad = a.take<unsigned long long>(4);
+    float4* tri = a.take<float4>(3 * F);
+    DS_REQUIRE(mm && bad && tri, "ds_mesh_sdf: workspace arena exhausted");
+    k_sdf_init<<<1, 32, 0, st>>>(mm, bad);
+    DS_LAUNCH_CHECK();
+    k_sdf_validate<<<296, 256, 0, st>>>(tri_verts, V, faces, F, points, P, bad);
+    DS_LAUNCH_CHECK();
+    unsigned long long bh[3];
+    DS_CUDA(cudaMemcpyAsync(bh, bad, sizeof(bh), cudaMemcpyDeviceToHost, st));
+    DS_CUDA(cudaStreamSynchronize(st));
+    DS_REQUIRE(bh[0] == ULLONG_MAX, "ds_mesh_sdf: face %llu has a vertex index outside [0, %lld)", bh[0], (long long)V);
+    DS_REQUIRE(bh[1] == ULLONG_MAX, "ds_mesh_sdf: vertex %llu has a non-finite coordinate", bh[1]);
+    DS_REQUIRE(bh[2] == ULLONG_MAX, "ds_mesh_sdf: query point %llu has a non-finite coordinate", bh[2]);
+
+    if (mode == 1) {
+        {
+            ProfScope prof(PROF_SDF_BUILD, st);
+            k_sdf_gather<<<nblk(F, 256), 256, 0, st>>>(tri_verts, faces, nullptr, F, tri);
+            DS_LAUNCH_CHECK();
+        }
+        ProfScope prof(PROF_SDF_QUERY, st);
+        k_sdf_query_brute<<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, (int)F, points, P, sdf_out);
+        DS_LAUNCH_CHECK();
+        return DS_OK;
+    }
+
+    float* cent = a.take<float>(3 * F);
+    uint32_t* codes = a.take<uint32_t>(nmax);
+    uint32_t* codes2 = a.take<uint32_t>(nmax);
+    uint32_t* iota = a.take<uint32_t>(nmax);
+    uint32_t* order = a.take<uint32_t>(F);
+    uint32_t* porder = a.take<uint32_t>(P);
+    BvhNode* nodes = a.take<BvhNode>(F);
+    int* parent = a.take<int>(2 * F);
+    int* arrived = a.take<int>(F);
+    void* scratch = a.take<char>(sort_tmp + 16);
+    DS_REQUIRE(cent && codes && codes2 && iota && order && porder && nodes && parent && arrived && scratch,
+               "ds_mesh_sdf: workspace arena exhausted");
+    uint32_t *mm_v = mm, *mm_c = mm + 8, *mm_p = mm + 16;
+    {
+    ProfScope prof(PROF_SDF_BUILD, st);
+    // triangles in Morton order of their centroids
+    k_sdf_centroids<<<nblk(F, 256), 256, 0, st>>>(tri_verts, faces, F, cent);
+    DS_LAUNCH_CHECK();
+    k_bbox<<<148, 256, 0, st>>>(cent, F, mm_c);
+    DS_LAUNCH_CHECK();
+    k_bbox<<<148, 256, 0, st>>>(tri_verts, V, mm_v);
+    DS_LAUNCH_CHECK();
+    k_bbox<<<148, 256, 0, st>>>(points, P, mm_p);
+    DS_LAUNCH_CHECK();
+    k_morton_codes<<<nblk(F, 256), 256, 0, st>>>(cent, F, mm_c, codes, iota);
+    DS_LAUNCH_CHECK();
+    DS_CUDA(cub::DeviceRadixSort::SortPairs(scratch, sort_tmp, codes, codes2, iota, order, (int)F, 0, 30, st));
+    count_launch();
+    k_sdf_gather<<<nblk(F, 256), 256, 0, st>>>(tri_verts, faces, order, F, tri);
+    DS_LAUNCH_CHECK();
+    if (F > 1) {
+        DS_CUDA(cudaMemsetAsync(arrived, 0, (size_t)F * sizeof(int), st));
+        k_sdf_karras<<<nblk(F - 1, 256), 256, 0, st>>>(codes2, (int)F, nodes, parent);
+        DS_LAUNCH_CHECK();
+        k_sdf_refit<<<nblk(F, 256), 256, 0, st>>>(tri, (int)F, nodes, parent, arrived, mm_v, mm_p);
+        DS_LAUNCH_CHECK();
+    }
+    }
+    // queries in Morton order of the points
+    ProfScope prof(PROF_SDF_QUERY, st);
+    k_morton_codes<<<nblk(P, 256), 256, 0, st>>>(points, P, mm_p, codes, iota);
+    DS_LAUNCH_CHECK();
+    DS_CUDA(cub::DeviceRadixSort::SortPairs(scratch, sort_tmp, codes, codes2, iota, porder, (int)P, 0, 30, st));
+    count_launch();
+    k_sdf_query_bvh<<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, nodes, (int)F, points, porder, P, sdf_out);
+    DS_LAUNCH_CHECK();
+    return DS_OK;
+}

@@ -1,4 +1,4 @@
-"""Tetrahedral mesh container: linear -> quadratic promotion, gmsh I/O.
+"""Tetrahedral mesh container: linear -> quadratic promotion, gmsh I/O, OBJ triangle-mesh input.
 
 API mirror of src/diffelastic/mesh.py:12-223 (`TetMesh`).  Node numbering of a
 promoted mesh is part of the parity contract (SURVEY.md A.3): quadratic node ids
@@ -109,6 +109,41 @@ def read_msh(filename):
     if points is None:
         raise ValueError(f"{filename}: no $Nodes section")
     return points, {k: np.concatenate(v, axis=0) for k, v in cells.items()}
+
+
+def read_obj(filename):
+    """Wavefront OBJ triangle mesh: returns (verts float32 (V,3), faces int64 (F,3)), the form the reference's `.obj`
+    targets (data/mesh/*.obj) take in `apply_sdf(path)`.  Reads `v` and `f` records only; face corners may be written
+    `i`, `i/j`, `i//k` or `i/j/k`, with 1-based or negative (relative to the vertices read so far) indices; polygons are
+    split into a triangle fan.  A missing file raises FileNotFoundError, a file without faces or with an index out of
+    range ValueError."""
+    verts, faces = [], []
+    with open(filename, "r") as f:
+        for lineno, raw in enumerate(f, 1):
+            rec = raw.split("#", 1)[0].split()
+            if not rec:
+                continue
+            if rec[0] == "v":
+                if len(rec) < 4:
+                    raise ValueError(f"{filename}:{lineno}: vertex with fewer than 3 coordinates")
+                verts.append((float(rec[1]), float(rec[2]), float(rec[3])))
+            elif rec[0] == "f":
+                if len(rec) < 4:
+                    raise ValueError(f"{filename}:{lineno}: face with fewer than 3 corners")
+                ids = []
+                for c in rec[1:]:
+                    i = int(c.split("/", 1)[0])
+                    j = i - 1 if i > 0 else len(verts) + i      # positive indices are checked once all vertices are read
+                    if i == 0 or j < 0:
+                        raise ValueError(f"{filename}:{lineno}: vertex index {i} out of range")
+                    ids.append(j)
+                faces.extend((ids[0], ids[k], ids[k + 1]) for k in range(1, len(ids) - 1))
+    if not faces:
+        raise ValueError(f"{filename}: no faces")
+    faces = np.asarray(faces, dtype=np.int64).reshape(-1, 3)
+    if faces.max() >= len(verts):
+        raise ValueError(f"{filename}: vertex index {int(faces.max()) + 1} out of range (1..{len(verts)})")
+    return np.asarray(verts, dtype=np.float32).reshape(-1, 3), faces
 
 
 def write_msh(filename, points, cells, cell_type):

@@ -12,10 +12,11 @@ gathers through the 16-case tables, `torch.unique` of the flattened tets, and th
 the reference's handful of element-wise fp32 torch operations (dmtet_thickness.py:133-148), in the same order, so the
 positions are bit-identical and autograd reaches the thickness parameter.
 
-Not reproduced: `apply_sdf(path)` samples a signed distance field from a triangle mesh with open3d ray casting
-(dmtet_thickness.py:301-314; SURVEY.md section 8f-4) -- here `apply_sdf` takes the sampled values (a tensor) or a callable
-evaluated at the grid vertices; the renderer's `mesh.Mesh` container (return_triangle=True) is replaced by a plain
-namespace with `v_pos` / `t_pos_idx`.
+`apply_sdf(path)` samples the signed distance of a triangle mesh (an OBJ file) at the grid vertices on the device
+(`native.mesh_sdf`, csrc/sdf.cu: BVH nearest-triangle queries and ray-crossing parity) where the reference uses open3d's
+`RaycastingScene` (dmtet_thickness.py:301-314; SURVEY.md section 8f-4); `apply_sdf` also takes the sampled values (a
+tensor) or a callable evaluated at the grid vertices.  Not reproduced: the renderer's `mesh.Mesh` container
+(return_triangle=True) is replaced by a plain namespace with `v_pos` / `t_pos_idx`.
 """
 import os
 import types
@@ -27,6 +28,7 @@ from ... import native
 from ...ddsp.oscillator import WeightedParam
 from ...diffelastic.diff_model import DiffSoundObj
 from ...diffelastic.material_model import MatSet
+from ...diffelastic.mesh import read_obj
 
 
 def _dev():
@@ -165,12 +167,15 @@ class DMTetGeometry(torch.nn.Module):
         return audio_loss
 
     def apply_sdf(self, sdf):
-        """`sdf`: tensor of signed distances at `self.verts` (positive inside, the sign convention `apply_sdf` of the
-        reference produces, dmtet_thickness.py:312) or a callable verts -> tensor.  A mesh file path is not supported:
-        sampling a triangle mesh needs the open3d ray-casting scene of the reference."""
+        """`sdf`: path of a triangle mesh (OBJ), tensor of signed distances at `self.verts`, or a callable verts -> tensor.
+        Signed distances are positive inside, the sign convention `apply_sdf` of the reference produces
+        (dmtet_thickness.py:312).  A path is read with `read_obj` and sampled at `self.verts` by `native.mesh_sdf`: exact
+        distance to the closest triangle, sign by ray-crossing parity (face orientation does not matter).  The mesh is
+        used as given, in its own coordinates, with no rescaling or recentring."""
         if isinstance(sdf, (str, os.PathLike)):
-            raise NotImplementedError("apply_sdf(path): triangle-mesh SDF sampling (open3d RaycastingScene) is not part of this "
-                                      "library; pass the sampled values or a callable")
+            v, f = read_obj(sdf)
+            dev = self.verts.device
+            sdf = native.mesh_sdf(torch.from_numpy(v).to(dev), torch.from_numpy(f).to(dev), self.verts.contiguous())
         values = sdf(self.verts) if callable(sdf) else sdf
         self.sdf = torch.as_tensor(values, dtype=torch.float32).to(self.verts.device).reshape(-1)
         self.marching_tets.max_thickness = self.sdf.max()

@@ -773,3 +773,21 @@ def largest_tet_component(tets, n_verts):
         tout = torch.empty(int(counts[2]), 4, dtype=torch.int64, device=dev)
         _lib.check(lib.ds_tet_components_fill(ws.handle, _p(tets), _p(kept), _p(tout), _stream()), "ds_tet_components_fill")
     return int(counts[0]), kept, tout, labels
+
+
+def mesh_sdf(tri_verts, faces, points, brute_force=False):
+    """Signed distance from each query point to a triangle mesh (ds_mesh_sdf): positive inside, negative outside, 0 on the
+    surface; the mesh is used in its own coordinates.  tri_verts (V, 3) fp32, faces (F, 3) int64, points (P, 3) fp32, all
+    on one device; returns (P,) fp32.  brute_force: every point against every face instead of the BVH (the test
+    reference; the outputs are bitwise equal)."""
+    lib = _lib.load()
+    assert tri_verts.dtype == torch.float32 and faces.dtype == torch.int64 and points.dtype == torch.float32
+    assert tri_verts.dim() == 2 and tri_verts.shape[1] == 3 and faces.dim() == 2 and faces.shape[1] == 3
+    assert points.dim() == 2 and points.shape[1] == 3
+    dev = points.device
+    ws = workspace(dev)
+    out = torch.empty(points.shape[0], dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.ds_mesh_sdf(ws.handle, _p(tri_verts), tri_verts.shape[0], _p(faces), faces.shape[0], _p(points),
+                                   points.shape[0], int(bool(brute_force)), _p(out), _stream()), "ds_mesh_sdf")
+    return out

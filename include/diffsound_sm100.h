@@ -422,6 +422,19 @@ int ds_tet_components_count(ds_workspace* ws, const int64_t* tets, int64_t T, in
                             int64_t* counts_host, void* stream);
 int ds_tet_components_fill(ds_workspace* ws, const int64_t* tets, int64_t* kept_verts, int64_t* tets_out, void* stream);
 
+/* ---- signed distance from points to a triangle mesh ---------------------------------------------------------------
+ * Replaces the open3d RaycastingScene sampling of DMTetGeometry.apply_sdf(path) (src/dmtet/geometry/dmtet_thickness.py:
+ * 301-314, whose compute_signed_distance is negated there): sdf_out[i] = +d inside, -d outside, with d the fp64 distance
+ * from points[i] to the closest point of the triangle set rounded once to fp32 (degenerate faces count as their edges;
+ * a point on the surface gives +0), inside = odd number of crossings for at least two of three fixed rays (watertight
+ * ray / triangle test, face orientation does not matter).  The mesh is used in its own coordinates.
+ * tri_verts fp32 [V x 3], faces int64 [F x 3], points fp32 [P x 3], sdf_out fp32 [P]; see csrc/sdf.cu.
+ * mode 0 = BVH, 1 = brute force (test reference; both give bitwise equal outputs).  Synchronises once: face indices
+ * outside [0, V) and non-finite coordinates return DS_ERR_ARG with a message, never a fault; so do V == 0, F == 0, a
+ * null pointer and an unknown mode.  P == 0 returns 0 without doing any work. */
+int ds_mesh_sdf(ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F, const float* points,
+                int64_t P, int mode, float* sdf_out, void* stream);
+
 /* ---- device-side timing per kernel class ---------------------------------------
  * Replaces the reference's opt-in torch.profiler hook of lobpcg (src/lobpcg/_lobpcg.py:357-369)
  * and the TICK/TOCK macros (src/include/macro.h:31-44): CUDA events around every launch site,
