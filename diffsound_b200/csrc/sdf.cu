@@ -22,6 +22,13 @@
 // or on the visit order, and BVH and brute-force outputs are bitwise equal.  Queries run in Morton order of the points.
 // Per-triangle arithmetic uses explicit round-to-nearest intrinsics (no contraction into FMA), so both kernels evaluate
 // bit-identical per-triangle values.
+//
+// Gradient (ds_mesh_sdf_nearest, ds_mesh_sdf_backward): the query kernels, instantiated to record the nearest face (the
+// lowest original index among faces at exactly the minimum, in both modes; ds_mesh_sdf runs the non-recording
+// instantiations, whose code is unchanged).  k_sdf_backward recomputes the closest point c = sum b_k v_k of that face by
+// the region analysis of tri_d2 and gives d sdf / d p = s u, d sdf / d v_k = -s b_k u (u = (p - c) / |p - c|; the
+// envelope theorem, so one formula for the face, edge and vertex regions).  The corner terms are reduced onto the
+// vertices in a fixed order (stable radix sort of the 3P corner vertex ids, fp64 sums per run): bitwise reproducible.
 #include "common.cuh"
 #include "../../include/diffsound_sm100.h"
 #include "kernels.cuh"
@@ -93,6 +100,67 @@ __device__ __forceinline__ double tri_d2(D3 p, float4 A4, float4 B4, float4 C4) 
     if (!(den > 0.0)) return fmin(fmin(seg_d2(p, a, b), seg_d2(p, b, c)), seg_d2(p, c, a));   // cancellation on a sliver
     const double v = vb / den, w = vc / den;
     return dist2(p, axpy3(axpy3(a, v, ab), w, ac));
+}
+
+// closest point of the segment [a, b] to p and its parameter t (c = a + t (b - a)): the arithmetic of seg_d2
+__device__ __forceinline__ D3 seg_closest(D3 p, D3 a, D3 b, double& t) {
+    const D3 ab = sub3(b, a);
+    const double l2 = dot3(ab, ab);
+    t = l2 > 0.0 ? dot3(sub3(p, a), ab) / l2 : 0.0;
+    t = fmin(fmax(t, 0.0), 1.0);
+    return axpy3(a, t, ab);
+}
+
+// closest point of the union of the three edges, the first of (ab, bc, ca) on ties, with its weights on (a, b, c)
+__device__ __forceinline__ D3 edges_closest(D3 p, D3 a, D3 b, D3 c, double (&w)[3]) {
+    double t0, t1, t2;
+    const D3 c0 = seg_closest(p, a, b, t0), c1 = seg_closest(p, b, c, t1), c2 = seg_closest(p, c, a, t2);
+    const double e0 = dist2(p, c0), e1 = dist2(p, c1), e2 = dist2(p, c2);
+    if (e0 <= e1 && e0 <= e2) { w[0] = 1.0 - t0; w[1] = t0; w[2] = 0.0; return c0; }
+    if (e1 <= e2) { w[0] = 0.0; w[1] = 1.0 - t1; w[2] = t1; return c1; }
+    w[0] = t2; w[1] = 0.0; w[2] = 1.0 - t2;
+    return c2;
+}
+
+// closest point of triangle (A, B, C) to p, by the same region analysis and arithmetic as tri_d2 (so dist2(p, c) is
+// the value tri_d2 returns), and its barycentric weights w on (A, B, C)
+__device__ __forceinline__ D3 tri_closest(D3 p, float4 A4, float4 B4, float4 C4, double (&w)[3]) {
+    const D3 a = d3(A4), b = d3(B4), c = d3(C4);
+    if (A4.w != 0.f) return edges_closest(p, a, b, c, w);
+    w[0] = w[1] = w[2] = 0.0;
+    const D3 ab = sub3(b, a), ac = sub3(c, a), ap = sub3(p, a);
+    const double d1 = dot3(ab, ap), d2 = dot3(ac, ap);
+    if (d1 <= 0.0 && d2 <= 0.0) { w[0] = 1.0; return a; }
+    const D3 bp = sub3(p, b);
+    const double d3_ = dot3(ab, bp), d4 = dot3(ac, bp);
+    if (d3_ >= 0.0 && d4 <= d3_) { w[1] = 1.0; return b; }
+    const double vc = dsub(dmul(d1, d4), dmul(d3_, d2));
+    if (vc <= 0.0 && d1 >= 0.0 && d3_ <= 0.0) {
+        const double t = d1 / dsub(d1, d3_);
+        w[0] = 1.0 - t; w[1] = t;
+        return axpy3(a, t, ab);
+    }
+    const D3 cp = sub3(p, c);
+    const double d5 = dot3(ab, cp), d6 = dot3(ac, cp);
+    if (d6 >= 0.0 && d5 <= d6) { w[2] = 1.0; return c; }
+    const double vb = dsub(dmul(d5, d2), dmul(d1, d6));
+    if (vb <= 0.0 && d2 >= 0.0 && d6 <= 0.0) {
+        const double t = d2 / dsub(d2, d6);
+        w[0] = 1.0 - t; w[2] = t;
+        return axpy3(a, t, ac);
+    }
+    const double va = dsub(dmul(d3_, d6), dmul(d5, d4));
+    const double e43 = dsub(d4, d3_), e56 = dsub(d5, d6);
+    if (va <= 0.0 && e43 >= 0.0 && e56 >= 0.0) {
+        const double t = e43 / dadd(e43, e56);
+        w[1] = 1.0 - t; w[2] = t;
+        return axpy3(b, t, sub3(c, b));
+    }
+    const double den = dadd(dadd(va, vb), vc);
+    if (!(den > 0.0)) return edges_closest(p, a, b, c, w);
+    const double v = vb / den, ww = vc / den;
+    w[0] = 1.0 - v - ww; w[1] = v; w[2] = ww;
+    return axpy3(axpy3(a, v, ab), ww, ac);
 }
 
 // ray from o along c_ray_dir[r], in the sheared frame of Woop et al.: kz = dominant axis, S = shear
@@ -191,10 +259,15 @@ __device__ __forceinline__ void load_node(const BvhNode* nodes, int n, float (&b
 }
 
 // ---- validation ------------------------------------------------------------------------------------------------
-// bad[0] = first face with an index outside [0, V), bad[1] = first non-finite vertex, bad[2] = first non-finite point
+// bad[0] = first face with an index outside [0, V), bad[1] = first non-finite vertex, bad[2] = first non-finite point,
+// bad[3] = first point whose nearest-face id (when given) is outside [0, F)
 __global__ void k_sdf_validate(const float* __restrict__ verts, int64_t V, const int64_t* __restrict__ faces, int64_t F,
-                               const float* __restrict__ pts, int64_t P, unsigned long long* __restrict__ bad) {
+                               const float* __restrict__ pts, int64_t P, const int32_t* __restrict__ nearest,
+                               unsigned long long* __restrict__ bad) {
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    if (nearest)
+        for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < P; i += stride)
+            if (nearest[i] < 0 || nearest[i] >= F) atomicMin(&bad[3], (unsigned long long)i);
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < 3 * F; i += stride) {
         const int64_t v = faces[i];
         if (v < 0 || v >= V) atomicMin(&bad[0], (unsigned long long)(i / 3));
@@ -215,32 +288,45 @@ __global__ void k_sdf_centroids(const float* __restrict__ verts, const int64_t* 
     for (int d = 0; d < 3; ++d) cent[3 * f + d] = (verts[3 * a + d] + verts[3 * b + d] + verts[3 * c + d]) * (1.0f / 3.0f);
 }
 
-// tri[3 i .. 3 i + 2] = corners of face order[i] (identity when order is NULL), sorted; A.w = 1 for a zero cross product
+// corners of face f, sorted, with their vertex ids; v[0].w = 1 for a zero cross product
+__device__ __forceinline__ void sorted_face(const float* __restrict__ verts, const int64_t* __restrict__ faces, int64_t f,
+                                            float4 (&v)[3], int64_t (&id)[3]) {
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        id[k] = faces[3 * f + k];
+        v[k] = make_float4(verts[3 * id[k]], verts[3 * id[k] + 1], verts[3 * id[k] + 2], 0.f);
+    }
+    // corners in lexicographic order: the per-triangle arithmetic then does not depend on how the face was written
+    // (orientation, first corner), so flipped or re-indexed meshes give bitwise equal results
+    auto cswap = [&](int i, int j) {
+        const float4 a = v[i], b = v[j];
+        const bool less = b.x < a.x || (b.x == a.x && (b.y < a.y || (b.y == a.y && b.z < a.z)));
+        if (less) {
+            v[i] = b; v[j] = a;
+            const int64_t t = id[i]; id[i] = id[j]; id[j] = t;
+        }
+    };
+    cswap(0, 1);
+    cswap(1, 2);
+    cswap(0, 1);
+    const D3 a = d3(v[0]), ab = sub3(d3(v[1]), a), ac = sub3(d3(v[2]), a);
+    const double nx = dsub(dmul(ab.y, ac.z), dmul(ab.z, ac.y));
+    const double ny = dsub(dmul(ab.z, ac.x), dmul(ab.x, ac.z));
+    const double nz = dsub(dmul(ab.x, ac.y), dmul(ab.y, ac.x));
+    v[0].w = (nx == 0.0 && ny == 0.0 && nz == 0.0) ? 1.f : 0.f;
+}
+
+// tri[3 i .. 3 i + 2] = corners of face order[i] (identity when order is NULL), sorted; A.w = 1 for a zero cross product,
+// B.w = the bits of the original face index (read only by the face-recording BVH query, which loads B whole anyway)
 __global__ void k_sdf_gather(const float* __restrict__ verts, const int64_t* __restrict__ faces,
                              const uint32_t* __restrict__ order, int64_t F, float4* __restrict__ tri) {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (i >= F) return;
     const int64_t f = order ? (int64_t)order[i] : i;
     float4 v[3];
-#pragma unroll
-    for (int k = 0; k < 3; ++k) {
-        const int64_t id = faces[3 * f + k];
-        v[k] = make_float4(verts[3 * id], verts[3 * id + 1], verts[3 * id + 2], 0.f);
-    }
-    // corners in lexicographic order: the per-triangle arithmetic then does not depend on how the face was written
-    // (orientation, first corner), so flipped or re-indexed meshes give bitwise equal results
-    auto cswap = [](float4& a, float4& b) {
-        const bool less = b.x < a.x || (b.x == a.x && (b.y < a.y || (b.y == a.y && b.z < a.z)));
-        if (less) { const float4 t = a; a = b; b = t; }
-    };
-    cswap(v[0], v[1]);
-    cswap(v[1], v[2]);
-    cswap(v[0], v[1]);
-    const D3 a = d3(v[0]), ab = sub3(d3(v[1]), a), ac = sub3(d3(v[2]), a);
-    const double nx = dsub(dmul(ab.y, ac.z), dmul(ab.z, ac.y));
-    const double ny = dsub(dmul(ab.z, ac.x), dmul(ab.x, ac.z));
-    const double nz = dsub(dmul(ab.x, ac.y), dmul(ab.y, ac.x));
-    v[0].w = (nx == 0.0 && ny == 0.0 && nz == 0.0) ? 1.f : 0.f;
+    int64_t id[3];
+    sorted_face(verts, faces, f, v, id);
+    v[1].w = __int_as_float((int)f);
     tri[3 * i] = v[0];
     tri[3 * i + 1] = v[1];
     tri[3 * i + 2] = v[2];
@@ -327,9 +413,13 @@ __device__ __forceinline__ float signed_out(double best, int votes) {
     return d == 0.0f ? 0.0f : (votes >= 2 ? d : -d);
 }
 
+// REC: also write the nearest face to face_out, as an original face index (B.w of the Morton-ordered triangle, see
+// k_sdf_gather); of several faces at exactly the same squared distance, the one with the lowest original index.  Boxes at a
+// distance equal to the current best are visited, so every face reaching the final minimum is evaluated.
+template <bool REC>
 __global__ void __launch_bounds__(SDF_BLOCK)
 k_sdf_query_bvh(const float4* __restrict__ tri, const BvhNode* __restrict__ nodes, int F, const float* __restrict__ pts,
-                const uint32_t* __restrict__ order, int64_t P, float* __restrict__ out) {
+                const uint32_t* __restrict__ order, int64_t P, float* __restrict__ out, int32_t* __restrict__ face_out) {
     __shared__ int s_node[SDF_STACK][SDF_BLOCK];
     __shared__ float s_d2[SDF_STACK][SDF_BLOCK];
     const int64_t i = blockIdx.x * (int64_t)SDF_BLOCK + threadIdx.x;
@@ -342,8 +432,10 @@ k_sdf_query_bvh(const float4* __restrict__ tri, const BvhNode* __restrict__ node
     int c[2];
     // nearest triangle
     double best = INFINITY;
+    int bestf = INT_MAX;
     if (F == 1) {
         best = tri_d2(p, tri[0], tri[1], tri[2]);
+        bestf = 0;
     } else {
         int sp = 0, node = 0;
         for (;;) {
@@ -354,7 +446,17 @@ k_sdf_query_bvh(const float4* __restrict__ tri, const BvhNode* __restrict__ node
             for (int s = 0; s < 2; ++s)
                 if (go[s] && c[s] < 0) {
                     const int t = ~c[s];
-                    best = fmin(best, tri_d2(p, tri[3 * t], tri[3 * t + 1], tri[3 * t + 2]));
+                    const float4 B = tri[3 * t + 1];
+                    const double d2 = tri_d2(p, tri[3 * t], B, tri[3 * t + 2]);
+                    if (REC) {
+                        const int f = __float_as_int(B.w);
+                        if (d2 < best || (d2 == best && f < bestf)) {
+                            best = d2;
+                            bestf = f;
+                        }
+                    } else {
+                        best = fmin(best, d2);
+                    }
                     go[s] = false;
                 }
             if (go[0] && go[1]) {
@@ -415,11 +517,15 @@ k_sdf_query_bvh(const float4* __restrict__ tri, const BvhNode* __restrict__ node
         votes += cnt & 1;
     }
     out[q] = signed_out(best, votes);
+    if (REC) face_out[q] = bestf;
 }
 
-// every point against every triangle (shared-memory tiles of SDF_TILE triangles): the reference for the BVH path
+// every point against every triangle (shared-memory tiles of SDF_TILE triangles): the reference for the BVH path.
+// REC: also write the nearest face (the first in index order at the minimum)
+template <bool REC>
 __global__ void __launch_bounds__(SDF_BLOCK)
-k_sdf_query_brute(const float4* __restrict__ tri, int F, const float* __restrict__ pts, int64_t P, float* __restrict__ out) {
+k_sdf_query_brute(const float4* __restrict__ tri, int F, const float* __restrict__ pts, int64_t P, float* __restrict__ out,
+                  int32_t* __restrict__ face_out) {
     __shared__ float4 s_tri[3 * SDF_TILE];
     const int64_t i = blockIdx.x * (int64_t)SDF_BLOCK + threadIdx.x;
     const bool valid = i < P;
@@ -427,6 +533,7 @@ k_sdf_query_brute(const float4* __restrict__ tri, int F, const float* __restrict
     const D3 p = {(double)px, (double)py, (double)pz};
     const Ray R0 = make_ray(px, py, pz, 0), R1 = make_ray(px, py, pz, 1), R2 = make_ray(px, py, pz, 2);
     double best = INFINITY;
+    int bestf = 0;
     int c0 = 0, c1 = 0, c2 = 0;
     for (int base = 0; base < F; base += SDF_TILE) {
         const int nt = min(SDF_TILE, F - base);
@@ -437,19 +544,91 @@ k_sdf_query_brute(const float4* __restrict__ tri, int F, const float* __restrict
 #pragma unroll 1
         for (int t = 0; t < nt; ++t) {
             const float4 A = s_tri[3 * t], B = s_tri[3 * t + 1], C = s_tri[3 * t + 2];
-            best = fmin(best, tri_d2(p, A, B, C));
+            if (REC) {
+                const double d2 = tri_d2(p, A, B, C);
+                if (d2 < best) {
+                    best = d2;
+                    bestf = base + t;
+                }
+            } else {
+                best = fmin(best, tri_d2(p, A, B, C));
+            }
             c0 += ray_hit(R0, A, B, C);
             c1 += ray_hit(R1, A, B, C);
             c2 += ray_hit(R2, A, B, C);
         }
     }
     if (valid) out[i] = signed_out(best, (c0 & 1) + (c1 & 1) + (c2 & 1));
+    if (REC && valid) face_out[i] = bestf;
 }
 
 __global__ void k_sdf_init(uint32_t* __restrict__ mm, unsigned long long* __restrict__ bad) {
     const int t = threadIdx.x;
     if (t < 24) mm[t] = (t % 8) < 3 ? 0xffffffffu : 0u;
-    if (t < 3) bad[t] = ULLONG_MAX;
+    if (t < 4) bad[t] = ULLONG_MAX;
+}
+
+// ---- backward --------------------------------------------------------------------------------------------------
+// One thread per point: closest point c of the point's nearest face (tri_closest on the sorted corners, as the forward
+// evaluated it), u = (p - c) / |p - c|, s = sign of sdf.  d sdf / d p = s u; d sdf / d v_k = -s b_k u for the corners
+// of the face.  gpt[p] = g s u (fp32, NULL: not written); coef[p] = -g s u (fp64) and w[3 p + k] = b_k, vid[3 p + k] =
+// vertex id of corner k, for the reduction onto the vertices (coef NULL: not written).  sdf == 0 or |p - c| == 0: 0.
+__global__ void k_sdf_backward(const float* __restrict__ verts, const int64_t* __restrict__ faces,
+                               const float* __restrict__ pts, int64_t P, const int32_t* __restrict__ nearest,
+                               const float* __restrict__ sdf, const float* __restrict__ g, float* __restrict__ gpt,
+                               double* __restrict__ coef, double* __restrict__ w, uint64_t* __restrict__ vid,
+                               uint32_t* __restrict__ entry) {
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i >= P) return;
+    float4 v[3];
+    int64_t id[3];
+    sorted_face(verts, faces, nearest[i], v, id);
+    const D3 p = {(double)pts[3 * i], (double)pts[3 * i + 1], (double)pts[3 * i + 2]};
+    double b[3];
+    const D3 c = tri_closest(p, v[0], v[1], v[2], b);
+    const D3 r = sub3(p, c);
+    const double d = sqrt(dot3(r, r));
+    const float s = sdf[i];
+    double gs = 0.0;
+    if (s != 0.0f && d > 0.0) gs = (s > 0.0f ? (double)g[i] : -(double)g[i]) / d;
+    const D3 gu = {dmul(gs, r.x), dmul(gs, r.y), dmul(gs, r.z)};
+    if (gpt) {
+        gpt[3 * i] = (float)gu.x;
+        gpt[3 * i + 1] = (float)gu.y;
+        gpt[3 * i + 2] = (float)gu.z;
+    }
+    if (coef) {
+        coef[3 * i] = -gu.x;
+        coef[3 * i + 1] = -gu.y;
+        coef[3 * i + 2] = -gu.z;
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            w[3 * i + k] = b[k];
+            vid[3 * i + k] = (uint64_t)id[k];
+            entry[3 * i + k] = (uint32_t)(3 * i + k);
+        }
+    }
+}
+
+// grad_verts: one thread per run of equal vertex ids in the sorted (vertex id, entry) list; the run's entries are in
+// ascending (point, corner) order (stable sort), summed in fp64, rounded once.  Vertices without entries stay 0.
+__global__ void k_sdf_vert_reduce(const uint64_t* __restrict__ key, const uint32_t* __restrict__ ent, int64_t n,
+                                  const double* __restrict__ coef, const double* __restrict__ w, float* __restrict__ gv) {
+    const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (i >= n || (i > 0 && key[i - 1] == key[i])) return;
+    const uint64_t k = key[i];
+    double sx = 0.0, sy = 0.0, sz = 0.0;
+    for (int64_t j = i; j < n && key[j] == k; ++j) {
+        const uint32_t e = ent[j];
+        const double b = w[e];
+        const int64_t q = e / 3;
+        sx = dadd(sx, dmul(b, coef[3 * q]));
+        sy = dadd(sy, dmul(b, coef[3 * q + 1]));
+        sz = dadd(sz, dmul(b, coef[3 * q + 2]));
+    }
+    gv[3 * k] = (float)sx;
+    gv[3 * k + 1] = (float)sy;
+    gv[3 * k + 2] = (float)sz;
 }
 
 inline unsigned nblk(int64_t n, int b) { return (unsigned)ceil_div(n > 0 ? n : 1, b); }
@@ -460,16 +639,42 @@ inline unsigned nblk(int64_t n, int b) { return (unsigned)ceil_div(n > 0 ? n : 1
 
 using namespace ds;
 
-extern "C" int ds_mesh_sdf(ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F,
-                           const float* points, int64_t P, int mode, float* sdf_out, void* stream) {
-    DS_REQUIRE(ws && tri_verts && faces, "ds_mesh_sdf: null argument");
-    DS_REQUIRE(V > 0 && F > 0, "ds_mesh_sdf: empty mesh (V = %lld, F = %lld)", (long long)V, (long long)F);
-    DS_REQUIRE(mode == 0 || mode == 1, "ds_mesh_sdf: unknown mode %d (0 = BVH, 1 = brute force)", mode);
-    DS_REQUIRE(P >= 0, "ds_mesh_sdf: negative point count");
+namespace {
+
+// the V / F / P checks and the limits every entry point shares
+int check_sizes(const char* fn, const ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F,
+                int64_t P) {
+    DS_REQUIRE(ws && tri_verts && faces, "%s: null argument", fn);
+    DS_REQUIRE(V > 0 && F > 0, "%s: empty mesh (V = %lld, F = %lld)", fn, (long long)V, (long long)F);
+    DS_REQUIRE(P >= 0, "%s: negative point count", fn);
     DS_REQUIRE(F < ((int64_t)1 << 30) && P < ((int64_t)1 << 31) - SDF_BLOCK && V < ((int64_t)1 << 40),
-               "ds_mesh_sdf: too many faces or points");
+               "%s: too many faces or points", fn);
+    return DS_OK;
+}
+
+// face indices in [0, V), finite coordinates and (nearest != NULL) nearest-face ids in [0, F): one synchronisation
+int validate(const char* fn, cudaStream_t st, unsigned long long* bad, const float* tri_verts, int64_t V,
+             const int64_t* faces, int64_t F, const float* points, int64_t P, const int32_t* nearest) {
+    k_sdf_validate<<<296, 256, 0, st>>>(tri_verts, V, faces, F, points, P, nearest, bad);
+    DS_LAUNCH_CHECK();
+    unsigned long long bh[4];
+    DS_CUDA(cudaMemcpyAsync(bh, bad, sizeof(bh), cudaMemcpyDeviceToHost, st));
+    DS_CUDA(cudaStreamSynchronize(st));
+    DS_REQUIRE(bh[0] == ULLONG_MAX, "%s: face %llu has a vertex index outside [0, %lld)", fn, bh[0], (long long)V);
+    DS_REQUIRE(bh[1] == ULLONG_MAX, "%s: vertex %llu has a non-finite coordinate", fn, bh[1]);
+    DS_REQUIRE(bh[2] == ULLONG_MAX, "%s: query point %llu has a non-finite coordinate", fn, bh[2]);
+    DS_REQUIRE(bh[3] == ULLONG_MAX, "%s: point %llu has nearest face outside [0, %lld)", fn, bh[3], (long long)F);
+    return DS_OK;
+}
+
+// ds_mesh_sdf and ds_mesh_sdf_nearest: face_out == NULL runs the non-recording kernels
+int mesh_sdf_impl(const char* fn, ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F,
+                  const float* points, int64_t P, int mode, float* sdf_out, int32_t* face_out, bool want_face,
+                  void* stream) {
+    DS_TRY(check_sizes(fn, ws, tri_verts, V, faces, F, P));
+    DS_REQUIRE(mode == 0 || mode == 1, "%s: unknown mode %d (0 = BVH, 1 = brute force)", fn, mode);
     if (P == 0) return DS_OK;
-    DS_REQUIRE(points && sdf_out, "ds_mesh_sdf: null argument");
+    DS_REQUIRE(points && sdf_out && (face_out || !want_face), "%s: null argument", fn);
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t nmax = std::max(F, P);
     size_t sort_tmp = 0;
@@ -481,17 +686,10 @@ extern "C" int ds_mesh_sdf(ds_workspace* ws, const float* tri_verts, int64_t V, 
     uint32_t* mm = a.take<uint32_t>(24);
     unsigned long long* bad = a.take<unsigned long long>(4);
     float4* tri = a.take<float4>(3 * F);
-    DS_REQUIRE(mm && bad && tri, "ds_mesh_sdf: workspace arena exhausted");
+    DS_REQUIRE(mm && bad && tri, "%s: workspace arena exhausted", fn);
     k_sdf_init<<<1, 32, 0, st>>>(mm, bad);
     DS_LAUNCH_CHECK();
-    k_sdf_validate<<<296, 256, 0, st>>>(tri_verts, V, faces, F, points, P, bad);
-    DS_LAUNCH_CHECK();
-    unsigned long long bh[3];
-    DS_CUDA(cudaMemcpyAsync(bh, bad, sizeof(bh), cudaMemcpyDeviceToHost, st));
-    DS_CUDA(cudaStreamSynchronize(st));
-    DS_REQUIRE(bh[0] == ULLONG_MAX, "ds_mesh_sdf: face %llu has a vertex index outside [0, %lld)", bh[0], (long long)V);
-    DS_REQUIRE(bh[1] == ULLONG_MAX, "ds_mesh_sdf: vertex %llu has a non-finite coordinate", bh[1]);
-    DS_REQUIRE(bh[2] == ULLONG_MAX, "ds_mesh_sdf: query point %llu has a non-finite coordinate", bh[2]);
+    DS_TRY(validate(fn, st, bad, tri_verts, V, faces, F, points, P, nullptr));
 
     if (mode == 1) {
         {
@@ -500,7 +698,10 @@ extern "C" int ds_mesh_sdf(ds_workspace* ws, const float* tri_verts, int64_t V, 
             DS_LAUNCH_CHECK();
         }
         ProfScope prof(PROF_SDF_QUERY, st);
-        k_sdf_query_brute<<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, (int)F, points, P, sdf_out);
+        if (face_out)
+            k_sdf_query_brute<true><<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, (int)F, points, P, sdf_out, face_out);
+        else
+            k_sdf_query_brute<false><<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, (int)F, points, P, sdf_out, nullptr);
         DS_LAUNCH_CHECK();
         return DS_OK;
     }
@@ -516,7 +717,7 @@ extern "C" int ds_mesh_sdf(ds_workspace* ws, const float* tri_verts, int64_t V, 
     int* arrived = a.take<int>(F);
     void* scratch = a.take<char>(sort_tmp + 16);
     DS_REQUIRE(cent && codes && codes2 && iota && order && porder && nodes && parent && arrived && scratch,
-               "ds_mesh_sdf: workspace arena exhausted");
+               "%s: workspace arena exhausted", fn);
     uint32_t *mm_v = mm, *mm_c = mm + 8, *mm_p = mm + 16;
     {
     ProfScope prof(PROF_SDF_BUILD, st);
@@ -549,7 +750,79 @@ extern "C" int ds_mesh_sdf(ds_workspace* ws, const float* tri_verts, int64_t V, 
     DS_LAUNCH_CHECK();
     DS_CUDA(cub::DeviceRadixSort::SortPairs(scratch, sort_tmp, codes, codes2, iota, porder, (int)P, 0, 30, st));
     count_launch();
-    k_sdf_query_bvh<<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, nodes, (int)F, points, porder, P, sdf_out);
+    if (face_out)
+        k_sdf_query_bvh<true><<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, nodes, (int)F, points, porder, P, sdf_out,
+                                                                         face_out);
+    else
+        k_sdf_query_bvh<false><<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, nodes, (int)F, points, porder, P, sdf_out,
+                                                                          nullptr);
+    DS_LAUNCH_CHECK();
+    return DS_OK;
+}
+
+}  // namespace
+
+extern "C" int ds_mesh_sdf(ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F,
+                           const float* points, int64_t P, int mode, float* sdf_out, void* stream) {
+    return mesh_sdf_impl("ds_mesh_sdf", ws, tri_verts, V, faces, F, points, P, mode, sdf_out, nullptr, false, stream);
+}
+
+extern "C" int ds_mesh_sdf_nearest(ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F,
+                                   const float* points, int64_t P, int mode, float* sdf_out, int32_t* face_out,
+                                   void* stream) {
+    return mesh_sdf_impl("ds_mesh_sdf_nearest", ws, tri_verts, V, faces, F, points, P, mode, sdf_out, face_out, true,
+                         stream);
+}
+
+extern "C" int ds_mesh_sdf_backward(ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F,
+                                    const float* points, int64_t P, const int32_t* face, const float* sdf,
+                                    const float* grad_sdf, float* grad_verts, float* grad_points, void* stream) {
+    const char* fn = "ds_mesh_sdf_backward";
+    DS_TRY(check_sizes(fn, ws, tri_verts, V, faces, F, P));
+    DS_REQUIRE(3 * P < ((int64_t)1 << 31), "%s: too many faces or points", fn);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (grad_verts) DS_CUDA(cudaMemsetAsync(grad_verts, 0, (size_t)V * 3 * sizeof(float), st));
+    if (P == 0) return DS_OK;
+    DS_REQUIRE(points && face && sdf && grad_sdf, "%s: null argument", fn);
+    int vbits = 1;
+    while (vbits < 64 && ((uint64_t)(V - 1) >> vbits) != 0) ++vbits;
+    const int64_t E = 3 * P;
+    size_t sort_tmp = 0;
+    DS_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, sort_tmp, (uint64_t*)nullptr, (uint64_t*)nullptr, (uint32_t*)nullptr,
+                                            (uint32_t*)nullptr, (int)E, 0, vbits, st));
+    const size_t need = (size_t)E * (8 + 8 + 16 + 8) + sort_tmp + (1 << 16);
+    DS_TRY(ws->arena.reserve(need, st));
+    Arena& a = ws->arena;
+    unsigned long long* bad = a.take<unsigned long long>(4);
+    uint32_t* mm = a.take<uint32_t>(24);
+    DS_REQUIRE(bad && mm, "%s: workspace arena exhausted", fn);
+    k_sdf_init<<<1, 32, 0, st>>>(mm, bad);
+    DS_LAUNCH_CHECK();
+    DS_TRY(validate(fn, st, bad, tri_verts, V, faces, F, points, P, face));
+    if (!grad_verts && !grad_points) return DS_OK;
+    double* coef = nullptr;
+    double* w = nullptr;
+    uint64_t *vid = nullptr, *vid2 = nullptr;
+    uint32_t *ent = nullptr, *ent2 = nullptr;
+    void* scratch = nullptr;
+    if (grad_verts) {
+        coef = a.take<double>(E);
+        w = a.take<double>(E);
+        vid = a.take<uint64_t>(E);
+        vid2 = a.take<uint64_t>(E);
+        ent = a.take<uint32_t>(E);
+        ent2 = a.take<uint32_t>(E);
+        scratch = a.take<char>(sort_tmp + 16);
+        DS_REQUIRE(coef && w && vid && vid2 && ent && ent2 && scratch, "%s: workspace arena exhausted", fn);
+    }
+    k_sdf_backward<<<nblk(P, 256), 256, 0, st>>>(tri_verts, faces, points, P, face, sdf, grad_sdf, grad_points, coef, w,
+                                                 vid, ent);
+    DS_LAUNCH_CHECK();
+    if (!grad_verts) return DS_OK;
+    // stable sort by vertex id: each vertex's entries stay in ascending (point, corner) order
+    DS_CUDA(cub::DeviceRadixSort::SortPairs(scratch, sort_tmp, vid, vid2, ent, ent2, (int)E, 0, vbits, st));
+    count_launch();
+    k_sdf_vert_reduce<<<nblk(E, 256), 256, 0, st>>>(vid2, ent2, E, coef, w, grad_verts);
     DS_LAUNCH_CHECK();
     return DS_OK;
 }

@@ -15,7 +15,9 @@ positions are bit-identical and autograd reaches the thickness parameter.
 `apply_sdf(path)` samples the signed distance of a triangle mesh (an OBJ file) at the grid vertices on the device
 (`native.mesh_sdf`, csrc/sdf.cu: BVH nearest-triangle queries and ray-crossing parity) where the reference uses open3d's
 `RaycastingScene` (dmtet_thickness.py:301-314; SURVEY.md section 8f-4); `apply_sdf` also takes the sampled values (a
-tensor) or a callable evaluated at the grid vertices.  Not reproduced: the renderer's `mesh.Mesh` container
+tensor) or a callable evaluated at the grid vertices.  `apply_sdf((verts, faces))` takes the triangle mesh as tensors and
+samples it through the differentiable `mesh_sdf` (mesh_sdf.py): with `verts.requires_grad` the mesh is sampled again on
+every `getMesh()`, so the loss of a `tick()` reaches the triangle-mesh vertices.  Not reproduced: the renderer's `mesh.Mesh` container
 (return_triangle=True) is replaced by a plain namespace with `v_pos` / `t_pos_idx`.
 """
 import os
@@ -29,6 +31,7 @@ from ...ddsp.oscillator import WeightedParam
 from ...diffelastic.diff_model import DiffSoundObj
 from ...diffelastic.material_model import MatSet
 from ...diffelastic.mesh import read_obj
+from .mesh_sdf import mesh_sdf
 
 
 def _dev():
@@ -119,6 +122,7 @@ class DMTetGeometry(torch.nn.Module):
         self.indices = torch.tensor(np.asarray(grid[1]), dtype=torch.long, device=dev)
         self.generate_edges()
         self.sdf = torch.zeros_like(self.verts[:, 0])
+        self._sdf_mesh = None       # (verts, faces) of apply_sdf((verts, faces)) when verts requires grad
 
     def generate_edges(self):
         """`all_edges` (unique sorted vertex pairs of the background grid, dmtet_thickness.py:225-230) is only read by the
@@ -139,6 +143,8 @@ class DMTetGeometry(torch.nn.Module):
         return torch.min(self.verts, dim=0).values, torch.max(self.verts, dim=0).values
 
     def getMesh(self, return_triangle=False, thickness_coef=None):
+        if self._sdf_mesh is not None:
+            self._sample_mesh(*self._sdf_mesh)
         verts, faces, verts_tetmesh, tets_tetmesh = self.marching_tets(self.verts, self.sdf, self.indices, thickness_coef)
         if return_triangle:
             return types.SimpleNamespace(v_pos=verts, t_pos_idx=faces)
@@ -171,13 +177,30 @@ class DMTetGeometry(torch.nn.Module):
         Signed distances are positive inside, the sign convention `apply_sdf` of the reference produces
         (dmtet_thickness.py:312).  A path is read with `read_obj` and sampled at `self.verts` by `native.mesh_sdf`: exact
         distance to the closest triangle, sign by ray-crossing parity (face orientation does not matter).  The mesh is
-        used as given, in its own coordinates, with no rescaling or recentring."""
+        used as given, in its own coordinates, with no rescaling or recentring.
+        `sdf` = (verts (V, 3), faces (F, 3)) tensors: the triangle mesh, sampled by the differentiable `mesh_sdf`.  If
+        verts.requires_grad, the geometry keeps the mesh and every `getMesh()` samples it again (and resets
+        `max_thickness`), so each `tick()` builds a fresh graph down to verts; otherwise it is sampled once, like a path."""
+        self._sdf_mesh = None
+        if isinstance(sdf, (tuple, list)) and len(sdf) == 2:
+            verts, faces = sdf
+            dev = self.verts.device
+            verts = torch.as_tensor(verts, device=dev)
+            faces = torch.as_tensor(faces, device=dev).to(torch.int64)
+            if verts.requires_grad:
+                self._sdf_mesh = (verts, faces)
+            self._sample_mesh(verts, faces)
+            return
         if isinstance(sdf, (str, os.PathLike)):
             v, f = read_obj(sdf)
             dev = self.verts.device
             sdf = native.mesh_sdf(torch.from_numpy(v).to(dev), torch.from_numpy(f).to(dev), self.verts.contiguous())
         values = sdf(self.verts) if callable(sdf) else sdf
         self.sdf = torch.as_tensor(values, dtype=torch.float32).to(self.verts.device).reshape(-1)
+        self.marching_tets.max_thickness = self.sdf.max()
+
+    def _sample_mesh(self, verts, faces):
+        self.sdf = mesh_sdf(verts, faces, self.verts.contiguous())
         self.marching_tets.max_thickness = self.sdf.max()
 
     def parameters(self):

@@ -791,3 +791,43 @@ def mesh_sdf(tri_verts, faces, points, brute_force=False):
         _lib.check(lib.ds_mesh_sdf(ws.handle, _p(tri_verts), tri_verts.shape[0], _p(faces), faces.shape[0], _p(points),
                                    points.shape[0], int(bool(brute_force)), _p(out), _stream()), "ds_mesh_sdf")
     return out
+
+
+def _check_mesh(tri_verts, faces, points):
+    assert tri_verts.dtype == torch.float32 and faces.dtype == torch.int64 and points.dtype == torch.float32
+    assert tri_verts.dim() == 2 and tri_verts.shape[1] == 3 and faces.dim() == 2 and faces.shape[1] == 3
+    assert points.dim() == 2 and points.shape[1] == 3
+
+
+def mesh_sdf_nearest(tri_verts, faces, points, brute_force=False):
+    """`mesh_sdf` and the nearest face of each point (ds_mesh_sdf_nearest): returns (sdf (P,) fp32, face (P,) int32).
+    sdf is bitwise equal to `mesh_sdf`; of faces at exactly the same distance, the lowest index (both modes)."""
+    lib = _lib.load()
+    _check_mesh(tri_verts, faces, points)
+    dev = points.device
+    ws = workspace(dev)
+    out = torch.empty(points.shape[0], dtype=torch.float32, device=dev)
+    face = torch.empty(points.shape[0], dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.ds_mesh_sdf_nearest(ws.handle, _p(tri_verts), tri_verts.shape[0], _p(faces), faces.shape[0],
+                                           _p(points), points.shape[0], int(bool(brute_force)), _p(out), _p(face),
+                                           _stream()), "ds_mesh_sdf_nearest")
+    return out, face
+
+
+def mesh_sdf_backward(tri_verts, faces, points, face, sdf, grad_sdf, want_verts=True, want_points=True):
+    """Gradient of `mesh_sdf` (ds_mesh_sdf_backward) given the (sdf, face) of `mesh_sdf_nearest` and the upstream
+    gradient grad_sdf (P,) fp32: returns (grad_verts (V, 3) or None, grad_points (P, 3) or None), fp32, bitwise
+    reproducible."""
+    lib = _lib.load()
+    _check_mesh(tri_verts, faces, points)
+    assert face.dtype == torch.int32 and sdf.dtype == torch.float32 and grad_sdf.dtype == torch.float32
+    dev = points.device
+    ws = workspace(dev)
+    gv = torch.empty(tri_verts.shape[0], 3, dtype=torch.float32, device=dev) if want_verts else None
+    gp = torch.empty(points.shape[0], 3, dtype=torch.float32, device=dev) if want_points else None
+    with torch.cuda.device(dev):
+        _lib.check(lib.ds_mesh_sdf_backward(ws.handle, _p(tri_verts), tri_verts.shape[0], _p(faces), faces.shape[0],
+                                            _p(points), points.shape[0], _p(face), _p(sdf), _p(grad_sdf), _p(gv), _p(gp),
+                                            _stream()), "ds_mesh_sdf_backward")
+    return gv, gp

@@ -434,6 +434,22 @@ int ds_tet_components_fill(ds_workspace* ws, const int64_t* tets, int64_t* kept_
  * null pointer and an unknown mode.  P == 0 returns 0 without doing any work. */
 int ds_mesh_sdf(ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F, const float* points,
                 int64_t P, int mode, float* sdf_out, void* stream);
+/* ds_mesh_sdf, and face_out int32 [P] = the face nearest to each point (an index into faces; of several faces at exactly
+ * the same fp64 squared distance, the lowest index, in both modes, so BVH and brute force give bitwise equal ids).
+ * sdf_out is bitwise equal to ds_mesh_sdf's.  Same checks and synchronisation as ds_mesh_sdf. */
+int ds_mesh_sdf_nearest(ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F,
+                        const float* points, int64_t P, int mode, float* sdf_out, int32_t* face_out, void* stream);
+/* Gradient of ds_mesh_sdf: with c = sum_k b_k v_k the closest point of face[i] to points[i] (the forward's region
+ * analysis; degenerate faces: the nearest edge), u = (p - c) / |p - c| and s = sign(sdf[i]):
+ *   grad_points[i] = grad_sdf[i] s u;   grad_verts[v] = sum over points i and corners k of face[i] with vertex id v of
+ *   -grad_sdf[i] s b_k u.
+ * Zero where sdf[i] == 0 or |p - c| == 0.  fp64 throughout, rounded once to fp32; grad_verts is summed in ascending
+ * (point, corner) order without atomics, so the result is bitwise reproducible.  face int32 [P] and sdf fp32 [P] as
+ * ds_mesh_sdf_nearest returned them, grad_sdf fp32 [P], grad_verts fp32 [V x 3], grad_points fp32 [P x 3]; either output
+ * may be NULL.  Synchronises once: the checks of ds_mesh_sdf, and a nearest-face id outside [0, F) returns DS_ERR_ARG. */
+int ds_mesh_sdf_backward(ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F,
+                         const float* points, int64_t P, const int32_t* face, const float* sdf, const float* grad_sdf,
+                         float* grad_verts, float* grad_points, void* stream);
 
 /* ---- device-side timing per kernel class ---------------------------------------
  * Replaces the reference's opt-in torch.profiler hook of lobpcg (src/lobpcg/_lobpcg.py:357-369)
