@@ -113,6 +113,8 @@ SIGNATURES = {
     "ds_mesh_sdf": (cint, [ptr, f32p, i64, i64p, i64, f32p, i64, cint, f32p, ptr]),
     "ds_mesh_sdf_nearest": (cint, [ptr, f32p, i64, i64p, i64, f32p, i64, cint, f32p, i32p, ptr]),
     "ds_mesh_sdf_backward": (cint, [ptr, f32p, i64, i64p, i64, f32p, i64, i32p, f32p, f32p, f32p, f32p, ptr]),
+    "ds_mesh_winding_number": (cint, [ptr, f32p, i64, i64p, i64, f32p, i64, cint, f32p, ptr]),
+    "ds_mesh_sdf_winding": (cint, [ptr, f32p, i64, i64p, i64, f32p, i64, cint, f32p, i32p, ptr]),
     "ds_lobpcg_residual": (cint, [f64p, f64p, i64, cint, i64, f64p, f64p, i64, f64p, f64p, ptr]),
     "ds_gather_cols_f32": (cint, [f64p, i64, C.POINTER(C.c_int), cint, cint, i64, f32p, ptr]),
     "ds_widen_f32": (cint, [f32p, cint, i64, f64p, i64, ptr]),

@@ -80,7 +80,7 @@ struct Arena {
 enum ProfClass {
     PROF_PATTERN = 0, PROF_GEOMETRY, PROF_ASSEMBLE, PROF_SPMM, PROF_CHEB, PROF_GRAM, PROF_GEMM, PROF_EIGH,
     PROF_RESIDUAL, PROF_COPY, PROF_GRAD, PROF_QUADFORM, PROF_SYNTH, PROF_OTHER, PROF_COARSE, PROF_TRANSFER, PROF_JACOBI,
-    PROF_SDF_BUILD, PROF_SDF_QUERY, PROF_NCLASS
+    PROF_SDF_BUILD, PROF_SDF_QUERY, PROF_SDF_WINDING, PROF_NCLASS
 };
 bool prof_enabled(int cls);
 void prof_begin(int cls, cudaStream_t s);

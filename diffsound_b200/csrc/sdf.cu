@@ -29,6 +29,17 @@
 // the region analysis of tri_d2 and gives d sdf / d p = s u, d sdf / d v_k = -s b_k u (u = (p - c) / |p - c|; the
 // envelope theorem, so one formula for the face, edge and vertex regions).  The corner terms are reduced onto the
 // vertices in a fixed order (stable radix sort of the 3P corner vertex ids, fp64 sums per run): bitwise reproducible.
+//
+// Winding number (ds_mesh_winding_number, ds_mesh_sdf_winding): w(p) = sum of the faces' oriented solid angles / 4 pi
+// (Jacobson, Kavan & Sorkine-Hornung 2013), each face's exact term 2 atan2(num, den) (Van Oosterom & Strackee) in fp64
+// from its sorted corners, times the orientation of the sort (C.w of the gathered triangle, k_sdf_gather<true>).  Brute
+// force: every face in face order.  BVH (Barill, Dickson, Schmidt, Levin & Jacobson 2018): a radix tree built as for
+// ds_mesh_sdf but from the centroids of the sorted corners (k_sdf_centroids<true>), so that the tree, and the order of
+// every sum over it, do not depend on how the faces are written (flipped faces give exactly -w, re-indexed or unshared
+// vertices the same bits, in both modes); k_sdf_wn_moments forms each node's moments bottom-up (child 0 + child 1,
+// fp64), and k_sdf_winding_bvh replaces a subtree far from the point by its far-field expansion (WN_BETA).
+// ds_mesh_sdf_winding writes +1 / -1 (|w| >= 1/2 in fp64) to sdf_out and runs the
+// query kernels instantiated WIND: the same nearest-face search, the sign taken from sdf_out instead of the rays.
 #include "common.cuh"
 #include "../../include/diffsound_sm100.h"
 #include "kernels.cuh"
@@ -279,17 +290,9 @@ __global__ void k_sdf_validate(const float* __restrict__ verts, int64_t V, const
 }
 
 // ---- build -----------------------------------------------------------------------------------------------------
-__global__ void k_sdf_centroids(const float* __restrict__ verts, const int64_t* __restrict__ faces, int64_t F,
-                                float* __restrict__ cent) {
-    const int64_t f = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
-    if (f >= F) return;
-    const int64_t a = faces[3 * f], b = faces[3 * f + 1], c = faces[3 * f + 2];
-#pragma unroll
-    for (int d = 0; d < 3; ++d) cent[3 * f + d] = (verts[3 * a + d] + verts[3 * b + d] + verts[3 * c + d]) * (1.0f / 3.0f);
-}
-
-// corners of face f, sorted, with their vertex ids; v[0].w = 1 for a zero cross product
-__device__ __forceinline__ void sorted_face(const float* __restrict__ verts, const int64_t* __restrict__ faces, int64_t f,
+// corners of face f, sorted, with their vertex ids; v[0].w = 1 for a zero cross product.  Returns the orientation of the
+// sorted corners relative to the face as written: +1 (even permutation) or -1 (odd)
+__device__ __forceinline__ float sorted_face(const float* __restrict__ verts, const int64_t* __restrict__ faces, int64_t f,
                                             float4 (&v)[3], int64_t (&id)[3]) {
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
@@ -298,12 +301,14 @@ __device__ __forceinline__ void sorted_face(const float* __restrict__ verts, con
     }
     // corners in lexicographic order: the per-triangle arithmetic then does not depend on how the face was written
     // (orientation, first corner), so flipped or re-indexed meshes give bitwise equal results
+    bool odd = false;
     auto cswap = [&](int i, int j) {
         const float4 a = v[i], b = v[j];
         const bool less = b.x < a.x || (b.x == a.x && (b.y < a.y || (b.y == a.y && b.z < a.z)));
         if (less) {
             v[i] = b; v[j] = a;
             const int64_t t = id[i]; id[i] = id[j]; id[j] = t;
+            odd = !odd;
         }
     };
     cswap(0, 1);
@@ -314,10 +319,35 @@ __device__ __forceinline__ void sorted_face(const float* __restrict__ verts, con
     const double ny = dsub(dmul(ab.z, ac.x), dmul(ab.x, ac.z));
     const double nz = dsub(dmul(ab.x, ac.y), dmul(ab.y, ac.x));
     v[0].w = (nx == 0.0 && ny == 0.0 && nz == 0.0) ? 1.f : 0.f;
+    return odd ? -1.f : 1.f;
+}
+
+// cent[3 f ..] = centroid of face f in fp32, its corners summed in the order written.  SORTED: summed in lexicographic
+// order instead (sorted_face), so the centroids, and with them the Morton order and the tree, do not depend on the face's
+// orientation or first corner: the winding number's far-field sums are then bitwise odd under flipping every face
+template <bool SORTED>
+__global__ void k_sdf_centroids(const float* __restrict__ verts, const int64_t* __restrict__ faces, int64_t F,
+                                float* __restrict__ cent) {
+    const int64_t f = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (f >= F) return;
+    if (SORTED) {
+        float4 v[3];
+        int64_t id[3];
+        sorted_face(verts, faces, f, v, id);
+        cent[3 * f] = (v[0].x + v[1].x + v[2].x) * (1.0f / 3.0f);
+        cent[3 * f + 1] = (v[0].y + v[1].y + v[2].y) * (1.0f / 3.0f);
+        cent[3 * f + 2] = (v[0].z + v[1].z + v[2].z) * (1.0f / 3.0f);
+        return;
+    }
+    const int64_t a = faces[3 * f], b = faces[3 * f + 1], c = faces[3 * f + 2];
+#pragma unroll
+    for (int d = 0; d < 3; ++d) cent[3 * f + d] = (verts[3 * a + d] + verts[3 * b + d] + verts[3 * c + d]) * (1.0f / 3.0f);
 }
 
 // tri[3 i .. 3 i + 2] = corners of face order[i] (identity when order is NULL), sorted; A.w = 1 for a zero cross product,
-// B.w = the bits of the original face index (read only by the face-recording BVH query, which loads B whole anyway)
+// B.w = the bits of the original face index (read only by the face-recording BVH query, which loads B whole anyway);
+// ORIENT: C.w = +1 / -1, the orientation of the sorted corners relative to the face as written (for the winding number)
+template <bool ORIENT>
 __global__ void k_sdf_gather(const float* __restrict__ verts, const int64_t* __restrict__ faces,
                              const uint32_t* __restrict__ order, int64_t F, float4* __restrict__ tri) {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
@@ -325,7 +355,8 @@ __global__ void k_sdf_gather(const float* __restrict__ verts, const int64_t* __r
     const int64_t f = order ? (int64_t)order[i] : i;
     float4 v[3];
     int64_t id[3];
-    sorted_face(verts, faces, f, v, id);
+    const float o = sorted_face(verts, faces, f, v, id);
+    if (ORIENT) v[2].w = o;
     v[1].w = __int_as_float((int)f);
     tri[3 * i] = v[0];
     tri[3 * i + 1] = v[1];
@@ -416,7 +447,9 @@ __device__ __forceinline__ float signed_out(double best, int votes) {
 // REC: also write the nearest face to face_out, as an original face index (B.w of the Morton-ordered triangle, see
 // k_sdf_gather); of several faces at exactly the same squared distance, the one with the lowest original index.  Boxes at a
 // distance equal to the current best are visited, so every face reaching the final minimum is evaluated.
-template <bool REC>
+// WIND: no rays; out[q] holds +1 / -1 on entry (inside / outside by the winding number, k_sdf_winding_*) and the sign
+// is taken from it.  The nearest-face search is the same code in every instantiation.
+template <bool REC, bool WIND = false>
 __global__ void __launch_bounds__(SDF_BLOCK)
 k_sdf_query_bvh(const float4* __restrict__ tri, const BvhNode* __restrict__ nodes, int F, const float* __restrict__ pts,
                 const uint32_t* __restrict__ order, int64_t P, float* __restrict__ out, int32_t* __restrict__ face_out) {
@@ -484,6 +517,8 @@ k_sdf_query_bvh(const float4* __restrict__ tri, const BvhNode* __restrict__ node
     }
     // crossing parity of the three rays
     int votes = 0;
+    if constexpr (WIND) votes = out[q] > 0.f ? 2 : 0;
+    else
 #pragma unroll 1
     for (int r = 0; r < 3; ++r) {
         const Ray R = make_ray(px, py, pz, r);
@@ -521,8 +556,8 @@ k_sdf_query_bvh(const float4* __restrict__ tri, const BvhNode* __restrict__ node
 }
 
 // every point against every triangle (shared-memory tiles of SDF_TILE triangles): the reference for the BVH path.
-// REC: also write the nearest face (the first in index order at the minimum)
-template <bool REC>
+// REC: also write the nearest face (the first in index order at the minimum); WIND: as k_sdf_query_bvh
+template <bool REC, bool WIND = false>
 __global__ void __launch_bounds__(SDF_BLOCK)
 k_sdf_query_brute(const float4* __restrict__ tri, int F, const float* __restrict__ pts, int64_t P, float* __restrict__ out,
                   int32_t* __restrict__ face_out) {
@@ -553,13 +588,221 @@ k_sdf_query_brute(const float4* __restrict__ tri, int F, const float* __restrict
             } else {
                 best = fmin(best, tri_d2(p, A, B, C));
             }
-            c0 += ray_hit(R0, A, B, C);
-            c1 += ray_hit(R1, A, B, C);
-            c2 += ray_hit(R2, A, B, C);
+            if constexpr (!WIND) {
+                c0 += ray_hit(R0, A, B, C);
+                c1 += ray_hit(R1, A, B, C);
+                c2 += ray_hit(R2, A, B, C);
+            }
         }
     }
+    if constexpr (WIND) c0 = c1 = valid && out[i] > 0.f ? 1 : 0;
     if (valid) out[i] = signed_out(best, (c0 & 1) + (c1 & 1) + (c2 & 1));
     if (REC && valid) face_out[i] = bestf;
+}
+
+// ---- generalised winding number ----------------------------------------------------------------------------------
+// Far-field acceptance: a subtree whose corners all lie within r of its centroid c is replaced by its expansion when
+// |q - c| > WN_BETA r.  The expansion goes through the first moment m (below).  Barill et al. use beta = 2; at 3 the BVH
+// mode's max |w - exact| measured 0.024 on the test meshes (tested bar 0.05) and 0.019 on the icospheres of
+// scripts/bench_winding.py.  This is a measurement, not a bound: the truncation error of a node grows with the face area
+// inside its radius, which is unbounded (many stacked or crumpled layers).
+constexpr double WN_BETA = 3.0;
+constexpr double WN_INV_4PI = 0.079577471545947667884;      // 1 / (4 pi)
+
+// Moments of an internal node's subtree (indexed like BvhNode), fp64: c = area-weighted centroid of the face centroids,
+// r = radius around c bounding every corner, n = sum of the oriented area vectors a_f, m[3 i + j] = sum a_f,i (c_f - c)_j
+// (Barill et al. 2018's second-order term), area = sum |a_f|
+struct __align__(16) WnNode {
+    double c[3], r;
+    double n[3], area;
+    double m[9], pad;
+};
+
+// solid angle of the oriented triangle (A, B, C) seen from p (Van Oosterom & Strackee 1983): 2 atan2(num, den) of the
+// sorted corners, times their orientation C.w; 0 for a degenerate face
+__device__ __forceinline__ double solid_angle(D3 p, float4 A4, float4 B4, float4 C4) {
+    if (A4.w != 0.f) return 0.0;
+    const D3 a = sub3(d3(A4), p), b = sub3(d3(B4), p), c = sub3(d3(C4), p);
+    const double la = sqrt(dot3(a, a)), lb = sqrt(dot3(b, b)), lc = sqrt(dot3(c, c));
+    const D3 bxc = {dsub(dmul(b.y, c.z), dmul(b.z, c.y)), dsub(dmul(b.z, c.x), dmul(b.x, c.z)), dsub(dmul(b.x, c.y), dmul(b.y, c.x))};
+    const double num = dot3(a, bxc);
+    const double den = dadd(dadd(dadd(dmul(dmul(la, lb), lc), dmul(dot3(a, b), lc)), dmul(dot3(a, c), lb)), dmul(dot3(b, c), la));
+    return dmul((double)C4.w, 2.0 * atan2(num, den));
+}
+
+// moments of one face (m = 0: the face's centroid is the expansion centre)
+__device__ __forceinline__ WnNode leaf_moments(float4 A4, float4 B4, float4 C4) {
+    WnNode L;
+    const D3 a = d3(A4), b = d3(B4), c = d3(C4);
+    const double third = 1.0 / 3.0;
+    const D3 g = {dmul(dadd(dadd(a.x, b.x), c.x), third), dmul(dadd(dadd(a.y, b.y), c.y), third),
+                  dmul(dadd(dadd(a.z, b.z), c.z), third)};
+    const D3 ab = sub3(b, a), ac = sub3(c, a);
+    D3 n = {dsub(dmul(ab.y, ac.z), dmul(ab.z, ac.y)), dsub(dmul(ab.z, ac.x), dmul(ab.x, ac.z)), dsub(dmul(ab.x, ac.y), dmul(ab.y, ac.x))};
+    const double s = A4.w != 0.f ? 0.0 : 0.5 * (double)C4.w;
+    n = {dmul(s, n.x), dmul(s, n.y), dmul(s, n.z)};
+    L.c[0] = g.x; L.c[1] = g.y; L.c[2] = g.z;
+    L.r = sqrt(fmax(fmax(dist2(a, g), dist2(b, g)), dist2(c, g)));
+    L.n[0] = n.x; L.n[1] = n.y; L.n[2] = n.z;
+    L.area = sqrt(dot3(n, n));
+#pragma unroll
+    for (int k = 0; k < 9; ++k) L.m[k] = 0.0;
+    L.pad = 0.0;
+    return L;
+}
+
+// moments of child s of a node: a leaf's from its triangle, an internal node's as stored (read through L2: written by
+// another thread of the same launch)
+__device__ __forceinline__ WnNode child_moments(const float4* __restrict__ tri, const WnNode* mom, int ch) {
+    if (ch < 0) {
+        const int t = ~ch;
+        return leaf_moments(tri[3 * t], tri[3 * t + 1], tri[3 * t + 2]);
+    }
+    WnNode M;
+    const double2* src = reinterpret_cast<const double2*>(mom + ch);
+    double2* dst = reinterpret_cast<double2*>(&M);
+#pragma unroll
+    for (int k = 0; k < 9; ++k) dst[k] = __ldcg(src + k);
+    return M;
+}
+
+// bottom-up moments, one thread per leaf; the second thread to reach a node forms it as child 0 + child 1 (so the
+// result does not depend on which thread arrives last):
+//   area = A0 + A1, c = (A0 c0 + A1 c1) / area (the midpoint when area == 0), n = n0 + n1,
+//   m = (m0 + n0 (c0 - c)^T) + (m1 + n1 (c1 - c)^T), r = max(|c0 - c| + r0, |c1 - c| + r1)
+__global__ void k_sdf_wn_moments(const float4* __restrict__ tri, int n, const BvhNode* __restrict__ nodes,
+                                 const int* __restrict__ parent, int* __restrict__ arrived, WnNode* mom) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    int p = parent[n - 1 + k];
+    while (p >= 0) {
+        __threadfence();
+        if (atomicAdd(&arrived[p], 1) == 0) return;
+        __threadfence();
+        const WnNode X = child_moments(tri, mom, nodes[p].child[0]);
+        const WnNode Y = child_moments(tri, mom, nodes[p].child[1]);
+        WnNode Z;
+        Z.area = dadd(X.area, Y.area);
+        const double wx = Z.area > 0.0 ? X.area / Z.area : 0.5, wy = Z.area > 0.0 ? Y.area / Z.area : 0.5;
+        double dx[3], dy[3];
+#pragma unroll
+        for (int d = 0; d < 3; ++d) {
+            Z.c[d] = dadd(dmul(wx, X.c[d]), dmul(wy, Y.c[d]));
+            Z.n[d] = dadd(X.n[d], Y.n[d]);
+            dx[d] = dsub(X.c[d], Z.c[d]);
+            dy[d] = dsub(Y.c[d], Z.c[d]);
+        }
+#pragma unroll
+        for (int i = 0; i < 3; ++i)
+#pragma unroll
+            for (int j = 0; j < 3; ++j)
+                Z.m[3 * i + j] = dadd(dadd(X.m[3 * i + j], dmul(X.n[i], dx[j])), dadd(Y.m[3 * i + j], dmul(Y.n[i], dy[j])));
+        const double ex = sqrt(dadd(dadd(dmul(dx[0], dx[0]), dmul(dx[1], dx[1])), dmul(dx[2], dx[2])));
+        const double ey = sqrt(dadd(dadd(dmul(dy[0], dy[0]), dmul(dy[1], dy[1])), dmul(dy[2], dy[2])));
+        Z.r = fmax(dadd(ex, X.r), dadd(ey, Y.r));
+        Z.pad = 0.0;
+        double2* dst = reinterpret_cast<double2*>(mom + p);
+        const double2* src = reinterpret_cast<const double2*>(&Z);
+#pragma unroll
+        for (int t = 0; t < 9; ++t) __stcg(dst + t, src[t]);
+        p = parent[p];
+    }
+}
+
+// far-field solid angle of node `node` seen from p when |p - c| > WN_BETA r (returns true and adds it to acc): with
+// x = c - p, sum_f a_f . G(c_f) for G(y) = (y - p) / |y - p|^3 to first order around c,
+//   n . x / |x|^3 + tr(m) / |x|^3 - 3 x^T m x / |x|^5
+__device__ __forceinline__ bool far_field(const WnNode* __restrict__ mom, int node, D3 p, double& acc) {
+    const double2* q = reinterpret_cast<const double2*>(mom + node);
+    const double2 c01 = __ldg(q), c2r = __ldg(q + 1);
+    const D3 x = {dsub(c01.x, p.x), dsub(c01.y, p.y), dsub(c2r.x, p.z)};
+    const double d2 = dot3(x, x);
+    if (!(d2 > WN_BETA * WN_BETA * c2r.y * c2r.y)) return false;
+    const double2 n01 = __ldg(q + 2), n2a = __ldg(q + 3), m01 = __ldg(q + 4), m23 = __ldg(q + 5), m45 = __ldg(q + 6),
+                  m67 = __ldg(q + 7), m8p = __ldg(q + 8);
+    const D3 nv = {n01.x, n01.y, n2a.x};
+    const double m[9] = {m01.x, m01.y, m23.x, m23.y, m45.x, m45.y, m67.x, m67.y, m8p.x};
+    const double d = sqrt(d2);
+    const double i3 = 1.0 / dmul(d2, d), i5 = i3 / d2;
+    const double mx0 = dadd(dadd(dmul(m[0], x.x), dmul(m[1], x.y)), dmul(m[2], x.z));
+    const double mx1 = dadd(dadd(dmul(m[3], x.x), dmul(m[4], x.y)), dmul(m[5], x.z));
+    const double mx2 = dadd(dadd(dmul(m[6], x.x), dmul(m[7], x.y)), dmul(m[8], x.z));
+    const double xmx = dadd(dadd(dmul(x.x, mx0), dmul(x.y, mx1)), dmul(x.z, mx2));
+    const double nx = dadd(dadd(dmul(nv.x, x.x), dmul(nv.y, x.y)), dmul(nv.z, x.z));
+    const double tr = dadd(dadd(m[0], m[4]), m[8]);
+    acc = dadd(acc, dsub(dmul(dadd(nx, tr), i3), dmul(3.0, dmul(xmx, i5))));
+    return true;
+}
+
+// generalised winding number, BVH mode: one thread per point in Morton order; the tree fixes the visit order (child 0
+// before child 1), so the sum is bitwise reproducible.  SIGN: out[q] = +1 where |w| >= 1/2 (decided in fp64), else -1;
+// otherwise out[q] = w rounded to fp32
+template <bool SIGN>
+__global__ void __launch_bounds__(SDF_BLOCK)
+k_sdf_winding_bvh(const float4* __restrict__ tri, const BvhNode* __restrict__ nodes, const WnNode* __restrict__ mom, int F,
+                  const float* __restrict__ pts, const uint32_t* __restrict__ order, int64_t P, float* __restrict__ out) {
+    __shared__ int s_node[SDF_STACK][SDF_BLOCK];
+    const int64_t i = blockIdx.x * (int64_t)SDF_BLOCK + threadIdx.x;
+    if (i >= P) return;
+    const int tid = threadIdx.x;
+    const int64_t q = order[i];
+    const D3 p = {(double)pts[3 * q], (double)pts[3 * q + 1], (double)pts[3 * q + 2]};
+    double acc = 0.0;
+    if (F == 1) {
+        acc = solid_angle(p, tri[0], tri[1], tri[2]);
+    } else if (!far_field(mom, 0, p, acc)) {
+        int sp = 0, node = 0;
+        for (;;) {
+            const int2 c = __ldg(reinterpret_cast<const int2*>(&nodes[node].child[0]));
+            bool go[2] = {false, false};
+#pragma unroll
+            for (int s = 0; s < 2; ++s) {
+                const int ch = s == 0 ? c.x : c.y;
+                if (ch < 0) {
+                    const int t = ~ch;
+                    acc = dadd(acc, solid_angle(p, tri[3 * t], tri[3 * t + 1], tri[3 * t + 2]));
+                } else {
+                    go[s] = !far_field(mom, ch, p, acc);
+                }
+            }
+            if (go[0] && go[1]) {
+                s_node[sp++][tid] = c.y;
+                node = c.x;
+            } else if (go[0] || go[1]) {
+                node = go[0] ? c.x : c.y;
+            } else if (sp > 0) {
+                node = s_node[--sp][tid];
+            } else {
+                break;
+            }
+        }
+    }
+    const double w = dmul(acc, WN_INV_4PI);
+    out[q] = SIGN ? (fabs(w) >= 0.5 ? 1.f : -1.f) : (float)w;
+}
+
+// generalised winding number, exact: every face in face order (shared-memory tiles), fp64 sum; the reference for the
+// BVH mode.  SIGN as k_sdf_winding_bvh
+template <bool SIGN>
+__global__ void __launch_bounds__(SDF_BLOCK)
+k_sdf_winding_brute(const float4* __restrict__ tri, int F, const float* __restrict__ pts, int64_t P, float* __restrict__ out) {
+    __shared__ float4 s_tri[3 * SDF_TILE];
+    const int64_t i = blockIdx.x * (int64_t)SDF_BLOCK + threadIdx.x;
+    const bool valid = i < P;
+    const D3 p = {valid ? (double)pts[3 * i] : 0.0, valid ? (double)pts[3 * i + 1] : 0.0, valid ? (double)pts[3 * i + 2] : 0.0};
+    double acc = 0.0;
+    for (int base = 0; base < F; base += SDF_TILE) {
+        const int nt = min(SDF_TILE, F - base);
+        __syncthreads();
+        for (int k = threadIdx.x; k < 3 * nt; k += SDF_BLOCK) s_tri[k] = tri[3 * (int64_t)base + k];
+        __syncthreads();
+        if (!valid) continue;
+#pragma unroll 1
+        for (int t = 0; t < nt; ++t) acc = dadd(acc, solid_angle(p, s_tri[3 * t], s_tri[3 * t + 1], s_tri[3 * t + 2]));
+    }
+    if (!valid) return;
+    const double w = dmul(acc, WN_INV_4PI);
+    out[i] = SIGN ? (fabs(w) >= 0.5 ? 1.f : -1.f) : (float)w;
 }
 
 __global__ void k_sdf_init(uint32_t* __restrict__ mm, unsigned long long* __restrict__ bad) {
@@ -667,10 +910,28 @@ int validate(const char* fn, cudaStream_t st, unsigned long long* bad, const flo
     return DS_OK;
 }
 
-// ds_mesh_sdf and ds_mesh_sdf_nearest: face_out == NULL runs the non-recording kernels
+// what mesh_sdf_impl computes: the signed distance with the ray-parity sign, the signed distance with the winding-number
+// sign, or the winding number alone (into sdf_out)
+enum SdfJob { SDF_PARITY, SDF_WINDING, SDF_WINDING_NUMBER };
+
+// the query kernel of a job: face_out == NULL runs the non-recording instantiations
+template <bool WIND>
+void launch_query(bool bvh, cudaStream_t st, const float4* tri, const BvhNode* nodes, int F, const float* points,
+                  const uint32_t* porder, int64_t P, float* sdf_out, int32_t* face_out) {
+    if (bvh && face_out)
+        k_sdf_query_bvh<true, WIND><<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, nodes, F, points, porder, P, sdf_out, face_out);
+    else if (bvh)
+        k_sdf_query_bvh<false, WIND><<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, nodes, F, points, porder, P, sdf_out, nullptr);
+    else if (face_out)
+        k_sdf_query_brute<true, WIND><<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, F, points, P, sdf_out, face_out);
+    else
+        k_sdf_query_brute<false, WIND><<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, F, points, P, sdf_out, nullptr);
+}
+
+// ds_mesh_sdf, ds_mesh_sdf_nearest, ds_mesh_sdf_winding and ds_mesh_winding_number
 int mesh_sdf_impl(const char* fn, ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F,
                   const float* points, int64_t P, int mode, float* sdf_out, int32_t* face_out, bool want_face,
-                  void* stream) {
+                  SdfJob job, void* stream) {
     DS_TRY(check_sizes(fn, ws, tri_verts, V, faces, F, P));
     DS_REQUIRE(mode == 0 || mode == 1, "%s: unknown mode %d (0 = BVH, 1 = brute force)", fn, mode);
     if (P == 0) return DS_OK;
@@ -680,7 +941,8 @@ int mesh_sdf_impl(const char* fn, ds_workspace* ws, const float* tri_verts, int6
     size_t sort_tmp = 0;
     DS_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, sort_tmp, (uint32_t*)nullptr, (uint32_t*)nullptr, (uint32_t*)nullptr,
                                             (uint32_t*)nullptr, (int)nmax, 0, 30, st));
-    const size_t need = (size_t)F * (12 + 16 + 48 + 64 + 12) + (size_t)P * 16 + sort_tmp + (1 << 16);
+    const size_t need = (size_t)F * (12 + 16 + 48 + 64 + 12 + (job == SDF_PARITY ? 0 : sizeof(WnNode))) + (size_t)P * 16 +
+                        sort_tmp + (1 << 16);
     DS_TRY(ws->arena.reserve(need, st));
     Arena& a = ws->arena;
     uint32_t* mm = a.take<uint32_t>(24);
@@ -694,14 +956,26 @@ int mesh_sdf_impl(const char* fn, ds_workspace* ws, const float* tri_verts, int6
     if (mode == 1) {
         {
             ProfScope prof(PROF_SDF_BUILD, st);
-            k_sdf_gather<<<nblk(F, 256), 256, 0, st>>>(tri_verts, faces, nullptr, F, tri);
+            if (job == SDF_PARITY)
+                k_sdf_gather<false><<<nblk(F, 256), 256, 0, st>>>(tri_verts, faces, nullptr, F, tri);
+            else
+                k_sdf_gather<true><<<nblk(F, 256), 256, 0, st>>>(tri_verts, faces, nullptr, F, tri);
             DS_LAUNCH_CHECK();
         }
+        if (job != SDF_PARITY) {
+            ProfScope prof(PROF_SDF_WINDING, st);
+            if (job == SDF_WINDING)
+                k_sdf_winding_brute<true><<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, (int)F, points, P, sdf_out);
+            else
+                k_sdf_winding_brute<false><<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, (int)F, points, P, sdf_out);
+            DS_LAUNCH_CHECK();
+            if (job == SDF_WINDING_NUMBER) return DS_OK;
+        }
         ProfScope prof(PROF_SDF_QUERY, st);
-        if (face_out)
-            k_sdf_query_brute<true><<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, (int)F, points, P, sdf_out, face_out);
+        if (job == SDF_WINDING)
+            launch_query<true>(false, st, tri, nullptr, (int)F, points, nullptr, P, sdf_out, face_out);
         else
-            k_sdf_query_brute<false><<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, (int)F, points, P, sdf_out, nullptr);
+            launch_query<false>(false, st, tri, nullptr, (int)F, points, nullptr, P, sdf_out, face_out);
         DS_LAUNCH_CHECK();
         return DS_OK;
     }
@@ -716,13 +990,17 @@ int mesh_sdf_impl(const char* fn, ds_workspace* ws, const float* tri_verts, int6
     int* parent = a.take<int>(2 * F);
     int* arrived = a.take<int>(F);
     void* scratch = a.take<char>(sort_tmp + 16);
-    DS_REQUIRE(cent && codes && codes2 && iota && order && porder && nodes && parent && arrived && scratch,
-               "%s: workspace arena exhausted", fn);
+    WnNode* mom = job == SDF_PARITY ? nullptr : a.take<WnNode>(F);
+    DS_REQUIRE(cent && codes && codes2 && iota && order && porder && nodes && parent && arrived && scratch &&
+               (mom || job == SDF_PARITY), "%s: workspace arena exhausted", fn);
     uint32_t *mm_v = mm, *mm_c = mm + 8, *mm_p = mm + 16;
     {
     ProfScope prof(PROF_SDF_BUILD, st);
     // triangles in Morton order of their centroids
-    k_sdf_centroids<<<nblk(F, 256), 256, 0, st>>>(tri_verts, faces, F, cent);
+    if (job == SDF_PARITY)
+        k_sdf_centroids<false><<<nblk(F, 256), 256, 0, st>>>(tri_verts, faces, F, cent);
+    else
+        k_sdf_centroids<true><<<nblk(F, 256), 256, 0, st>>>(tri_verts, faces, F, cent);
     DS_LAUNCH_CHECK();
     k_bbox<<<148, 256, 0, st>>>(cent, F, mm_c);
     DS_LAUNCH_CHECK();
@@ -734,7 +1012,10 @@ int mesh_sdf_impl(const char* fn, ds_workspace* ws, const float* tri_verts, int6
     DS_LAUNCH_CHECK();
     DS_CUDA(cub::DeviceRadixSort::SortPairs(scratch, sort_tmp, codes, codes2, iota, order, (int)F, 0, 30, st));
     count_launch();
-    k_sdf_gather<<<nblk(F, 256), 256, 0, st>>>(tri_verts, faces, order, F, tri);
+    if (job == SDF_PARITY)
+        k_sdf_gather<false><<<nblk(F, 256), 256, 0, st>>>(tri_verts, faces, order, F, tri);
+    else
+        k_sdf_gather<true><<<nblk(F, 256), 256, 0, st>>>(tri_verts, faces, order, F, tri);
     DS_LAUNCH_CHECK();
     if (F > 1) {
         DS_CUDA(cudaMemsetAsync(arrived, 0, (size_t)F * sizeof(int), st));
@@ -744,18 +1025,36 @@ int mesh_sdf_impl(const char* fn, ds_workspace* ws, const float* tri_verts, int6
         DS_LAUNCH_CHECK();
     }
     }
-    // queries in Morton order of the points
+    // queries in Morton order of the points (for the winding jobs the point order is part of the winding stage)
+    auto point_order = [&]() -> int {
+        k_morton_codes<<<nblk(P, 256), 256, 0, st>>>(points, P, mm_p, codes, iota);
+        DS_LAUNCH_CHECK();
+        DS_CUDA(cub::DeviceRadixSort::SortPairs(scratch, sort_tmp, codes, codes2, iota, porder, (int)P, 0, 30, st));
+        count_launch();
+        return DS_OK;
+    };
+    if (job != SDF_PARITY) {
+        ProfScope prof(PROF_SDF_WINDING, st);
+        if (F > 1) {
+            DS_CUDA(cudaMemsetAsync(arrived, 0, (size_t)F * sizeof(int), st));
+            k_sdf_wn_moments<<<nblk(F, 256), 256, 0, st>>>(tri, (int)F, nodes, parent, arrived, mom);
+            DS_LAUNCH_CHECK();
+        }
+        DS_TRY(point_order());
+        if (job == SDF_WINDING)
+            k_sdf_winding_bvh<true><<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, nodes, mom, (int)F, points, porder, P, sdf_out);
+        else
+            k_sdf_winding_bvh<false><<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, nodes, mom, (int)F, points, porder, P, sdf_out);
+        DS_LAUNCH_CHECK();
+        if (job == SDF_WINDING_NUMBER) return DS_OK;
+    }
     ProfScope prof(PROF_SDF_QUERY, st);
-    k_morton_codes<<<nblk(P, 256), 256, 0, st>>>(points, P, mm_p, codes, iota);
-    DS_LAUNCH_CHECK();
-    DS_CUDA(cub::DeviceRadixSort::SortPairs(scratch, sort_tmp, codes, codes2, iota, porder, (int)P, 0, 30, st));
-    count_launch();
-    if (face_out)
-        k_sdf_query_bvh<true><<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, nodes, (int)F, points, porder, P, sdf_out,
-                                                                         face_out);
-    else
-        k_sdf_query_bvh<false><<<nblk(P, SDF_BLOCK), SDF_BLOCK, 0, st>>>(tri, nodes, (int)F, points, porder, P, sdf_out,
-                                                                          nullptr);
+    if (job == SDF_PARITY) {
+        DS_TRY(point_order());
+        launch_query<false>(true, st, tri, nodes, (int)F, points, porder, P, sdf_out, face_out);
+    } else {
+        launch_query<true>(true, st, tri, nodes, (int)F, points, porder, P, sdf_out, face_out);
+    }
     DS_LAUNCH_CHECK();
     return DS_OK;
 }
@@ -764,14 +1063,28 @@ int mesh_sdf_impl(const char* fn, ds_workspace* ws, const float* tri_verts, int6
 
 extern "C" int ds_mesh_sdf(ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F,
                            const float* points, int64_t P, int mode, float* sdf_out, void* stream) {
-    return mesh_sdf_impl("ds_mesh_sdf", ws, tri_verts, V, faces, F, points, P, mode, sdf_out, nullptr, false, stream);
+    return mesh_sdf_impl("ds_mesh_sdf", ws, tri_verts, V, faces, F, points, P, mode, sdf_out, nullptr, false, SDF_PARITY,
+                         stream);
 }
 
 extern "C" int ds_mesh_sdf_nearest(ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F,
                                    const float* points, int64_t P, int mode, float* sdf_out, int32_t* face_out,
                                    void* stream) {
     return mesh_sdf_impl("ds_mesh_sdf_nearest", ws, tri_verts, V, faces, F, points, P, mode, sdf_out, face_out, true,
-                         stream);
+                         SDF_PARITY, stream);
+}
+
+extern "C" int ds_mesh_winding_number(ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F,
+                                      const float* points, int64_t P, int mode, float* w_out, void* stream) {
+    return mesh_sdf_impl("ds_mesh_winding_number", ws, tri_verts, V, faces, F, points, P, mode, w_out, nullptr, false,
+                         SDF_WINDING_NUMBER, stream);
+}
+
+extern "C" int ds_mesh_sdf_winding(ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F,
+                                   const float* points, int64_t P, int mode, float* sdf_out, int32_t* face_out,
+                                   void* stream) {
+    return mesh_sdf_impl("ds_mesh_sdf_winding", ws, tri_verts, V, faces, F, points, P, mode, sdf_out, face_out, false,
+                         SDF_WINDING, stream);
 }
 
 extern "C" int ds_mesh_sdf_backward(ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F,

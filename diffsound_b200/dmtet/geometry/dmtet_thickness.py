@@ -17,7 +17,8 @@ positions are bit-identical and autograd reaches the thickness parameter.
 `RaycastingScene` (dmtet_thickness.py:301-314; SURVEY.md section 8f-4); `apply_sdf` also takes the sampled values (a
 tensor) or a callable evaluated at the grid vertices.  `apply_sdf((verts, faces))` takes the triangle mesh as tensors and
 samples it through the differentiable `mesh_sdf` (mesh_sdf.py): with `verts.requires_grad` the mesh is sampled again on
-every `getMesh()`, so the loss of a `tick()` reaches the triangle-mesh vertices.  Not reproduced: the renderer's `mesh.Mesh` container
+every `getMesh()`, so the loss of a `tick()` reaches the triangle-mesh vertices.  `apply_sdf(..., sign="winding")` takes
+the sign from the generalised winding number instead of the ray parity (open or self-intersecting meshes).  Not reproduced: the renderer's `mesh.Mesh` container
 (return_triangle=True) is replaced by a plain namespace with `v_pos` / `t_pos_idx`.
 """
 import os
@@ -122,7 +123,7 @@ class DMTetGeometry(torch.nn.Module):
         self.indices = torch.tensor(np.asarray(grid[1]), dtype=torch.long, device=dev)
         self.generate_edges()
         self.sdf = torch.zeros_like(self.verts[:, 0])
-        self._sdf_mesh = None       # (verts, faces) of apply_sdf((verts, faces)) when verts requires grad
+        self._sdf_mesh = None       # (verts, faces, sign) of apply_sdf((verts, faces), sign) when verts requires grad
 
     def generate_edges(self):
         """`all_edges` (unique sorted vertex pairs of the background grid, dmtet_thickness.py:225-230) is only read by the
@@ -172,7 +173,7 @@ class DMTetGeometry(torch.nn.Module):
             self.writer.add_scalar("thickness", self.marching_tets.thickness_coef().item(), it)
         return audio_loss
 
-    def apply_sdf(self, sdf):
+    def apply_sdf(self, sdf, sign="parity"):
         """`sdf`: path of a triangle mesh (OBJ), tensor of signed distances at `self.verts`, or a callable verts -> tensor.
         Signed distances are positive inside, the sign convention `apply_sdf` of the reference produces
         (dmtet_thickness.py:312).  A path is read with `read_obj` and sampled at `self.verts` by `native.mesh_sdf`: exact
@@ -180,27 +181,36 @@ class DMTetGeometry(torch.nn.Module):
         used as given, in its own coordinates, with no rescaling or recentring.
         `sdf` = (verts (V, 3), faces (F, 3)) tensors: the triangle mesh, sampled by the differentiable `mesh_sdf`.  If
         verts.requires_grad, the geometry keeps the mesh and every `getMesh()` samples it again (and resets
-        `max_thickness`), so each `tick()` builds a fresh graph down to verts; otherwise it is sampled once, like a path."""
+        `max_thickness`), so each `tick()` builds a fresh graph down to verts; otherwise it is sampled once, like a path.
+        `sign` (path and mesh forms): "parity", the ray-crossing parity, right for closed meshes that do not cross
+        themselves whatever their face orientation; or "winding", inside where the generalised winding number |w| >= 1/2,
+        for meshes with holes or cracks and for surfaces folded through themselves (their overlap stays solid), which
+        needs consistently oriented faces.  A tensor or callable `sdf` takes only "parity"."""
+        is_mesh = isinstance(sdf, (tuple, list)) and len(sdf) == 2
+        is_path = isinstance(sdf, (str, os.PathLike))
+        if native._sdf_sign(sign) and not (is_mesh or is_path):
+            raise ValueError("apply_sdf: sign='winding' needs a triangle mesh (a path or (verts, faces)), not sampled values")
         self._sdf_mesh = None
-        if isinstance(sdf, (tuple, list)) and len(sdf) == 2:
+        if is_mesh:
             verts, faces = sdf
             dev = self.verts.device
             verts = torch.as_tensor(verts, device=dev)
             faces = torch.as_tensor(faces, device=dev).to(torch.int64)
             if verts.requires_grad:
-                self._sdf_mesh = (verts, faces)
-            self._sample_mesh(verts, faces)
+                self._sdf_mesh = (verts, faces, sign)
+            self._sample_mesh(verts, faces, sign)
             return
-        if isinstance(sdf, (str, os.PathLike)):
+        if is_path:
             v, f = read_obj(sdf)
             dev = self.verts.device
-            sdf = native.mesh_sdf(torch.from_numpy(v).to(dev), torch.from_numpy(f).to(dev), self.verts.contiguous())
+            sdf = native.mesh_sdf(torch.from_numpy(v).to(dev), torch.from_numpy(f).to(dev), self.verts.contiguous(),
+                                  sign=sign)
         values = sdf(self.verts) if callable(sdf) else sdf
         self.sdf = torch.as_tensor(values, dtype=torch.float32).to(self.verts.device).reshape(-1)
         self.marching_tets.max_thickness = self.sdf.max()
 
-    def _sample_mesh(self, verts, faces):
-        self.sdf = mesh_sdf(verts, faces, self.verts.contiguous())
+    def _sample_mesh(self, verts, faces, sign):
+        self.sdf = mesh_sdf(verts, faces, self.verts.contiguous(), sign=sign)
         self.marching_tets.max_thickness = self.sdf.max()
 
     def parameters(self):

@@ -775,15 +775,25 @@ def largest_tet_component(tets, n_verts):
     return int(counts[0]), kept, tout, labels
 
 
-def mesh_sdf(tri_verts, faces, points, brute_force=False):
+def _sdf_sign(sign):
+    if sign not in ("parity", "winding"):
+        raise ValueError(f"sign must be 'parity' or 'winding', not {sign!r}")
+    return sign == "winding"
+
+
+def mesh_sdf(tri_verts, faces, points, brute_force=False, sign="parity"):
     """Signed distance from each query point to a triangle mesh (ds_mesh_sdf): positive inside, negative outside, 0 on the
     surface; the mesh is used in its own coordinates.  tri_verts (V, 3) fp32, faces (F, 3) int64, points (P, 3) fp32, all
     on one device; returns (P,) fp32.  brute_force: every point against every face instead of the BVH (the test
-    reference; the outputs are bitwise equal)."""
+    reference; the outputs are bitwise equal).  sign: "parity" (ray-crossing parity: closed meshes that do not cross
+    themselves, any face orientation) or "winding" (ds_mesh_sdf_winding: inside where the generalised winding number
+    |w| >= 1/2; open, cracked and self-intersecting meshes whose faces are consistently oriented; same distances)."""
     lib = _lib.load()
     assert tri_verts.dtype == torch.float32 and faces.dtype == torch.int64 and points.dtype == torch.float32
     assert tri_verts.dim() == 2 and tri_verts.shape[1] == 3 and faces.dim() == 2 and faces.shape[1] == 3
     assert points.dim() == 2 and points.shape[1] == 3
+    if _sdf_sign(sign):
+        return mesh_sdf_nearest(tri_verts, faces, points, brute_force, sign, want_face=False)[0]
     dev = points.device
     ws = workspace(dev)
     out = torch.empty(points.shape[0], dtype=torch.float32, device=dev)
@@ -793,26 +803,46 @@ def mesh_sdf(tri_verts, faces, points, brute_force=False):
     return out
 
 
+def mesh_winding_number(tri_verts, faces, points, brute_force=False):
+    """Generalised winding number of a triangle mesh at each query point (ds_mesh_winding_number): 1 inside and 0 outside
+    a closed, outward-oriented surface, 2 where two overlap, smooth across holes.  Arguments as `mesh_sdf`; returns (P,)
+    fp32.  brute_force: the exact fp64 sum over all faces; otherwise the BVH with far-field expansions, whose error is
+    measured, not bounded (at most 0.024 on the test meshes; it grows with the face area packed inside a subtree)."""
+    lib = _lib.load()
+    _check_mesh(tri_verts, faces, points)
+    dev = points.device
+    ws = workspace(dev)
+    out = torch.empty(points.shape[0], dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.ds_mesh_winding_number(ws.handle, _p(tri_verts), tri_verts.shape[0], _p(faces), faces.shape[0],
+                                              _p(points), points.shape[0], int(bool(brute_force)), _p(out), _stream()),
+                   "ds_mesh_winding_number")
+    return out
+
+
 def _check_mesh(tri_verts, faces, points):
     assert tri_verts.dtype == torch.float32 and faces.dtype == torch.int64 and points.dtype == torch.float32
     assert tri_verts.dim() == 2 and tri_verts.shape[1] == 3 and faces.dim() == 2 and faces.shape[1] == 3
     assert points.dim() == 2 and points.shape[1] == 3
 
 
-def mesh_sdf_nearest(tri_verts, faces, points, brute_force=False):
-    """`mesh_sdf` and the nearest face of each point (ds_mesh_sdf_nearest): returns (sdf (P,) fp32, face (P,) int32).
-    sdf is bitwise equal to `mesh_sdf`; of faces at exactly the same distance, the lowest index (both modes)."""
+def mesh_sdf_nearest(tri_verts, faces, points, brute_force=False, sign="parity", want_face=True):
+    """`mesh_sdf` and the nearest face of each point (ds_mesh_sdf_nearest, or ds_mesh_sdf_winding for sign="winding"):
+    returns (sdf (P,) fp32, face (P,) int32, None when not want_face).  sdf is bitwise equal to `mesh_sdf` with the same
+    sign; of faces at exactly the same distance, the lowest index (both modes and both signs)."""
     lib = _lib.load()
     _check_mesh(tri_verts, faces, points)
+    winding = _sdf_sign(sign)
     dev = points.device
     ws = workspace(dev)
     out = torch.empty(points.shape[0], dtype=torch.float32, device=dev)
-    face = torch.empty(points.shape[0], dtype=torch.int32, device=dev)
+    face = torch.empty(points.shape[0], dtype=torch.int32, device=dev) if want_face or not winding else None
+    fn = lib.ds_mesh_sdf_winding if winding else lib.ds_mesh_sdf_nearest
+    name = "ds_mesh_sdf_winding" if winding else "ds_mesh_sdf_nearest"
     with torch.cuda.device(dev):
-        _lib.check(lib.ds_mesh_sdf_nearest(ws.handle, _p(tri_verts), tri_verts.shape[0], _p(faces), faces.shape[0],
-                                           _p(points), points.shape[0], int(bool(brute_force)), _p(out), _p(face),
-                                           _stream()), "ds_mesh_sdf_nearest")
-    return out, face
+        _lib.check(fn(ws.handle, _p(tri_verts), tri_verts.shape[0], _p(faces), faces.shape[0], _p(points), points.shape[0],
+                      int(bool(brute_force)), _p(out), _p(face), _stream()), name)
+    return out, (face if want_face else None)
 
 
 def mesh_sdf_backward(tri_verts, faces, points, face, sdf, grad_sdf, want_verts=True, want_points=True):

@@ -450,6 +450,26 @@ int ds_mesh_sdf_nearest(ds_workspace* ws, const float* tri_verts, int64_t V, con
 int ds_mesh_sdf_backward(ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F,
                          const float* points, int64_t P, const int32_t* face, const float* sdf, const float* grad_sdf,
                          float* grad_verts, float* grad_points, void* stream);
+/* Generalised winding number w(p) = sum over faces of the oriented solid angle / 4 pi (Jacobson, Kavan & Sorkine-Hornung
+ * 2013): 1 inside and 0 outside a closed surface whose faces are consistently oriented with outward normals (-1 / 0 when
+ * they all point inward), 2 where two such surfaces overlap, and a smooth value between across holes.  Degenerate faces
+ * contribute 0.  w_out fp32 [P].  mode 1 = exact: the fp64 sum over all faces in face order (Van Oosterom-Strackee solid
+ * angles), rounded once.  mode 0 = BVH over the faces (a radix tree on the centroids of the sorted corners), with subtrees
+ * far from the point replaced by their far-field expansion (Barill et al. 2018, through the first moment, acceptance
+ * |p - centroid| > 3 x the subtree's radius).  Its error is measured, not bounded: at most 0.024 on the test meshes, whose
+ * bar is 0.05; it grows with the face area packed inside a subtree (many stacked or crumpled layers).  Both modes are
+ * bitwise reproducible; flipping every face gives exactly -w, and neither the first corner written nor vertex sharing
+ * changes the result.  Same checks and synchronisation as ds_mesh_sdf. */
+int ds_mesh_winding_number(ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F,
+                           const float* points, int64_t P, int mode, float* w_out, void* stream);
+/* ds_mesh_sdf with the sign of the winding number: inside (+) where |w| >= 1/2 (decided in fp64 from the w of
+ * ds_mesh_winding_number in the same mode), so the overlap of a self-intersecting surface stays inside and holes do not
+ * streak the sign.  Needs consistently oriented faces (either way round); for inconsistently oriented meshes the ray
+ * parity of ds_mesh_sdf is the right rule.  |sdf_out| and face_out are bitwise those of ds_mesh_sdf_nearest (same
+ * search, tie rule and ids), a point at distance 0 gives +0.  face_out int32 [P] may be NULL.  Same checks and
+ * synchronisation as ds_mesh_sdf. */
+int ds_mesh_sdf_winding(ds_workspace* ws, const float* tri_verts, int64_t V, const int64_t* faces, int64_t F,
+                        const float* points, int64_t P, int mode, float* sdf_out, int32_t* face_out, void* stream);
 
 /* ---- device-side timing per kernel class ---------------------------------------
  * Replaces the reference's opt-in torch.profiler hook of lobpcg (src/lobpcg/_lobpcg.py:357-369)
