@@ -119,6 +119,12 @@ SIGNATURES = {
     "ds_stuff_edges_fill": (cint, [ptr, ptr, i64p, i64p, ptr]),
     "ds_stuff_count": (cint, [ptr, ptr, i64, i64, i64, C.POINTER(C.c_double), dbl, i64p, f64p, i64, C.POINTER(C.c_int64), ptr]),
     "ds_stuff_fill": (cint, [ptr, ptr, i64p, f64p, i64p, f32p, ptr]),
+    "ds_tet_boundary_count": (cint, [ptr, f32p, i64, i32p, i64, cint, C.POINTER(C.c_int64), ptr]),
+    "ds_tet_boundary_fill": (cint, [ptr, i32p, i32p, i32p, ptr]),
+    "ds_modal_gains": (cint, [ptr, f32p, i64, i32p, i64, cint, i32p, i32p, i32p, i64, f32p, i32p, f32p, i64, f64p, i64, cint,
+                              f32p, f32p, ptr]),
+    "ds_modal_gains_backward": (cint, [ptr, f32p, i64, i32p, i64, cint, i32p, i32p, i32p, i64, f32p, i32p, f32p, i64, f64p,
+                                       i64, cint, f32p, f32p, f32p, ptr]),
     "ds_lobpcg_residual": (cint, [f64p, f64p, i64, cint, i64, f64p, f64p, i64, f64p, f64p, ptr]),
     "ds_gather_cols_f32": (cint, [f64p, i64, C.POINTER(C.c_int), cint, cint, i64, f32p, ptr]),
     "ds_widen_f32": (cint, [f32p, cint, i64, f64p, i64, ptr]),

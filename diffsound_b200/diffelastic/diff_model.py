@@ -22,7 +22,7 @@ import torch
 import torch.nn as nn
 
 from .. import native
-from ..ddsp.oscillator import WeightedParam
+from ..ddsp.oscillator import WeightedParam, modal_synth
 from .deform import Deform
 from .mass_matrix import get_elememt_mass_matrix  # noqa: F401  (re-exported like the reference)
 from .material_model import Material, MatSet
@@ -203,6 +203,33 @@ class _StiffFunc(torch.autograd.Function):
         return gx, gmu, gla, None
 
 
+class _ModalGains(torch.autograd.Function):
+    """g[p, m] = d_p . u_m(closest(p)) on the boundary face `face[p]` (native.modal_gains).  Differentiable in the points
+    and the directions only: the mode shapes and the mesh are constants here."""
+
+    @staticmethod
+    def forward(ctx, points, directions, obj, face):
+        d = obj.deform
+        pts = points.detach().to(torch.float32).contiguous()
+        dirs = None if directions is None else directions.detach().to(torch.float32).contiguous()
+        g, closest = native.modal_gains(obj._verts32, d.tets_i32, obj.tetmesh.order, obj._boundary(), pts,
+                                        face, dirs, obj.U_hat)
+        obj.last_strike_points = closest
+        ctx.obj, ctx.U = obj, obj.U_hat
+        ctx.save_for_backward(pts, face, dirs)
+        ctx.dtypes = (points.dtype, None if directions is None else directions.dtype)
+        return g
+
+    @staticmethod
+    def backward(ctx, grad):
+        pts, face, dirs = ctx.saved_tensors
+        obj = ctx.obj
+        gp, gd = native.modal_gains_backward(obj._verts32, obj.deform.tets_i32, obj.tetmesh.order,
+                                             obj._boundary(), pts, face, dirs, ctx.U,
+                                             grad.to(torch.float32).contiguous())
+        return gp.to(ctx.dtypes[0]), (None if gd is None else gd.to(ctx.dtypes[1])), None, None
+
+
 class DiffSoundObj:
     #: options of the eigensolver (see ds_lobpcg_opts in include/diffsound_sm100.h)
     # relative residual ||K u - lam M u|| / (lam ||M u||).  Eigenvalue error ~ tol^2, eigenvector (and
@@ -252,6 +279,7 @@ class DiffSoundObj:
         self._warm = []
         self._q = None
         self.eig_stats = None
+        self.last_strike_points = None
 
     # ------------------------------------------------------------------ parameters
     def parameters(self):
@@ -516,3 +544,75 @@ class DiffSoundObj:
         """(mode_num, 1) fp32 eigenvalues, differentiable w.r.t. the vertex positions
         (diff_model.py:390-399)."""
         return _EigvalShape.apply(self.tetmesh.vertices, self)
+
+    # ------------------------------------------------------------------ striking the object
+    def _boundary(self):
+        """(faces, owner, local) int32 of native.tet_boundary, cached per object."""
+        if "_bnd" not in self.__dict__:
+            d = self.deform
+            self._bnd = native.tet_boundary(d.verts_f32(), d.tets_i32, self.tetmesh.order)
+        return self._bnd
+
+    def surface(self):
+        """Boundary triangles of the tet mesh, cached: (faces (F, 3) int64 corner node ids into tetmesh.vertices, oriented
+        outward; owner (F,) int64 tet; local (F,) int64 the tet corner opposite the face), in ascending order of the sorted
+        corner triple (native.tet_boundary)."""
+        if "_surface" not in self.__dict__:
+            self._surface = tuple(x.long() for x in self._boundary())
+        return self._surface
+
+    def modal_gains(self, points, directions=None):
+        """(P, mode_num) fp32 gains g[p, m] = d_p . u_m(x_p) of the mode_num modes of U_hat (the rigid six excluded): what
+        a unit impulse at surface point x_p in direction d_p puts into each mass-normalised mode.  points (P, 3) are put
+        on the surface first: x_p is the closest point of the nearest boundary face (native.mesh_sdf_nearest over the
+        corner-node boundary faces; of faces at the same distance the lowest index) and is kept in
+        `last_strike_points`.  directions (P, 3) default to the outward unit normal of that face; they are used as
+        given (not normalised).
+
+        Differentiable in `points` (along the surface: the normal component of the gradient is 0) and `directions`.
+        The mode shapes and the mesh are constants here: no gradient reaches the vertices or the material through a
+        gain.  Raises if eigen_decomposition() has not run."""
+        if getattr(self, "U_hat", None) is None:
+            raise RuntimeError("modal_gains: run eigen_decomposition() first")
+        dev = self.deform.device
+        points = points.reshape(-1, 3)
+        if directions is not None:
+            directions = directions.reshape(-1, 3)
+        pts = points.detach().to(device=dev, dtype=torch.float32).contiguous()
+        _, face = native.mesh_sdf_nearest(self._verts32, self.surface()[0], pts, want_face=True)
+        return _ModalGains.apply(points, directions, self, face)
+
+    def impulse_response(self, strike, sample_num, sr, pickup=None, strike_dir=None, pickup_dir=None, alpha=None,
+                         beta=None):
+        """(P, sample_num) fp32 displacement in metres per N s of impulse at the pickup point along pickup_dir, for a unit
+        impulse at the strike point along strike_dir (directions default to the outward surface normal):
+
+            y(t) = sum_m g_m(strike) g_m(pickup) / w_m exp(-c_m t) sin(w_m t),  c_m = (alpha + beta lambda_m) / 2,
+            w_m = sqrt(lambda_m - c_m^2),
+
+        sampled at t = (n + 1) / sr for n < sample_num (modal_synth's convention), with lambda = self.eigenvalues
+        (detached) and Rayleigh damping alpha, beta (default: the material's).  pickup
+        defaults to the strike point and direction (the driving-point response).  A mode with lambda_m <= c_m^2 is not
+        oscillatory (over-damped) and gets amplitude 0.  Rendered by modal_synth; differentiable in the points, the
+        directions, alpha and beta.  The product g_strike g_pickup makes the result independent of the sign of each
+        eigenvector, and strike and pickup swap exactly."""
+        dev = self.deform.device
+        mat = self.material_model.mat
+
+        def coef(x, default):
+            x = default if x is None else x
+            return (x if torch.is_tensor(x) else torch.tensor(float(x))).to(device=dev, dtype=torch.float64)
+
+        a, b = coef(alpha, mat.alpha), coef(beta, mat.beta)
+        lam = self.eigenvalues.detach()
+        c = 0.5 * (a + b * lam)
+        w2 = lam - c * c
+        osc = w2 > 0
+        omega = torch.sqrt(torch.where(osc, w2, torch.ones_like(w2)))
+        if pickup is None:
+            g_pick = g_strike = self.modal_gains(strike, strike_dir)
+        else:
+            g_pick = self.modal_gains(pickup, pickup_dir)
+            g_strike = self.modal_gains(strike, strike_dir)
+        amp = torch.where(osc, g_strike * g_pick / omega.float(), torch.zeros((), device=dev))
+        return modal_synth(amp, c.float(), (omega / (2 * np.pi)).float(), int(sample_num), float(sr))

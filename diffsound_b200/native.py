@@ -900,3 +900,67 @@ def stuff(signs, dims, origin, h, edges, t):
         pos = torch.empty(nv + edges.shape[0], 3, dtype=torch.float32, device=dev)
         _lib.check(lib.ds_stuff_fill(ws.handle, _p(signs), _p(edges), _p(t), _p(tets), _p(pos), _stream()), "ds_stuff_fill")
     return tets, pos, int(counts[1])
+
+
+def tet_boundary(verts_f32, tets_i32, order):
+    """Boundary triangles of a tet mesh (ds_tet_boundary_*): the faces that belong to exactly one tet, in ascending order
+    of their sorted corner triple.  verts (n, 3) fp32, tets (T, npe) int32 (corner local nodes of shape_func.CORNER_LOCAL).
+    Returns (faces (F, 3) int32 corner node ids oriented outward, owner (F,) int32 tet, local (F,) int32 the tet corner
+    opposite the face); bitwise reproducible, independent of tet order and corner rotation."""
+    lib = _lib.load()
+    assert verts_f32.dtype == torch.float32 and tets_i32.dtype == torch.int32 and tets_i32.dim() == 2
+    dev = verts_f32.device
+    ws = workspace(dev)
+    n = C.c_int64(0)
+    with torch.cuda.device(dev):
+        _lib.check(lib.ds_tet_boundary_count(ws.handle, _p(verts_f32), verts_f32.shape[0], _p(tets_i32), tets_i32.shape[0],
+                                             int(order), C.byref(n), _stream()), "ds_tet_boundary_count")
+        F = int(n.value)
+        faces = torch.empty(F, 3, dtype=torch.int32, device=dev)
+        owner = torch.empty(F, dtype=torch.int32, device=dev)
+        local = torch.empty(F, dtype=torch.int32, device=dev)
+        _lib.check(lib.ds_tet_boundary_fill(ws.handle, _p(faces), _p(owner), _p(local), _stream()), "ds_tet_boundary_fill")
+    return faces, owner, local
+
+
+def _gains_args(verts_f32, tets_i32, order, boundary, points, face, dirs, U):
+    faces, owner, local = boundary
+    assert verts_f32.dtype == torch.float32 and tets_i32.dtype == torch.int32 and points.dtype == torch.float32
+    assert faces.dtype == torch.int32 and owner.dtype == torch.int32 and local.dtype == torch.int32
+    assert face.dtype == torch.int32 and U.dtype == torch.float64 and points.dim() == 2 and points.shape[1] == 3
+    assert dirs is None or (dirs.dtype == torch.float32 and dirs.shape == points.shape)
+    up, ldu = _pv(U)
+    return (_p(verts_f32), verts_f32.shape[0], _p(tets_i32), tets_i32.shape[0], int(order), _p(faces), _p(owner), _p(local),
+            faces.shape[0], _p(points), _p(face), _p(dirs), points.shape[0], up, ldu, U.shape[1])
+
+
+def modal_gains(verts_f32, tets_i32, order, boundary, points, face, dirs, U):
+    """Gains of the modes U (n_dofs, k) fp64 row-major view (read in place) at points (P, 3) fp32 put on their boundary
+    faces face (P,) int32 of boundary = tet_boundary(...) (ds_modal_gains): g[p, m] = d_p . u_m(closest point), d_p =
+    dirs[p] (P, 3) fp32 or, for dirs None, the outward unit normal of the face.  Returns (gains (P, k) fp32, closest
+    points (P, 3) fp32)."""
+    lib = _lib.load()
+    args = _gains_args(verts_f32, tets_i32, order, boundary, points, face, dirs, U)
+    dev = points.device
+    ws = workspace(dev)
+    g = torch.empty(points.shape[0], U.shape[1], dtype=torch.float32, device=dev)
+    cp = torch.empty(points.shape[0], 3, dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.ds_modal_gains(ws.handle, *args, _p(g), _p(cp), _stream()), "ds_modal_gains")
+    return g, cp
+
+
+def modal_gains_backward(verts_f32, tets_i32, order, boundary, points, face, dirs, U, grad):
+    """Gradient of `modal_gains` (ds_modal_gains_backward) given the upstream gradient (P, k) fp32: returns
+    (grad_points (P, 3), grad_dirs (P, 3) or None when dirs is None), fp32, bitwise reproducible."""
+    lib = _lib.load()
+    args = _gains_args(verts_f32, tets_i32, order, boundary, points, face, dirs, U)
+    assert grad.dtype == torch.float32 and grad.shape == (points.shape[0], U.shape[1])
+    dev = points.device
+    ws = workspace(dev)
+    gp = torch.empty(points.shape[0], 3, dtype=torch.float32, device=dev)
+    gd = torch.empty(points.shape[0], 3, dtype=torch.float32, device=dev) if dirs is not None else None
+    with torch.cuda.device(dev):
+        _lib.check(lib.ds_modal_gains_backward(ws.handle, *args, _p(grad), _p(gp), _p(gd), _stream()),
+                   "ds_modal_gains_backward")
+    return gp, gd

@@ -495,6 +495,46 @@ int ds_stuff_count(ds_workspace* ws, const int8_t* signs, int64_t nx, int64_t ny
 int ds_stuff_fill(ds_workspace* ws, const int8_t* signs, const int64_t* edges, const double* t, int64_t* tets_out,
                   float* pos_out, void* stream);
 
+/* ---- modal gains: where a struck surface point excites each mode ------------------------------------------------
+ * New capability: nothing in the reference computes mode gains from the mode shapes (its audio paths take the mode
+ * amplitudes from learned parameters or ones).  See csrc/gains.cu and the definition in oracle/modal_gains.py.
+ * Meshes: verts fp32 [n_nodes x 3], tets int32 [T x npe] (npe = 4 at order 1, 10 at order 2 in the local node order of
+ * shape_func.P2_NODES; the corners are the local nodes 0, 1, 2, 3 / 0, 2, 4, 9).
+ *
+ * ds_tet_boundary_count -> the number F of triangles that belong to exactly one tet; ds_tet_boundary_fill -> faces_out
+ * int32 [F x 3] (corner node ids, oriented so that (b - a) x (c - a) points out of the owning tet, decided by an fp64
+ * determinant), owner_out int32 [F] (the tet), local_out int32 [F] (the tet corner the face is opposite to), in
+ * ascending order of the sorted corner triple: independent of the tet order and of corner rotation within a tet, and
+ * bitwise reproducible.  The inputs of the count call must stay alive until the fill call.  The count call
+ * synchronises; a node id outside [0, n_nodes), a non-finite coordinate, a face shared by more than two tets
+ * (non-conforming mesh), order not 1 or 2, an empty mesh or null pointers return DS_ERR_ARG with a message. */
+int ds_tet_boundary_count(ds_workspace* ws, const float* verts, int64_t n_nodes, const int32_t* tets, int64_t T, int order,
+                          int64_t* n_faces_host, void* stream);
+int ds_tet_boundary_fill(ds_workspace* ws, int32_t* faces_out, int32_t* owner_out, int32_t* local_out, void* stream);
+/* Gains of the modes at surface points: for point p on boundary face face[p] (the arrays of ds_tet_boundary_*), x = the
+ * closest point of that face to points[p] (fp64 region analysis), L = the owning tet's barycentrics of x (0 at the
+ * corner opposite the face), N_a = the P1 / P2 shape functions at L and d = dirs[p] (fp32 [P x 3]; NULL: the face's
+ * outward unit normal):  gains_out[p, m] = sum_a N_a sum_c d_c U[(3 node_a + c) ldu + m], m < k, summed in fp64 in
+ * that order (local node, then component) and rounded once to fp32 [P x k].  U is an fp64 row-major block read in
+ * place (leading dimension ldu >= k), e.g. the mass-normalised mode shapes of ds_lobpcg.  closest_out fp32 [P x 3] = x.
+ * Synchronises once: order not 1 or 2, k < 1, ldu < k, a face id outside [0, F), non-finite points or directions, a
+ * boundary record that is not a face of its owning tet, empty meshes or null pointers return DS_ERR_ARG. */
+int ds_modal_gains(ds_workspace* ws, const float* verts, int64_t n_nodes, const int32_t* tets, int64_t T, int order,
+                   const int32_t* bfaces, const int32_t* bowner, const int32_t* blocal, int64_t F, const float* points,
+                   const int32_t* face, const float* dirs, int64_t P, const double* U, int64_t ldu, int k, float* gains_out,
+                   float* closest_out, void* stream);
+/* Gradient of ds_modal_gains (same inputs) given the upstream gradient grad_gains fp32 [P x k]:
+ *   grad_points [P x 3] = J^T sum_m up[p, m] sum_a (d . u_{a,m}) grad N_a, grad N_a in physical coordinates from the
+ *   corner Jacobian (fp64) and J the Jacobian of the closest-point map: I - n n^T in the face region, t t^T on an edge
+ *   (t its unit direction), 0 at a vertex; so it is the gradient of p -> g(closest(p)) on the given face.
+ *   grad_dirs [P x 3] = sum_m up[p, m] u_m(x); written only when dirs is not NULL.
+ * fp32 outputs of fp64 sums; each output belongs to one point (no atomics), bitwise reproducible.  Same checks and
+ * synchronisation as ds_modal_gains. */
+int ds_modal_gains_backward(ds_workspace* ws, const float* verts, int64_t n_nodes, const int32_t* tets, int64_t T, int order,
+                            const int32_t* bfaces, const int32_t* bowner, const int32_t* blocal, int64_t F,
+                            const float* points, const int32_t* face, const float* dirs, int64_t P, const double* U,
+                            int64_t ldu, int k, const float* grad_gains, float* grad_points, float* grad_dirs, void* stream);
+
 /* ---- device-side timing per kernel class ---------------------------------------
  * Replaces the reference's opt-in torch.profiler hook of lobpcg (src/lobpcg/_lobpcg.py:357-369)
  * and the TICK/TOCK macros (src/include/macro.h:31-44): CUDA events around every launch site,
