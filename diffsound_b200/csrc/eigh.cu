@@ -316,7 +316,10 @@ k_eigh_jacobi(int N, double* __restrict__ scratch, int* __restrict__ info) {
     // A sweep in which every rotated cosine was below 3.2e-9 is the last one: a rotation zeroes its own pair and disturbs the
     // inner product of another pair (i, k) by cos(i, j) cos(j, k), so whatever the <= N - 1 rotations of row i leave behind is
     // below N * 1e-17 <= 1.44e-15, the threshold itself.  Without this test every solve paid one more full sweep that only
-    // confirmed that nothing is left to rotate (1 of ~10 at N = 132).
+    // confirmed that nothing is left to rotate (1 of ~10 at N = 132).  The rotation's tangent must be below 3.2e-9 as
+    // well: two rows of nearly equal norm (a cluster of theta + sigma, e.g. every value of a pencil whose shift dominates)
+    // turn by a large angle at a tiny cosine, which carries the other pairs' inner products over instead of shrinking them
+    // (N = 144, spectrum [-1e-5, 1] at sigma = 1e5: stopping on the cosine alone left theta_min wrong by 1.3e-6).
     const double big2 = 1e-17;
     int big = 0;
 
@@ -351,11 +354,11 @@ k_eigh_jacobi(int N, double* __restrict__ scratch, int* __restrict__ info) {
         }
         const double ga = warp_sum(g0 + g1);
         if (!(enable && ga * ga > tol2 * nx * ny)) return 0;
-        big |= ga * ga > big2 * nx * ny;
         // tan(theta) = 2 ga / (d + sign(d) sqrt(d^2 + 4 ga^2)),  d = ny - nx
         const double d = ny - nx;
         const double h = sqrt(fma(d, d, 4.0 * ga * ga));
         const double t = 2.0 * ga / (d + (d >= 0.0 ? h : -h));
+        big |= ga * ga > big2 * nx * ny || t * t > big2;
         const double c = rsqrt(fma(t, t, 1.0)), sn = c * t;
 #pragma unroll
         for (int i = 0; i < JC_E; ++i) {

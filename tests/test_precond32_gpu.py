@@ -200,15 +200,21 @@ def test_persistent_chebyshev_matches_stepwise(meshes, name, order, ncols, degre
     """The cooperative one-launch Chebyshev solve (records in shared memory, grid barrier per step) against the same
     recurrence run as one SpMM launch per step: identical arithmetic, so the iterates agree to fp32 rounding, and both
     reduce the residual of K z = r."""
-    from diffsound_b200 import native
+    from diffsound_b200 import _lib, native
+    lib = _lib.load()
     v, t = meshes[name]
     _, _, _, _, pat, Kval, Mblk, K = _assembled(v, t, order)
     rec, invD = native.k32_pack(pat, Kval)
     g = torch.Generator(device=DEV).manual_seed(11)
     R = torch.randn(pat.n, ncols, device=DEV, generator=g) * float(np.abs(K.data).max())
     lmax, ratio = 2.8, 0.4 * degree * degree + 2.0
+    n0 = lib.ds_launch_count()
     za = native.cheb32_solve(pat, rec, invD, R, degree, lmax, ratio, persistent=True)
+    n1 = lib.ds_launch_count()
     zb = native.cheb32_solve(pat, rec, invD, R, degree, lmax, ratio, persistent=False)
+    # launches: the row-chunk table, then the one cooperative kernel, or the Jacobi step and degree - 1 SpMM steps
+    assert n1 - n0 == 2, "the persistent kernel did not run"
+    assert lib.ds_launch_count() - n1 == 1 + degree
     assert torch.isfinite(za).all()
     scale = float(zb.abs().max())
     assert float((za - zb).abs().max()) <= 2e-5 * scale
