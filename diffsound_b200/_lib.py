@@ -26,13 +26,14 @@ class LobpcgOpts(C.Structure):
                 ("sigma", C.c_double), ("cheb_ratio", C.c_double), ("n_rigid", C.c_int), ("verbose", C.c_int),
                 ("smooth_steps", C.c_int), ("coarse_degree", C.c_int), ("smooth_ratio", C.c_double),
                 ("coarse_ratio", C.c_double), ("nested", C.c_int), ("nested_tol", C.c_double),
-                ("nested_degree", C.c_int), ("coords", C.c_void_p), ("locked", C.c_void_p), ("n_locked", C.c_int), ("precond_fp64", C.c_int), ("ortho_w", C.c_int)]
+                ("nested_degree", C.c_int), ("coords", C.c_void_p), ("locked", C.c_void_p), ("n_locked", C.c_int), ("precond_fp64", C.c_int), ("ortho_w", C.c_int),
+                ("fixed", C.c_void_p)]
 
 
 class PmgLevel(C.Structure):
     _fields_ = [("brow", C.c_void_p), ("bcol", C.c_void_p), ("n_nodes", C.c_int64), ("nnzb", C.c_int64),
                 ("Kval", C.c_void_p), ("Mblk", C.c_void_p), ("parents", C.c_void_p), ("rptr", C.c_void_p),
-                ("rlist", C.c_void_p), ("coords", C.c_void_p)]
+                ("rlist", C.c_void_p), ("coords", C.c_void_p), ("fixed", C.c_void_p)]
 
 
 # name -> (restype, argtypes); mirrors include/diffsound_sm100.h one to one
@@ -50,6 +51,7 @@ SIGNATURES = {
     "ds_assemble_km_tets": (cint, [f32p, i32p, i64, cint, i64, dbl, dbl, f64p, f64p, i32p, i32p, i32p, i32p, i32p, cint, i64,
                                    f64p, f64p, f64p, ptr]),
     "ds_mass_expand": (cint, [i32p, i64, i64, f64p, f64p, ptr]),
+    "ds_fix_nodes_km": (cint, [i32p, i32p, i64, i64, ptr, f64p, f64p, ptr]),
     "ds_assemble_mass_coo": (cint, [f64p, i32p, i64, cint, f64p, dbl, f64p, i32p, i32p, ptr]),
     "ds_spmm_km": (cint, [i32p, i32p, i64, f64p, f64p, dbl, f64p, i64, cint, dbl, dbl, f64p, i64, f64p, i64, ptr]),
     "ds_spmm_k_and_m": (cint, [i32p, i32p, i64, f64p, f64p, f64p, i64, cint, f64p, i64, f64p, i64, ptr]),

@@ -48,6 +48,11 @@ int gather_cols_f32(const double* src, int64_t lds, const ColIdx& idx, int count
 int widen_f32(const float* src, int width, int64_t n, double* dst, int64_t ldd, cudaStream_t st,
               const int32_t* perm = nullptr);
 int colnorm2_f32(const float* V, int w, int64_t n, double* partial, int ctas, cudaStream_t st);
+// fixed.cu: V[3 i + q, :w] = 0 for the nodes i of a row numbering with fixed[perm ? perm[i] : i] (timed as PROF_FIXED)
+int mask_fixed_rows_f64(const uint8_t* fixed, const int32_t* perm, int64_t n_nodes, double* V, int64_t ld, int w,
+                        cudaStream_t st);
+int mask_fixed_rows_f32(const uint8_t* fixed, const int32_t* perm, int64_t n_nodes, float* V, int64_t ld, int w,
+                        cudaStream_t st);
 int fill_random_f32(float* V, int64_t count, uint64_t seed, cudaStream_t st);
 
 // Morton codes of points (also used by the triangle-mesh BVH of sdf.cu).  ordered_key maps a float to a uint32 whose

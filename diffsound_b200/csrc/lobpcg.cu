@@ -14,6 +14,10 @@
 // way T is a fixed SPD polynomial in the SpMM kernel, so the eigen-solve is a stream of SpMM
 // (HBM-bound) + DMMA Gram/GEMM kernels + one single-CTA Jacobi per step.
 //
+// Clamped nodes (ds_lobpcg_opts.fixed, csrc/fixed.cu): K and M arrive constrained, and the rows of the fixed nodes are
+// zeroed in the start block (after the nested start's prolongation) and in every preconditioner output, one masking
+// launch each.  X, W and P then stay exactly zero there, so the iteration is the one of the reduced problem.
+//
 // Storage: three wide row-major buffers S, KS, MS of n x 3m (columns [X | W | P]) plus a
 // ping-pong copy, so the Ritz update is one tall-skinny GEMM per buffer.
 #include "common.cuh"
@@ -507,6 +511,7 @@ struct Driver {
         dc.o.locked = nullptr;
         dc.o.n_locked = 0;
         dc.o.coords = cl->coords;
+        dc.o.fixed = cl->fixed;
         dc.o.tol = o.nested_tol > 0.0 ? o.nested_tol : 3e-2;
         dc.o.maxit = 40;
         const int deg = o.nested_degree > 0
@@ -558,6 +563,7 @@ int Driver::run(double* X, double* lambda_out, double* resid_out, int64_t* stats
     // ---- initial Rayleigh-Ritz on X
     cur = 0;
     DS_CUDA(cudaMemcpy2DAsync(Xb(0), ld * 8, X, m * 8, m * 8, n, cudaMemcpyDeviceToDevice, st));
+    if (o.fixed) DS_TRY(mask_fixed_rows_f64(o.fixed, nullptr, n_nodes, Xb(0), ld, m, st));
     if (nq) {
         for (int c0 = 0; c0 < nq; c0 += 64) {
             const int wc = std::min(64, nq - c0);
@@ -666,9 +672,12 @@ int Driver::run(double* X, double* lambda_out, double* resid_out, int64_t* stats
             const int deg64 = o.cheb_degree > 0 ? o.cheb_degree : 16;
             DS_TRY(apply_precond64(wpad, deg64, o.cheb_ratio > 1.0 ? o.cheb_ratio : 0.4 * deg64 * deg64, 1.25 * fine.lmax / 1.1,
                                    Wb(cur), ld));
+            if (o.fixed) DS_TRY(mask_fixed_rows_f64(o.fixed, nullptr, n_nodes, Wb(cur), ld, wpad, st));
         } else {
             DS_TRY(gather_cols_f32(R, m, ci, na, wpad, n, R32, st, fine.perm));
             DS_TRY(apply_precond(wpad, &Zres));
+            // Zres is in the preconditioner's numbering (read as is by k_spmm_dual_z32): mask it through the permutation
+            if (o.fixed) DS_TRY(mask_fixed_rows_f32(o.fixed, fine.perm, n_nodes, Zres, wpad, wpad, st));
             DS_TRY(widen_f32(Zres, wpad, n, Wb(cur), ld, st, fine.perm));
         }
         if (o.verbose && !o.precond_fp64) {          // diagnostics: energy norm of the residuals, r_j^T T r_j / lambda_j
@@ -818,6 +827,7 @@ extern "C" int ds_lobpcg(ds_workspace* ws, const int32_t* brow, const int32_t* b
                (long long)(3 * n_nodes), 3 * m);
     DS_REQUIRE(opts->cheb_degree >= 1 && opts->maxit >= 1 && opts->tol > 0, "ds_lobpcg: bad options");
     DS_REQUIRE(opts->n_rigid >= -1 && opts->n_rigid <= opts->nev, "ds_lobpcg: bad n_rigid");
+    DS_REQUIRE(!opts->fixed || opts->n_rigid == 0, "ds_lobpcg: clamped nodes leave no rigid modes: n_rigid must be 0");
     if (coarse) {
         DS_REQUIRE(coarse->brow && coarse->bcol && coarse->Kval && coarse->parents && coarse->rptr && coarse->rlist &&
                        coarse->n_nodes > 0 && coarse->nnzb > 0,

@@ -119,6 +119,22 @@ def build_model(mesh_dir, mode_num, order, mat, task, vertices=None, tets=None, 
     return model
 
 
+def check_fixed_mask(vertices, mask):
+    """Host validation of a clamp mask (DiffSoundObj.fix_nodes): a boolean (n_nodes,) tensor over `vertices` whose nodes
+    contain three non-collinear points, so that the clamps remove all rigid motion.  Raises ValueError otherwise."""
+    n_nodes = vertices.shape[0]
+    if not torch.is_tensor(mask) or mask.dtype != torch.bool:
+        raise ValueError("fix_nodes: mask must be a boolean tensor")
+    if mask.shape != (n_nodes,):
+        raise ValueError(f"fix_nodes: mask has shape {tuple(mask.shape)}, expected ({n_nodes},) over tetmesh.vertices")
+    p = vertices.detach()[mask].double().cpu()
+    sv = torch.linalg.svdvals(p - p.mean(0)) if p.shape[0] >= 3 else torch.zeros(2, dtype=torch.float64)
+    # relative to the extent of the fixed set: fp32 coordinates of points on one line are collinear to ~1e-7
+    if p.shape[0] < 3 or not bool(sv[1] > 1e-6 * sv[0]):
+        raise ValueError(f"fix_nodes: the {p.shape[0]} fixed nodes do not contain three non-collinear points, so rigid "
+                         "motion would remain; clamp a larger set or none (fix_nodes(None))")
+
+
 def _gram_diag(X, Y):
     """diag(X^T Y) for (n, k) fp64 blocks, in chunks the Gram kernel accepts (<= 64 columns, multiples of 8)."""
     k = X.shape[1]
@@ -142,7 +158,8 @@ class _EigvalShape(torch.autograd.Function):
         d = obj.deform
         pat = d.pattern
         KX, MX = native.spmm_k_and_m(pat, obj._Kval, obj._Mblk, X)
-        lo, hi = 6, 6 + obj.mode_num
+        lo = obj._n_rigid
+        hi = lo + obj.mode_num
         uku = _gram_diag(X, KX)[lo:hi]
         umu = _gram_diag(X, MX)[lo:hi]
         predict = torch.zeros(obj.mode_num, dtype=torch.float32, device=X.device)
@@ -280,6 +297,8 @@ class DiffSoundObj:
         self._q = None
         self.eig_stats = None
         self.last_strike_points = None
+        self.fixed_nodes = None
+        self._fixed_u8 = None
 
     # ------------------------------------------------------------------ parameters
     def parameters(self):
@@ -315,6 +334,8 @@ class DiffSoundObj:
             self._geom = torch.empty(d.num_tets * 14, dtype=torch.float64, device=d.device)
         self._Kval, self._Mblk = native.assemble_km(self._verts32, d.tets_i32, self.tetmesh.order, pat, mu, lam, d.ctab,
                                                     d.mtab(density), Kval=self._Kval, Mblk=self._Mblk, geom=self._geom)
+        if self._fixed_u8 is not None:
+            native.fix_nodes_km(pat, self._fixed_u8, self._Kval, self._Mblk)
         self._density_used = float(density)
         self._lame_used = (mu, lam)
         self.__dict__.pop("_stiff_coo", None)
@@ -366,8 +387,38 @@ class DiffSoundObj:
             mt = d.mtab(self.material_model.mat.density)
             Kmu, _ = native.assemble_km(v32, d.tets_i32, self.tetmesh.order, d.pattern, 1.0, 0.0, d.ctab, mt)
             Kla, _ = native.assemble_km(v32, d.tets_i32, self.tetmesh.order, d.pattern, 0.0, 1.0, d.ctab, mt)
+            if self._fixed_u8 is not None:
+                native.fix_nodes_km(d.pattern, self._fixed_u8, Kmu)
+                native.fix_nodes_km(d.pattern, self._fixed_u8, Kla)
             self._Kunit = (Kmu, Kla)
         return self._Kunit
+
+    # ------------------------------------------------------------------ boundary conditions
+    def fix_nodes(self, mask):
+        """Clamp the object: every node of the boolean (n_nodes,) CUDA mask over `tetmesh.vertices` (the promoted nodes,
+        so the caller chooses the P2 mid-edge nodes too) has all three displacement components fixed to zero.  K and M
+        are constrained on their pattern (native.fix_nodes_km) after every assembly, the eigensolver keeps the rows of
+        the fixed nodes at zero, and `eigenvalues` / `U_hat` are the lowest `mode_num` pairs of the clamped object (it
+        has no rigid modes).  The fixed nodes must contain three non-collinear points, so that no rigid motion remains.
+        `fix_nodes(None)` frees the object again.  Either way the warm start and the cached operators are dropped."""
+        if mask is not None:
+            if torch.is_tensor(mask) and mask.device != self.tetmesh.vertices.device:
+                raise ValueError(f"fix_nodes: mask is on {mask.device}, the mesh on {self.tetmesh.vertices.device}")
+            check_fixed_mask(self.tetmesh.vertices, mask)
+        self.fixed_nodes = mask
+        self._fixed_u8 = None if mask is None else mask.to(torch.uint8).contiguous()
+        self._n_fixed = 0 if mask is None else int(mask.sum())
+        self._warm = []
+        self._q = None
+        for key in ("_Kunit", "_stiff_coo", "_mass_coo"):
+            self.__dict__.pop(key, None)
+        if self._Kval is not None:
+            self._assemble(self._density_used)
+
+    @property
+    def _n_rigid(self):
+        """Rigid-body modes at the bottom of the spectrum: six free-free, none when clamped."""
+        return 6 if self._fixed_u8 is None else 0
 
     # ------------------------------------------------------------------ eigen-solve
     def eigen_decomposition(self):
@@ -377,7 +428,8 @@ class DiffSoundObj:
     def _start_block(self, m, batch=0):
         """Start block of batch `batch` (n, m): the previous decomposition's Ritz block of this mesh when there is
         one (warm start; COPIED -- ds_lobpcg overwrites its block in place and earlier U_hat views / pending
-        backward passes keep the old storage), else the six analytic rigid-body modes + seeded random columns."""
+        backward passes keep the old storage), else the six analytic rigid-body modes (free objects only) + seeded random
+        columns."""
         n = self.deform.pattern.n
         dev = self.deform.device
         prev = self._warm[batch] if batch < len(self._warm) else None
@@ -385,7 +437,7 @@ class DiffSoundObj:
             return prev.clone(), True
         g = torch.Generator(device=dev).manual_seed(batch)
         X = torch.randn(n, m, dtype=torch.float64, device=dev, generator=g)
-        if batch == 0:
+        if batch == 0 and self._n_rigid:
             p = self._verts32.double()
             p = p - p.mean(0, keepdim=True)
             X[:, :6] = 0
@@ -420,22 +472,26 @@ class DiffSoundObj:
         return next((c for c in (16, 32, 48) if c >= need + min(4, c // 8)), None)
 
     def eigen_decomposition_arpack(self):
-        """Lowest mode_num + 6 eigenpairs of K u = lambda M u, rigid six dropped.  The name is the
+        """Lowest mode_num + 6 eigenpairs of K u = lambda M u, rigid six dropped (a clamped object: the lowest mode_num
+        pairs, see fix_nodes).  The name is the
         reference's (diff_model.py:335-369: SciPy ARPACK shift-invert on the CPU); the solver is the
         device-resident LOBPCG of csrc/lobpcg.cu.  More pairs than one 48-column block holds are found in
         batches: every batch runs M-orthogonal to the pairs already converged (ds_lobpcg_opts.locked) and
         starts from the previous batch's guard columns."""
         k = self.mode_num
-        need = k + 6
+        nr = self._n_rigid
+        need = k + nr
         pat = self.deform.pattern
-        if pat.n < 3 * 16 or pat.n < need + 16:
-            raise ValueError(f"mesh too small for {k} modes (n={pat.n})")
+        n_dof = pat.n if self._fixed_u8 is None else pat.n - 3 * self._n_fixed   # a block spans free dofs only
+        if n_dof < 3 * 16 or n_dof < need + 16:
+            raise ValueError(f"mesh too small for {k} modes (n={n_dof} free dofs)")
         deg = int(self.cheb_degree) or int(min(40, max(8, round(pat.n ** (1.0 / 3.0) / 3.0))))
         kw = {}
         coarse = self.deform.coarse if self.two_level else None
         if coarse is not None and 3 * coarse.n_nodes >= 3 * 48:
             # two-level p-multigrid preconditioner: P1 operator of the same mesh, same material
             mu, la = self._lame_used
+            coarse.fixed = None if self._fixed_u8 is None else self._fixed_u8[coarse.corner_nodes].contiguous()
             coarse.assemble(self._verts32, mu, la, coarse.ctab, self.deform.coarse_mtab(self._density_used))
             # n_c^(1/3) scaling fits compact bodies; thin shells (the bowl fixture) need the floor: 37 -> 28 outer iterations
             cdeg = int(self.coarse_degree) or int(min(64, max(32, round((3 * coarse.n_nodes) ** (1.0 / 3.0) / 1.2))))
@@ -447,10 +503,10 @@ class DiffSoundObj:
         while done < need:
             want = min(need - done, self.max_batch)
             m = self._block_for(want)
-            while pat.n < 3 * m and m > 16:
+            while n_dof < 3 * m and m > 16:
                 m -= 16
             if m < want:
-                raise ValueError(f"mesh too small for {k} modes (n={pat.n})")
+                raise ValueError(f"mesh too small for {k} modes (n={n_dof} free dofs)")
             X, is_warm = self._start_block(m, batch)
             if guard is not None and not is_warm:
                 gcols = min(guard.shape[1], m)
@@ -462,8 +518,8 @@ class DiffSoundObj:
                 locked[:, :done] = torch.cat(found_X, dim=1)
             if kw:
                 kw["nested"] = self.nested_start and not is_warm and batch == 0
-            common = dict(nev=want, tol=self.eig_tol, n_rigid=6 if batch == 0 else 0,
-                          coords=self._verts32 if self.morton else None, locked=locked)
+            common = dict(nev=want, tol=self.eig_tol, n_rigid=nr if batch == 0 else 0,
+                          coords=self._verts32 if self.morton else None, locked=locked, fixed=self._fixed_u8)
             stats = None
             if not (self.fp64_fallback and self._has_slivers()):
                 try:
@@ -492,7 +548,7 @@ class DiffSoundObj:
             found_lam.append(lam[:want])
             guard = X[:, want:]
             if batch == 0:
-                self.ritz_values = lam          # all block columns of the first batch (rigid six, modes, guard columns)
+                self.ritz_values = lam          # all block columns of the first batch (rigid modes, modes, guard columns)
             done += want
             batch += 1
         self._warm = warm
@@ -507,8 +563,8 @@ class DiffSoundObj:
             lam_all, order = torch.sort(torch.cat(found_lam))
             self.U_hat_full = torch.cat(found_X, dim=1)[:, order].contiguous()
             self._X = self.U_hat_full
-        self.eigenvalues = lam_all[6:need].clone()
-        self.U_hat = self.U_hat_full[:, 6:need]
+        self.eigenvalues = lam_all[nr:need].clone()
+        self.U_hat = self.U_hat_full[:, nr:need]
         # all wanted columns zero-padded to a multiple of 16 for the SpMM of get_vals()
         if self._X.shape[1] % 16 == 0:
             self._Xpad = self._X

@@ -183,6 +183,18 @@ def assemble_km(verts_f32, tets_i32, order, pattern, mu, lam, ctab, mtab, Kval=N
     return Kval, Mblk
 
 
+def fix_nodes_km(pattern, fixed, Kval, Mblk=None):
+    """Clamp the nodes of the uint8 (n_nodes,) CUDA mask `fixed` in K (and M) in place (ds_fix_nodes_km): every
+    off-diagonal block that touches a fixed node becomes zero; the diagonal blocks and the pattern are kept."""
+    lib = _lib.load()
+    assert fixed.dtype == torch.uint8 and fixed.shape == (pattern.n_nodes,)
+    assert Kval.numel() == pattern.nnz and (Mblk is None or Mblk.numel() == pattern.nnzb)
+    with torch.cuda.device(Kval.device):
+        _lib.check(lib.ds_fix_nodes_km(_p(pattern.brow), _p(pattern.bcol), pattern.n_nodes, pattern.nnzb, _p(fixed),
+                                       _p(Kval), _p(Mblk), _stream()), "ds_fix_nodes_km")
+    return Kval, Mblk
+
+
 def mass_expand(pattern, Mblk):
     lib = _lib.load()
     Mval = torch.empty(pattern.nnz, dtype=torch.float64, device=Mblk.device)
@@ -343,14 +355,17 @@ class CoarseLevel:
         self.corner_nodes = torch.nonzero(self.cid >= 0).squeeze(1)     # fine id of coarse node c, ascending
         self.Kval = self.Mblk = self.geom = None
         self.use_coords = True
+        self.fixed = None           # uint8 (n_nodes,) clamped corner nodes, applied after every assemble()
 
     def assemble(self, verts_f32, mu, lam, ctab1, mtab1):
-        """P1 stiffness (and mass) on the corner nodes at the current vertex positions."""
+        """P1 stiffness (and mass) on the corner nodes at the current vertex positions, clamped at `fixed` when set."""
         self.verts = verts_f32[self.corner_nodes].contiguous()
         if self.geom is None:
             self.geom = torch.empty(self.tets.shape[0] * 14, dtype=torch.float64, device=self.tets.device)
         self.Kval, self.Mblk = assemble_km(self.verts, self.tets, 1, self.pattern, mu, lam, ctab1, mtab1,
                                            Kval=self.Kval, Mblk=self.Mblk, geom=self.geom)
+        if self.fixed is not None:
+            fix_nodes_km(self.pattern, self.fixed, self.Kval, self.Mblk)
 
     def struct(self):
         assert self.Kval is not None, "CoarseLevel: assemble the P1 operator first"
@@ -358,7 +373,8 @@ class CoarseLevel:
                              n_nodes=self.n_nodes, nnzb=self.pattern.nnzb, Kval=self.Kval.data_ptr(),
                              Mblk=self.Mblk.data_ptr() if self.Mblk is not None else None,
                              parents=self.parents.data_ptr(), rptr=self.rptr.data_ptr(), rlist=self.rlist.data_ptr(),
-                             coords=self.verts.data_ptr() if self.use_coords else None)
+                             coords=self.verts.data_ptr() if self.use_coords else None,
+                             fixed=self.fixed.data_ptr() if self.fixed is not None else None)
 
 
 def k32_pack(pattern, Kval, Mblk=None, shift=0.0):
@@ -431,11 +447,13 @@ def pmg_prolong_add32(coarse, zc, z):
 
 def lobpcg(pattern, Kval, Mblk, X, nev, tol=1e-4, maxit=200, cheb_degree=8, sigma=0.0, cheb_ratio=30.0, n_rigid=6,
            verbose=0, coarse=None, smooth_steps=3, smooth_ratio=8.0, coarse_degree=20, coarse_ratio=160.0, nested=True,
-           nested_tol=3e-2, nested_degree=0, coords=None, locked=None, ortho_w=False, precond_fp64=False):
+           nested_tol=3e-2, nested_degree=0, coords=None, locked=None, ortho_w=False, precond_fp64=False, fixed=None):
     """Lowest `nev` pairs of K u = lam M u from the start block X (n, m) fp64 (overwritten with the
     M-orthonormal Ritz vectors).  `coarse`: a CoarseLevel with assembled Kval -> two-level
     preconditioner.  `locked`: (n, q) fp64 contiguous, q a multiple of 16 -- M-orthonormal eigenvectors
     found by earlier calls; the iteration stays M-orthogonal to them and returns the next lowest pairs.
+    `fixed`: uint8 (n_nodes,) clamped nodes (K, M constrained by fix_nodes_km, n_rigid = 0); the Ritz vectors are
+    exactly zero on their rows.  The coarse level's own mask is `coarse.fixed`.
     Returns (lam (m,), resid (m,), stats dict)."""
     lib = _lib.load()
     assert X.dtype == torch.float64 and X.is_contiguous()
@@ -458,6 +476,9 @@ def lobpcg(pattern, Kval, Mblk, X, nev, tol=1e-4, maxit=200, cheb_degree=8, sigm
     if coords is not None:
         assert coords.dtype == torch.float32 and coords.is_contiguous() and coords.shape == (pattern.n_nodes, 3)
         opts.coords = coords.data_ptr()
+    if fixed is not None:
+        assert fixed.dtype == torch.uint8 and fixed.is_cuda and fixed.shape == (pattern.n_nodes,)
+        opts.fixed = fixed.data_ptr()
     stats = (C.c_int64 * 12)()
     ws = workspace(dev)
     if coarse is not None:

@@ -594,6 +594,9 @@ def eigen_decomposition_rowpart(obj, group=None, verbose=False, solver=None, kee
     Assembly is replicated; on return `obj` holds the same attributes as after the single-GPU call, on every rank.
     `solver`: a RowPartLOBPCG of an earlier call on the same topology (partition and peer buffers are reused, only the values
     are refreshed); `keep=True` returns (stats, solver) and leaves the solver open for the next call."""
+    if obj.fixed_nodes is not None:
+        raise NotImplementedError("row-partitioned eigen-solve: clamped objects (DiffSoundObj.fix_nodes) are not supported; "
+                                  "use eigen_decomposition() on one GPU")
     obj._assemble(obj.material_model.mat.density)
     if obj.tetmesh.order != 2 or obj.deform.coarse is None:
         raise NotImplementedError("row-partitioned eigen-solve: quadratic meshes only (two-level preconditioner)")

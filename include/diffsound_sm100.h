@@ -89,6 +89,13 @@ int ds_assemble_km_tets(const float* verts, const int32_t* tets, int64_t T, int 
                         const int32_t* brow, const int32_t* bcol, const int32_t* contrib_ptr,
                         const int32_t* contrib, const int32_t* slot, int max_deg, int64_t nnzb, double* geom,
                         double* Kval, double* Mblk, void* stream);
+/* Clamped nodes (csrc/fixed.cu): homogeneous Dirichlet conditions on whole nodes.  No reference interface: the reference
+ * solves every object free-free.  In place on the block pattern of K (scalar-CSR order, as ds_assemble_km writes it) and M
+ * (one scalar per block, may be NULL): every off-diagonal block (i, j) with fixed[i] || fixed[j] (device uint8 [n_nodes])
+ * becomes zero; diagonal blocks stay as assembled, so M stays SPD.  The pattern and the value order are unchanged.  One
+ * warp per node row, no atomics, deterministic. */
+int ds_fix_nodes_km(const int32_t* brow, const int32_t* bcol, int64_t n_nodes, int64_t nnzb, const uint8_t* fixed,
+                    double* Kval, double* Mblk, void* stream);
 int ds_mass_expand(const int32_t* brow, int64_t n_nodes, int64_t nnzb, const double* Mblk,
                    double* Mval, void* stream);
 /* Legacy twin of the reference export `assemble_mass_matrix` (massMatrixDouble.cu:138-158):
@@ -199,6 +206,10 @@ typedef struct ds_lobpcg_opts {
     int ortho_w;        /* != 0: M-orthogonalise the new search block W against X in FP64 before K W / M W are formed
                            (round-1 behaviour; lobpcg/_lobpcg.py 'ortho').  0 (default): W is the fp32 preconditioner
                            output as is and K W, M W are formed from it directly (k_spmm_dual_z32) */
+    const uint8_t* fixed; /* device [n_nodes] or NULL.  Clamped nodes: K and M carry the constraint of ds_fix_nodes_km and
+                           the driver keeps the rows of these nodes exactly zero in X, W and P (start block, nested start,
+                           preconditioner output), so the iteration runs on the reduced problem of the free dofs.  The
+                           clamps must remove all rigid motion (n_rigid = 0).  NULL: free-free, no extra launch */
 } ds_lobpcg_opts;
 /* Coarse level of the two-level preconditioner: the P1 operator on the corner nodes of a quadratic
  * mesh (pattern + values from ds_pattern_* / ds_assemble_km at order 1 on ds_pmg_coarse_fill's
@@ -214,6 +225,8 @@ typedef struct ds_pmg_level {
     const int32_t* rptr;      /* [n_nodes+1]  transpose (gather) lists of the prolongation */
     const int32_t* rlist;     /* [2*n_fine_nodes] */
     const float* coords;      /* fp32 [n_nodes x 3] coarse node coordinates or NULL (see ds_lobpcg_opts.coords) */
+    const uint8_t* fixed;     /* [n_nodes] clamped coarse nodes (the fine mask at the corner nodes; Kval / Mblk constrained
+                                 by ds_fix_nodes_km) or NULL; used by the nested start's coarse eigen-solve */
 } ds_pmg_level;
 int ds_lobpcg(ds_workspace* ws, const int32_t* brow, const int32_t* bcol, int64_t n_nodes,
               const double* Kval, const double* Mblk, const ds_pmg_level* coarse /* may be NULL */,
