@@ -16,6 +16,8 @@
 //   M_ab = mtab[a][b] |det6V| I3.
 // Owner-computes: the warp that owns node row i sums all element contributions of its blocks
 // (i, bcol[brow[i]+p]) in ascending element order, the work split evenly over its lanes (k_assemble_rows).
+// Material fields (FIELD = true): mu, lam and the mass table entry come from tet e's own (mu_e, lam_e, rho_e) with the
+// scalar kernels' operation order, so a constant field reproduces the homogeneous K and M bit for bit.
 #include "common.cuh"
 #include "../../include/diffsound_sm100.h"
 #include <algorithm>
@@ -101,15 +103,39 @@ __global__ void k_tet_geometry(const float* __restrict__ verts, const int32_t* _
     g[13] = fabs(__dadd_rn(__dadd_rn(t1, t2), t3));
 }
 
+// Per-tet material of the field variants (ds_assemble_km_field): Lame parameters (fp64) and density (fp32) of tet e, and
+// the fp32 unit-density mass table.  The scalar kernels are the FIELD = false instantiations and never read it.
+struct FieldArgs {
+    const double* __restrict__ mu;
+    const double* __restrict__ lam;
+    const float* __restrict__ rho;
+    const float* __restrict__ m32;
+};
+
+// mass table entry of one element: s_mtab holds double(float32(m_ab) * float32(rho)) for one material, double(m_ab) for a
+// field, whose entry is then rounded exactly as mass_density_table rounds the scalar density: a constant field gives
+// the homogeneous M bit for bit
+template <bool FIELD>
+__device__ __forceinline__ double mass_entry(double tab, float rho_e) {
+    return FIELD ? (double)__fmul_rn((float)tab, rho_e) : tab;
+}
+
+template <bool FIELD>
+__device__ __forceinline__ void stage_mtab(double* s_mtab, const double* __restrict__ mtab_g, const FieldArgs& f, int n) {
+    for (int t = threadIdx.x; t < n; t += blockDim.x) s_mtab[t] = FIELD ? (double)f.m32[t] : mtab_g[t];
+}
+
 // one element contribution (tet e, local nodes a, b) added to a 3x3 accumulator and the mass scalar
-template <int ORDER>
+template <int ORDER, bool FIELD>
 __device__ __forceinline__ void add_contribution(int pair, const double* __restrict__ geom, const double* s_ctab,
-                                                 const double* s_mtab, double mu, double lam, double (&acc)[3][3],
-                                                 double& macc) {
+                                                 const double* s_mtab, double mu_s, double lam_s, const FieldArgs& f,
+                                                 double (&acc)[3][3], double& macc) {
     constexpr int NPE = ORDER == 1 ? 4 : 10;
     constexpr int NPE2 = NPE * NPE;
     const int e = pair / NPE2;
     const int ab = pair - e * NPE2;
+    const double mu = FIELD ? __ldg(f.mu + e) : mu_s;
+    const double lam = FIELD ? __ldg(f.lam + e) : lam_s;
     const int a = ab / NPE, b = ab - a * NPE;
     const double* g = geom + (int64_t)e * GEOM_STRIDE;
     double S[3][3] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}};
@@ -146,7 +172,7 @@ __device__ __forceinline__ void add_contribution(int pair, const double* __restr
             if (c == d) v += tr;
             acc[c][d] += detK * v;
         }
-    macc += s_mtab[ab] * detM;
+    macc += mass_entry<FIELD>(s_mtab[ab], FIELD ? __ldg(f.rho + e) : 0.0f) * detM;
 }
 
 // Owner-computes with BALANCED lanes.  A warp owns one node row; the element contributions of all its block slots
@@ -158,12 +184,12 @@ __device__ __forceinline__ void add_contribution(int pair, const double* __restr
 // (The lane-per-slot version spent 7x the instructions of a balanced warp waiting for the longest slot.)
 constexpr int AS_WARPS = 4;
 
-template <int ORDER>
+template <int ORDER, bool FIELD>
 __global__ void __launch_bounds__(32 * AS_WARPS)
 k_assemble_rows(const double* __restrict__ geom, const double* __restrict__ ctab_g,
                 const double* __restrict__ mtab_g, const int32_t* __restrict__ brow,
                 const int32_t* __restrict__ contrib_ptr, const int32_t* __restrict__ contrib,
-                int64_t n_nodes, double mu, double lam, double* __restrict__ Kval, double* __restrict__ Mblk) {
+                int64_t n_nodes, double mu, double lam, FieldArgs f, double* __restrict__ Kval, double* __restrict__ Mblk) {
     constexpr int NPE = ORDER == 1 ? 4 : 10;
     constexpr int NPE2 = NPE * NPE;
     __shared__ double s_ctab[NPE2 * 16];
@@ -171,7 +197,7 @@ k_assemble_rows(const double* __restrict__ geom, const double* __restrict__ ctab
     __shared__ double s_part[AS_WARPS][32][2][10];     // [lane][head / tail][9 stiffness entries + mass]
     __shared__ int s_head[AS_WARPS][32];               // slot of the lane's head partial, -1: none
     for (int t = threadIdx.x; t < NPE2 * 16; t += blockDim.x) s_ctab[t] = ctab_g[t];
-    for (int t = threadIdx.x; t < NPE2; t += blockDim.x) s_mtab[t] = mtab_g[t];
+    stage_mtab<FIELD>(s_mtab, mtab_g, f, NPE2);
     __syncthreads();
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     double (*part)[2][10] = s_part[warp];
@@ -225,7 +251,7 @@ k_assemble_rows(const double* __restrict__ geom, const double* __restrict__ ctab
                     s_begin = s_end;
                     s_end = contrib_ptr[cur + 1];
                 }
-                add_contribution<ORDER>(contrib[q], geom, s_ctab, s_mtab, mu, lam, acc, macc);
+                add_contribution<ORDER, FIELD>(contrib[q], geom, s_ctab, s_mtab, mu, lam, f, acc, macc);
             }
             // the slot in progress at the end of the chunk
             const bool began_here = s_begin >= qa, ends_here = s_end == qb;
@@ -279,11 +305,12 @@ constexpr int AT_WARPS = 8;
 constexpr int AT_SLOT = 11;                       // doubles per slot of the row image: 9 + 1 + one of padding (an odd pitch
                                                   // spreads the 64-bit accesses over all bank pairs; 10 gave 5-way conflicts)
 
+template <bool FIELD>
 __global__ void __launch_bounds__(32 * AT_WARPS)
 k_assemble_rows_tets2(const double* __restrict__ geom, const double* __restrict__ ctab_g, const double* __restrict__ mtab_g,
                       const int32_t* __restrict__ brow, const int32_t* __restrict__ bcol,
                       const int32_t* __restrict__ contrib_ptr, const int32_t* __restrict__ contrib,
-                      const int32_t* __restrict__ slot, int64_t n_nodes, int cap, double mu, double lam,
+                      const int32_t* __restrict__ slot, int64_t n_nodes, int cap, double mu_s, double lam_s, FieldArgs f,
                       double* __restrict__ Kval, double* __restrict__ Mblk) {
     constexpr int NPE = 10, NPE2 = 100;
     extern __shared__ __align__(16) double s_dyn[];
@@ -296,7 +323,7 @@ k_assemble_rows_tets2(const double* __restrict__ geom, const double* __restrict_
         const bool ok = li < c_nsup2[a] && mi < c_nsup2[b];
         s_ct4[t] = ok ? ctab_g[ab * 16 + c_sup2[a][li] * 4 + c_sup2[b][mi]] : 0.0;
     }
-    for (int t = threadIdx.x; t < NPE2; t += blockDim.x) s_mtab[t] = mtab_g[t];
+    stage_mtab<FIELD>(s_mtab, mtab_g, f, NPE2);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     double* acc = s_acc + (size_t)warp * cap * AT_SLOT;
     for (int t = lane; t < cap * AT_SLOT; t += 32) acc[t] = 0.0;
@@ -324,6 +351,9 @@ k_assemble_rows_tets2(const double* __restrict__ geom, const double* __restrict_
             const int e = pair / NPE2;
             const int a = (pair - e * NPE2) / NPE;                       // the entry is (e, a, a)
             const double* __restrict__ g = geom + (int64_t)e * GEOM_STRIDE;
+            const double mu = FIELD ? __ldg(f.mu + e) : mu_s;                 // warp-uniform: broadcast loads
+            const double lam = FIELD ? __ldg(f.lam + e) : lam_s;
+            const float rho = FIELD ? __ldg(f.rho + e) : 0.0f;
             const int la0 = 3 * c_sup2[a][0], la1 = 3 * c_sup2[a][1];    // warp-uniform
             const int so = lane_on ? __ldg(slot + (int64_t)e * NPE2 + a * NPE + bb) - b0 : 0;
             const double2 ct01 = *reinterpret_cast<const double2*>(s_ct4 + (a * NPE + bb) * 4);       // (l0,m0) (l0,m1)
@@ -362,7 +392,7 @@ k_assemble_rows_tets2(const double* __restrict__ geom, const double* __restrict_
                 out[0] += detK * (c == 0 ? v[0] + tr : v[0]);
                 out[1] += detK * (c == 1 ? v[1] + tr : v[1]);
                 out[2] += detK * (c == 2 ? v[2] + tr : v[2]);
-                if (c == 0) acc[so * AT_SLOT + 9] += s_mtab[a * NPE + bb] * detM;
+                if (c == 0) acc[so * AT_SLOT + 9] += mass_entry<FIELD>(s_mtab[a * NPE + bb], rho) * detM;
             }
             __syncwarp();
             pair = pair_next;
@@ -437,33 +467,84 @@ __global__ void k_mass_coo(const double* __restrict__ vertices, const int32_t* _
 
 using namespace ds;
 
-extern "C" int ds_assemble_km(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes,
-                              double mu, double lam, const double* ctab, const double* mtab,
-                              const int32_t* brow, const int32_t* bcol, const int32_t* contrib_ptr,
-                              const int32_t* contrib, int64_t nnzb, double* geom, double* Kval, double* Mblk,
-                              void* stream_) {
-    cudaStream_t stream = (cudaStream_t)stream_;
-    (void)bcol; (void)nnzb;
-    DS_REQUIRE(order == 1 || order == 2, "ds_assemble_km: order must be 1 or 2 (got %d)", order);
-    DS_REQUIRE(verts && tets && ctab && mtab && brow && contrib_ptr && contrib && geom && Kval && Mblk,
-               "ds_assemble_km: null argument");
-    DS_REQUIRE(T > 0 && n_nodes > 0, "ds_assemble_km: empty mesh");
+static void assemble_account(int64_t T, int npe, int64_t n_nodes, int64_t nnzb, bool field) {
+    prof_account(PROF_ASSEMBLE, 2.0 * 9.0 * (double)nnzb * 8.0 + (double)T * npe * 4.0 + (double)n_nodes * 12.0 + (double)T * npe * npe * 4.0 +
+                 (field ? (double)T * 20.0 : 0.0), 0.0);
+}
+
+template <bool FIELD>
+static int assemble_rows(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes, double mu,
+                         double lam, const FieldArgs& f, const double* ctab, const double* mtab, const int32_t* brow,
+                         const int32_t* contrib_ptr, const int32_t* contrib, int64_t nnzb, double* geom, double* Kval,
+                         double* Mblk, cudaStream_t stream) {
     int npe = order == 1 ? 4 : 10;
     ProfScope prof(PROF_ASSEMBLE, stream);
-    prof_account(PROF_ASSEMBLE, 2.0 * 9.0 * (double)nnzb * 8.0 + (double)T * npe * 4.0 + (double)n_nodes * 12.0 + (double)T * npe * npe * 4.0,
-                 0.0);
+    assemble_account(T, npe, n_nodes, nnzb, FIELD);
     k_tet_geometry<<<(unsigned)ceil_div(T, 128), 128, 0, stream>>>(verts, tets, T, npe, order, geom);
     DS_LAUNCH_CHECK();
     // grid-stride over rows: the per-order tables are staged into shared memory once per CTA
     unsigned blocks = (unsigned)std::min<int64_t>(ceil_div(n_nodes, AS_WARPS), 148 * 12);
     if (order == 1)
-        k_assemble_rows<1><<<blocks, 32 * AS_WARPS, 0, stream>>>(geom, ctab, mtab, brow, contrib_ptr, contrib, n_nodes,
-                                                                 mu, lam, Kval, Mblk);
+        k_assemble_rows<1, FIELD><<<blocks, 32 * AS_WARPS, 0, stream>>>(geom, ctab, mtab, brow, contrib_ptr, contrib, n_nodes,
+                                                                        mu, lam, f, Kval, Mblk);
     else
-        k_assemble_rows<2><<<blocks, 32 * AS_WARPS, 0, stream>>>(geom, ctab, mtab, brow, contrib_ptr, contrib, n_nodes,
-                                                                 mu, lam, Kval, Mblk);
+        k_assemble_rows<2, FIELD><<<blocks, 32 * AS_WARPS, 0, stream>>>(geom, ctab, mtab, brow, contrib_ptr, contrib, n_nodes,
+                                                                        mu, lam, f, Kval, Mblk);
     DS_LAUNCH_CHECK();
     return DS_OK;
+}
+
+template <bool FIELD>
+static int assemble_tets(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes, double mu,
+                         double lam, const FieldArgs& f, const double* ctab, const double* mtab, const int32_t* brow,
+                         const int32_t* bcol, const int32_t* contrib_ptr, const int32_t* contrib, const int32_t* slot,
+                         int max_deg, int64_t nnzb, double* geom, double* Kval, double* Mblk, cudaStream_t stream) {
+    const int npe = 10;
+    ProfScope prof(PROF_ASSEMBLE, stream);
+    assemble_account(T, npe, n_nodes, nnzb, FIELD);
+    k_tet_geometry<<<(unsigned)ceil_div(T, 128), 128, 0, stream>>>(verts, tets, T, npe, order, geom);
+    DS_LAUNCH_CHECK();
+    const int cap = (max_deg + 3) & ~3;
+    const size_t smem = (size_t)(100 * 4 + 100 + (size_t)AT_WARPS * cap * AT_SLOT) * sizeof(double);
+    DS_CUDA(cudaFuncSetAttribute(k_assemble_rows_tets2<FIELD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int per_sm = 1;
+    DS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_assemble_rows_tets2<FIELD>, 32 * AT_WARPS, smem));
+    int dev = 0, sms = 148;
+    DS_CUDA(cudaGetDevice(&dev));
+    DS_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    const unsigned blocks = (unsigned)std::min<int64_t>(ceil_div(n_nodes, AT_WARPS), (int64_t)sms * std::max(per_sm, 1));
+    k_assemble_rows_tets2<FIELD><<<blocks, 32 * AT_WARPS, smem, stream>>>(geom, ctab, mtab, brow, bcol, contrib_ptr, contrib,
+                                                                          slot, n_nodes, cap, mu, lam, f, Kval, Mblk);
+    DS_LAUNCH_CHECK();
+    return DS_OK;
+}
+
+extern "C" int ds_assemble_km(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes,
+                              double mu, double lam, const double* ctab, const double* mtab,
+                              const int32_t* brow, const int32_t* bcol, const int32_t* contrib_ptr,
+                              const int32_t* contrib, int64_t nnzb, double* geom, double* Kval, double* Mblk,
+                              void* stream_) {
+    (void)bcol;
+    DS_REQUIRE(order == 1 || order == 2, "ds_assemble_km: order must be 1 or 2 (got %d)", order);
+    DS_REQUIRE(verts && tets && ctab && mtab && brow && contrib_ptr && contrib && geom && Kval && Mblk,
+               "ds_assemble_km: null argument");
+    DS_REQUIRE(T > 0 && n_nodes > 0, "ds_assemble_km: empty mesh");
+    return assemble_rows<false>(verts, tets, T, order, n_nodes, mu, lam, FieldArgs{}, ctab, mtab, brow, contrib_ptr, contrib,
+                                nnzb, geom, Kval, Mblk, (cudaStream_t)stream_);
+}
+
+extern "C" int ds_assemble_km_field(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes,
+                                    const double* mu_t, const double* lam_t, const float* rho_t, const double* ctab,
+                                    const float* m32, const int32_t* brow, const int32_t* bcol, const int32_t* contrib_ptr,
+                                    const int32_t* contrib, int64_t nnzb, double* geom, double* Kval, double* Mblk,
+                                    void* stream_) {
+    (void)bcol;
+    DS_REQUIRE(order == 1 || order == 2, "ds_assemble_km_field: order must be 1 or 2 (got %d)", order);
+    DS_REQUIRE(verts && tets && mu_t && lam_t && rho_t && ctab && m32 && brow && contrib_ptr && contrib && geom && Kval && Mblk,
+               "ds_assemble_km_field: null argument");
+    DS_REQUIRE(T > 0 && n_nodes > 0, "ds_assemble_km_field: empty mesh");
+    return assemble_rows<true>(verts, tets, T, order, n_nodes, 0.0, 0.0, FieldArgs{mu_t, lam_t, rho_t, m32}, ctab, nullptr,
+                               brow, contrib_ptr, contrib, nnzb, geom, Kval, Mblk, (cudaStream_t)stream_);
 }
 
 // Same result as ds_assemble_km for quadratic tets through the tet-sequential row kernel (k_assemble_rows_tets2);
@@ -473,32 +554,29 @@ extern "C" int ds_assemble_km_tets(const float* verts, const int32_t* tets, int6
                                    const int32_t* brow, const int32_t* bcol, const int32_t* contrib_ptr,
                                    const int32_t* contrib, const int32_t* slot, int max_deg, int64_t nnzb, double* geom,
                                    double* Kval, double* Mblk, void* stream_) {
-    cudaStream_t stream = (cudaStream_t)stream_;
     DS_REQUIRE(order == 2, "ds_assemble_km_tets: quadratic tets only (order 1 goes through ds_assemble_km)");
     DS_REQUIRE(verts && tets && ctab && mtab && brow && bcol && contrib_ptr && contrib && slot && geom && Kval && Mblk,
                "ds_assemble_km_tets: null argument");
     DS_REQUIRE(T > 0 && n_nodes > 0, "ds_assemble_km_tets: empty mesh");
     DS_REQUIRE(max_deg >= 1 && max_deg <= 256, "ds_assemble_km_tets: max_deg=%d must be in [1, 256] (longer rows: ds_assemble_km)",
                max_deg);
-    const int npe = 10;
-    ProfScope prof(PROF_ASSEMBLE, stream);
-    prof_account(PROF_ASSEMBLE, 2.0 * 9.0 * (double)nnzb * 8.0 + (double)T * npe * 4.0 + (double)n_nodes * 12.0 + (double)T * npe * npe * 4.0,
-                 0.0);
-    k_tet_geometry<<<(unsigned)ceil_div(T, 128), 128, 0, stream>>>(verts, tets, T, npe, order, geom);
-    DS_LAUNCH_CHECK();
-    const int cap = (max_deg + 3) & ~3;
-    const size_t smem = (size_t)(100 * 4 + 100 + (size_t)AT_WARPS * cap * AT_SLOT) * sizeof(double);
-    DS_CUDA(cudaFuncSetAttribute(k_assemble_rows_tets2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int per_sm = 1;
-    DS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_assemble_rows_tets2, 32 * AT_WARPS, smem));
-    int dev = 0, sms = 148;
-    DS_CUDA(cudaGetDevice(&dev));
-    DS_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    const unsigned blocks = (unsigned)std::min<int64_t>(ceil_div(n_nodes, AT_WARPS), (int64_t)sms * std::max(per_sm, 1));
-    k_assemble_rows_tets2<<<blocks, 32 * AT_WARPS, smem, stream>>>(geom, ctab, mtab, brow, bcol, contrib_ptr, contrib, slot,
-                                                                  n_nodes, cap, mu, lam, Kval, Mblk);
-    DS_LAUNCH_CHECK();
-    return DS_OK;
+    return assemble_tets<false>(verts, tets, T, order, n_nodes, mu, lam, FieldArgs{}, ctab, mtab, brow, bcol, contrib_ptr,
+                                contrib, slot, max_deg, nnzb, geom, Kval, Mblk, (cudaStream_t)stream_);
+}
+
+extern "C" int ds_assemble_km_tets_field(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes,
+                                         const double* mu_t, const double* lam_t, const float* rho_t, const double* ctab,
+                                         const float* m32, const int32_t* brow, const int32_t* bcol,
+                                         const int32_t* contrib_ptr, const int32_t* contrib, const int32_t* slot, int max_deg,
+                                         int64_t nnzb, double* geom, double* Kval, double* Mblk, void* stream_) {
+    DS_REQUIRE(order == 2, "ds_assemble_km_tets_field: quadratic tets only (order 1 goes through ds_assemble_km_field)");
+    DS_REQUIRE(verts && tets && mu_t && lam_t && rho_t && ctab && m32 && brow && bcol && contrib_ptr && contrib && slot && geom &&
+               Kval && Mblk, "ds_assemble_km_tets_field: null argument");
+    DS_REQUIRE(T > 0 && n_nodes > 0, "ds_assemble_km_tets_field: empty mesh");
+    DS_REQUIRE(max_deg >= 1 && max_deg <= 256,
+               "ds_assemble_km_tets_field: max_deg=%d must be in [1, 256] (longer rows: ds_assemble_km_field)", max_deg);
+    return assemble_tets<true>(verts, tets, T, order, n_nodes, 0.0, 0.0, FieldArgs{mu_t, lam_t, rho_t, m32}, ctab, nullptr,
+                               brow, bcol, contrib_ptr, contrib, slot, max_deg, nnzb, geom, Kval, Mblk, (cudaStream_t)stream_);
 }
 
 extern "C" int ds_mass_expand(const int32_t* brow, int64_t n_nodes, int64_t nnzb, const double* Mblk,

@@ -19,6 +19,9 @@
 // Material forms.  lane = mode.  Linear tets have a constant displacement gradient F; for quadratic
 // tets F is linear in the barycentric coordinates, F(L) = sum_m L_m F_m with F_m its value at corner
 // m, so the exact integral of a quadratic form phi is |det A|/120 (phi(sum_m F_m) + sum_m phi(F_m)).
+//
+// Material fields.  The same element forms per (tet, mode) give d lambda_i / d(mu_t, lam_t, rho_t) and the element
+// energies (k_material_field); the shape gradient reads (mu_t, lam_t, rho_t) per element (k_eigval_grad_shape<_, true>).
 #include "common.cuh"
 #include "../../include/diffsound_sm100.h"
 #include "kernels.cuh"
@@ -126,10 +129,19 @@ struct GradSmem {
     double Q[GS_WARPS][192];                             // 144 Q entries, 12 dE/dG, 12 G (at 160), 12 dD (at 172)
 };
 
-template <int ORDER>
+// Per-tet material of the field variant (ds_eigval_grad_shape_field); unused by the scalar instantiation.
+struct GradField {
+    const double* __restrict__ mu;
+    const double* __restrict__ lam;
+    const float* __restrict__ rho;
+};
+
+// FIELD: mu, lam of element e from the field, mtab_g the unit-density table (promoted fp32) and the mass part of the
+// element scaled by rho_e.
+template <int ORDER, bool FIELD>
 __global__ void __launch_bounds__(GS_WARPS * 32)
-k_eigval_grad_shape(const float* __restrict__ verts, const int32_t* __restrict__ tets, int64_t T, double mu,
-                    double lam, const double* __restrict__ ctab_g, const double* __restrict__ mtab_g,
+k_eigval_grad_shape(const float* __restrict__ verts, const int32_t* __restrict__ tets, int64_t T, double mu_s,
+                    double lam_s, GradField f, const double* __restrict__ ctab_g, const double* __restrict__ mtab_g,
                     const double* __restrict__ U, int64_t ldu, int k, const double* __restrict__ lamv,
                     const double* __restrict__ gv, double* __restrict__ tet_grad) {
     using SM = GradSmem<ORDER>;
@@ -158,6 +170,8 @@ k_eigval_grad_shape(const float* __restrict__ verts, const int32_t* __restrict__
     const int64_t wstride = (int64_t)gridDim.x * GS_WARPS;
     for (int64_t e = (int64_t)blockIdx.x * GS_WARPS + warp; e < T; e += wstride) {
         const int32_t* tp = tets + e * NPE;
+        const double mu = FIELD ? __ldg(f.mu + e) : mu_s;
+        const double lam = FIELD ? __ldg(f.lam + e) : lam_s;
         int32_t cn[4];
         load_corners(tp, ORDER, cn);
         TetGeom geo;
@@ -234,6 +248,7 @@ k_eigval_grad_shape(const float* __restrict__ verts, const int32_t* __restrict__
                 }
         }
         s_mass = warp_sum(s_mass);
+        if (FIELD) s_mass *= (double)__ldg(f.rho + e);
         __syncwarp();
         // ---- Q_lm = sum_ab ctab[a][b][l][m] W_ab
         for (int o = lane; o < 144; o += 32) {
@@ -465,6 +480,140 @@ __global__ void k_quadform_reduce(const double* __restrict__ partial, int nparts
     out[t] = s;
 }
 
+// ---------------------------------------------------------------------------
+// material-field gradient and element energies
+// ---------------------------------------------------------------------------
+// One warp per tet, lane = mode (chunks of 32 modes), the element forms of k_quadforms per (tet, mode):
+//     q_mu = u^T K_mu,t u,  q_lam = u^T K_lam,t u,  q_m = u^T Mhat_t u  (Mhat_t: unit-density mass of tet t).
+// GRAD:   out[t] = (sum_i g_i q_mu, sum_i g_i q_lam, -sum_i g_i lam_i q_m), summed over the lanes by a fixed xor-shuffle
+//         tree -- no atomics, so two runs are bitwise equal.
+// ENERGY: strain[t, i] = mu_t q_mu + lam_t q_lam, kinetic[t, i] = u^T M_t u with the mass table entries rounded as the
+//         field assembly rounds them (float32(m_ab) * float32(rho_t)).
+constexpr int MF_WARPS = 4;
+
+template <int ORDER, bool ENERGY>
+__global__ void __launch_bounds__(MF_WARPS * 32)
+k_material_field(const float* __restrict__ verts, const int32_t* __restrict__ tets, int64_t T, const float* __restrict__ m32,
+                 double wsum, const double* __restrict__ U, int64_t ldu, int k, const double* __restrict__ lamv,
+                 const double* __restrict__ gv, const double* __restrict__ mu_t, const double* __restrict__ lam_t,
+                 const float* __restrict__ rho_t, double* __restrict__ out, double* __restrict__ out2) {
+    constexpr int NPE = ORDER == 1 ? 4 : 10;
+    __shared__ float s_m32[NPE * NPE];
+    for (int t = threadIdx.x; t < NPE * NPE; t += blockDim.x) s_m32[t] = m32[t];
+    __syncthreads();
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t wstride = (int64_t)gridDim.x * MF_WARPS;
+    const int kpad = (k + 31) & ~31;
+    for (int64_t e = (int64_t)blockIdx.x * MF_WARPS + warp; e < T; e += wstride) {
+        const int32_t* tp = tets + e * NPE;
+        int32_t cn[4];
+        load_corners(tp, ORDER, cn);
+        TetGeom geo;
+        tet_geometry<false>(verts, cn, geo);
+        const float rho = ENERGY ? __ldg(rho_t + e) : 1.0f;
+        double a_mu = 0.0, a_la = 0.0, a_m = 0.0;
+        for (int i0 = 0; i0 < kpad; i0 += 32) {
+            const int i = i0 + lane;
+            const bool on = i < k;
+            double u[NPE][3];
+#pragma unroll
+            for (int a = 0; a < NPE; ++a) {
+                const int64_t node = __ldg(tp + a);
+#pragma unroll
+                for (int c = 0; c < 3; ++c) u[a][c] = on ? __ldg(U + (3 * node + c) * ldu + i) : 0.0;
+            }
+            // mass form, as k_quadforms
+            double ms = 0.0;
+#pragma unroll
+            for (int a = 0; a < NPE; ++a) {
+                double ta[3] = {0.0, 0.0, 0.0};
+#pragma unroll
+                for (int b = a + 1; b < NPE; ++b) {
+                    const double mab = ENERGY ? (double)__fmul_rn(s_m32[a * NPE + b], rho) : (double)s_m32[a * NPE + b];
+                    ta[0] = fma(mab, u[b][0], ta[0]);
+                    ta[1] = fma(mab, u[b][1], ta[1]);
+                    ta[2] = fma(mab, u[b][2], ta[2]);
+                }
+                const double maa = ENERGY ? (double)__fmul_rn(s_m32[a * NPE + a], rho) : (double)s_m32[a * NPE + a];
+#pragma unroll
+                for (int c = 0; c < 3; ++c) ms = fma(u[a][c], fma(maa, u[a][c], 2.0 * ta[c]), ms);
+            }
+            const double q_m = geo.detM * ms;
+            double q_mu, q_la;
+            if (ORDER == 1) {
+                double F[3][3];
+#pragma unroll
+                for (int r = 0; r < 3; ++r)
+#pragma unroll
+                    for (int j = 0; j < 3; ++j)
+                        F[r][j] = u[0][r] * geo.G[0][j] + u[1][r] * geo.G[1][j] + u[2][r] * geo.G[2][j] +
+                                  u[3][r] * geo.G[3][j];
+                double pm, pl;
+                phi_pair(F, pm, pl);
+                q_mu = geo.detK * wsum * pm;
+                q_la = geo.detK * wsum * pl;
+            } else {
+                constexpr int CORNER[4] = {0, 2, 4, 9};
+                constexpr int EDGE[4][4] = {{-1, 1, 5, 6}, {1, -1, 3, 7}, {5, 3, -1, 8}, {6, 7, 8, -1}};
+                double S[3][3] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}};
+                double smu = 0.0, sla = 0.0;
+#pragma unroll
+                for (int m = 0; m < 4; ++m) {
+                    double F[3][3] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}};
+#pragma unroll
+                    for (int l = 0; l < 4; ++l) {
+                        double h[3];
+#pragma unroll
+                        for (int r = 0; r < 3; ++r)
+                            h[r] = (l == m) ? 3.0 * u[CORNER[l]][r] : 4.0 * u[EDGE[l][m] < 0 ? 0 : EDGE[l][m]][r] - u[CORNER[l]][r];
+#pragma unroll
+                        for (int r = 0; r < 3; ++r)
+#pragma unroll
+                            for (int j = 0; j < 3; ++j) F[r][j] = fma(h[r], geo.G[l][j], F[r][j]);
+                    }
+                    double pm, pl;
+                    phi_pair(F, pm, pl);
+                    smu += pm;
+                    sla += pl;
+#pragma unroll
+                    for (int r = 0; r < 3; ++r)
+#pragma unroll
+                        for (int j = 0; j < 3; ++j) S[r][j] += F[r][j];
+                }
+                double pm, pl;
+                phi_pair(S, pm, pl);
+                const double w = geo.detK * (1.0 / 120.0);
+                q_mu = w * (smu + pm);
+                q_la = w * (sla + pl);
+            }
+            if (ENERGY) {
+                if (on) {
+                    __stcs(out + e * k + i, fma(__ldg(mu_t + e), q_mu, __ldg(lam_t + e) * q_la));
+                    __stcs(out2 + e * k + i, q_m);
+                }
+            } else if (on) {
+                const double g = __ldg(gv + i);
+                a_mu = fma(g, q_mu, a_mu);
+                a_la = fma(g, q_la, a_la);
+                a_m = fma(-g * __ldg(lamv + i), q_m, a_m);
+            }
+        }
+        if (!ENERGY) {
+#pragma unroll
+            for (int off = 16; off > 0; off >>= 1) {
+                a_mu += __shfl_xor_sync(0xffffffffu, a_mu, off);
+                a_la += __shfl_xor_sync(0xffffffffu, a_la, off);
+                a_m += __shfl_xor_sync(0xffffffffu, a_m, off);
+            }
+            if (lane == 0) {
+                out[3 * e + 0] = a_mu;
+                out[3 * e + 1] = a_la;
+                out[3 * e + 2] = a_m;
+            }
+        }
+    }
+}
+
 static int qf_ctas(int64_t T) {
     int64_t c = ceil_div(T, QF_WARPS * 8);
     if (c < 1) c = 1;
@@ -504,6 +653,38 @@ extern "C" int ds_corner_incidence(ds_workspace* ws, const int32_t* tets, int64_
     return DS_OK;
 }
 
+template <bool FIELD>
+static int grad_shape(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes, double mu,
+                      double lam_lame, const GradField& f, const double* ctab, const double* mtab, const double* U,
+                      int64_t ldu, int k, const double* lam, const double* g, const int32_t* inc_ptr, const int32_t* inc,
+                      double* tet_grad, float* grad_verts, cudaStream_t stream) {
+    const int kpad = (k + 15) & ~15;
+    ProfScope prof(PROF_GRAD, stream);
+    {   // SURVEY 8d: n k 8 (U once) + T npe 4 + nodes 12 + nodes 24; flops: per tet and mode the quadratic forms of the 4 corner
+        // derivatives, ~ 2 (3 npe)^2 x 12 / 4 (counted from the kernel's DMMA tiles in DESIGN.md)
+        const int npe_ = order == 1 ? 4 : 10;
+        prof_account(PROF_GRAD, (double)n_nodes * 3.0 * k * 8.0 + (double)T * npe_ * 4.0 + (double)n_nodes * 36.0 +
+                     (FIELD ? (double)T * 20.0 : 0.0), 0.0);
+    }
+    int64_t ctas64 = ceil_div(T, GS_WARPS);
+    int ctas = (int)(ctas64 < 148 * 8 ? ctas64 : 148 * 8);
+    if (order == 1) {
+        size_t smem = sizeof(GradSmem<1>) + 2 * kpad * sizeof(double);
+        DS_CUDA(cudaFuncSetAttribute(k_eigval_grad_shape<1, FIELD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        k_eigval_grad_shape<1, FIELD><<<ctas, GS_WARPS * 32, smem, stream>>>(verts, tets, T, mu, lam_lame, f, ctab, mtab, U, ldu,
+                                                                             k, lam, g, tet_grad);
+    } else {
+        size_t smem = sizeof(GradSmem<2>) + 2 * kpad * sizeof(double);
+        DS_CUDA(cudaFuncSetAttribute(k_eigval_grad_shape<2, FIELD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        k_eigval_grad_shape<2, FIELD><<<ctas, GS_WARPS * 32, smem, stream>>>(verts, tets, T, mu, lam_lame, f, ctab, mtab, U, ldu,
+                                                                             k, lam, g, tet_grad);
+    }
+    DS_LAUNCH_CHECK();
+    k_node_gather<<<(unsigned)ceil_div(3 * n_nodes, 256), 256, 0, stream>>>(inc_ptr, inc, tet_grad, n_nodes, grad_verts);
+    DS_LAUNCH_CHECK();
+    return DS_OK;
+}
+
 extern "C" int ds_eigval_grad_shape(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes,
                                     double mu, double lam_lame, const double* ctab, const double* mtab,
                                     const double* U, int64_t ldu, int k, const double* lam, const double* g,
@@ -514,30 +695,64 @@ extern "C" int ds_eigval_grad_shape(const float* verts, const int32_t* tets, int
     DS_REQUIRE(verts && tets && ctab && mtab && U && lam && g && inc_ptr && inc && tet_grad && grad_verts,
                "ds_eigval_grad_shape: null argument");
     DS_REQUIRE(T > 0 && n_nodes > 0 && k > 0 && k <= 1024 && ldu >= k, "ds_eigval_grad_shape: bad sizes");
-    const int kpad = (k + 15) & ~15;
-    ProfScope prof(PROF_GRAD, stream);
-    {   // SURVEY 8d: n k 8 (U once) + T npe 4 + nodes 12 + nodes 24; flops: per tet and mode the quadratic forms of the 4 corner
-        // derivatives, ~ 2 (3 npe)^2 x 12 / 4 (counted from the kernel's DMMA tiles in DESIGN.md)
-        const int npe_ = order == 1 ? 4 : 10;
-        prof_account(PROF_GRAD, (double)n_nodes * 3.0 * k * 8.0 + (double)T * npe_ * 4.0 + (double)n_nodes * 36.0, 0.0);
+    return grad_shape<false>(verts, tets, T, order, n_nodes, mu, lam_lame, GradField{}, ctab, mtab, U, ldu, k, lam, g, inc_ptr,
+                             inc, tet_grad, grad_verts, (cudaStream_t)stream_);
+}
+
+extern "C" int ds_eigval_grad_shape_field(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes,
+                                          const double* mu_t, const double* lam_t, const float* rho_t, const double* ctab,
+                                          const double* mtab1, const double* U, int64_t ldu, int k, const double* lam,
+                                          const double* g, const int32_t* inc_ptr, const int32_t* inc, double* tet_grad,
+                                          float* grad_verts, void* stream_) {
+    DS_REQUIRE(order == 1 || order == 2, "ds_eigval_grad_shape_field: order must be 1 or 2 (got %d)", order);
+    DS_REQUIRE(verts && tets && mu_t && lam_t && rho_t && ctab && mtab1 && U && lam && g && inc_ptr && inc && tet_grad &&
+               grad_verts, "ds_eigval_grad_shape_field: null argument");
+    DS_REQUIRE(T > 0 && n_nodes > 0 && k > 0 && k <= 1024 && ldu >= k, "ds_eigval_grad_shape_field: bad sizes");
+    return grad_shape<true>(verts, tets, T, order, n_nodes, 0.0, 0.0, GradField{mu_t, lam_t, rho_t}, ctab, mtab1, U, ldu, k, lam,
+                            g, inc_ptr, inc, tet_grad, grad_verts, (cudaStream_t)stream_);
+}
+
+template <bool ENERGY>
+static int material_field(const float* verts, const int32_t* tets, int64_t T, int order, const float* m32,
+                          double wsum, const double* U, int64_t ldu, int k, const double* lam, const double* g,
+                          const double* mu_t, const double* lam_t, const float* rho_t, double* out, double* out2,
+                          cudaStream_t stream) {
+    ProfScope prof(PROF_MATERIAL_FIELD, stream);
+    {   // U rows of every tet (re-read per tet: L2), geometry, per-tet material / outputs
+        const int npe = order == 1 ? 4 : 10;
+        prof_account(PROF_MATERIAL_FIELD, (double)T * (npe * 3.0 * k * 8.0 + npe * 4.0 + 48.0) +
+                     (ENERGY ? (double)T * (20.0 + 16.0 * k) : (double)T * 24.0), 0.0);
     }
-    int64_t ctas64 = ceil_div(T, GS_WARPS);
-    int ctas = (int)(ctas64 < 148 * 8 ? ctas64 : 148 * 8);
-    if (order == 1) {
-        size_t smem = sizeof(GradSmem<1>) + 2 * kpad * sizeof(double);
-        DS_CUDA(cudaFuncSetAttribute(k_eigval_grad_shape<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_eigval_grad_shape<1><<<ctas, GS_WARPS * 32, smem, stream>>>(verts, tets, T, mu, lam_lame, ctab, mtab, U, ldu, k,
-                                                                      lam, g, tet_grad);
-    } else {
-        size_t smem = sizeof(GradSmem<2>) + 2 * kpad * sizeof(double);
-        DS_CUDA(cudaFuncSetAttribute(k_eigval_grad_shape<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_eigval_grad_shape<2><<<ctas, GS_WARPS * 32, smem, stream>>>(verts, tets, T, mu, lam_lame, ctab, mtab, U, ldu, k,
-                                                                      lam, g, tet_grad);
-    }
-    DS_LAUNCH_CHECK();
-    k_node_gather<<<(unsigned)ceil_div(3 * n_nodes, 256), 256, 0, stream>>>(inc_ptr, inc, tet_grad, n_nodes, grad_verts);
+    const int64_t ctas64 = ceil_div(T, MF_WARPS);
+    const unsigned ctas = (unsigned)(ctas64 < 148 * 16 ? ctas64 : 148 * 16);
+    if (order == 1)
+        k_material_field<1, ENERGY><<<ctas, MF_WARPS * 32, 0, stream>>>(verts, tets, T, m32, wsum, U, ldu, k, lam, g, mu_t, lam_t,
+                                                                        rho_t, out, out2);
+    else
+        k_material_field<2, ENERGY><<<ctas, MF_WARPS * 32, 0, stream>>>(verts, tets, T, m32, wsum, U, ldu, k, lam, g, mu_t, lam_t,
+                                                                        rho_t, out, out2);
     DS_LAUNCH_CHECK();
     return DS_OK;
+}
+
+extern "C" int ds_material_field_grad(const float* verts, const int32_t* tets, int64_t T, int order, const float* m32,
+                                      double wsum, const double* U, int64_t ldu, int k, const double* lam, const double* g,
+                                      double* out, void* stream_) {
+    DS_REQUIRE(order == 1 || order == 2, "ds_material_field_grad: order must be 1 or 2 (got %d)", order);
+    DS_REQUIRE(verts && tets && m32 && U && lam && g && out, "ds_material_field_grad: null argument");
+    DS_REQUIRE(T > 0 && k > 0 && ldu >= k, "ds_material_field_grad: bad sizes");
+    return material_field<false>(verts, tets, T, order, m32, wsum, U, ldu, k, lam, g, nullptr,
+                                 nullptr, nullptr, out, nullptr, (cudaStream_t)stream_);
+}
+
+extern "C" int ds_element_energies(const float* verts, const int32_t* tets, int64_t T, int order, const float* m32,
+                                   double wsum, const double* U, int64_t ldu, int k, const double* mu_t, const double* lam_t,
+                                   const float* rho_t, double* strain, double* kinetic, void* stream_) {
+    DS_REQUIRE(order == 1 || order == 2, "ds_element_energies: order must be 1 or 2 (got %d)", order);
+    DS_REQUIRE(verts && tets && m32 && U && mu_t && lam_t && rho_t && strain && kinetic, "ds_element_energies: null argument");
+    DS_REQUIRE(T > 0 && k > 0 && ldu >= k, "ds_element_energies: bad sizes");
+    return material_field<true>(verts, tets, T, order, m32, wsum, U, ldu, k, nullptr, nullptr, mu_t,
+                                lam_t, rho_t, strain, kinetic, (cudaStream_t)stream_);
 }
 
 extern "C" int64_t ds_quadform_scratch_elems(int k) { return (int64_t)QF_MAX_CTAS * QF_WARPS * 3 * k; }

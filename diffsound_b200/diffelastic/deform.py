@@ -94,6 +94,14 @@ class Deform:
             cache[key] = _mm.mass_density_table(self.tetmesh.order, key).to(self.device)
         return cache[key]
 
+    def m32(self, order=None):
+        """fp32 unit-density mass table of this mesh's order (or of `order`) on the device, for the material-field kernels."""
+        order = self.tetmesh.order if order is None else order
+        cache = self.__dict__.setdefault("_m32", {})
+        if order not in cache:
+            cache[order] = _mm.unit_mass_table32(order).to(self.device)
+        return cache[order]
+
     def verts_f32(self):
         return self.tetmesh.vertices.detach().to(torch.float32).contiguous()
 

@@ -135,6 +135,47 @@ def check_fixed_mask(vertices, mask):
                          "motion would remain; clamp a larger set or none (fix_nodes(None))")
 
 
+def check_material_field(num_tets, device, youngs=None, poisson=None, density=None):
+    """Host validation of a material field (DiffSoundObj.set_material_field): each given part is a finite fp32 / fp64
+    (num_tets,) tensor on `device` with E > 0, -1 < nu < 0.5 and rho > 0.  Raises ValueError otherwise."""
+    for name, t in (("youngs", youngs), ("poisson", poisson), ("density", density)):
+        if t is None:
+            continue
+        if not torch.is_tensor(t) or t.dtype not in (torch.float32, torch.float64):
+            raise ValueError(f"set_material_field: {name} must be a float32 or float64 tensor")
+        if t.shape != (num_tets,):
+            raise ValueError(f"set_material_field: {name} has shape {tuple(t.shape)}, expected ({num_tets},): one value per "
+                             "row of tetmesh.tets")
+        if t.device != torch.device(device):
+            raise ValueError(f"set_material_field: {name} is on {t.device}, the mesh on {device}")
+        x = t.detach()
+        if not bool(torch.isfinite(x).all()):
+            raise ValueError(f"set_material_field: {name} has non-finite values")
+        if name == "poisson":
+            ok = bool(((x > -1) & (x < 0.5)).all())
+            cond = "-1 < poisson < 0.5"
+        else:
+            ok = bool((x > 0).all())
+            cond = f"{name} > 0"
+        if not ok:
+            raise ValueError(f"set_material_field: {name} violates {cond}")
+
+
+def material_field_from_regions(labels, materials):
+    """(youngs, poisson, density), each (T,) fp64 on the device of `labels`: the material `materials[labels[t]]` (MatSet
+    tuples) of every tet, for DiffSoundObj.set_material_field."""
+    if not torch.is_tensor(labels) or labels.dtype not in (torch.int32, torch.int64) or labels.dim() != 1:
+        raise ValueError("material_field_from_regions: labels must be a 1-D integer tensor")
+    if len(materials) == 0:
+        raise ValueError("material_field_from_regions: no materials")
+    if labels.numel() and (int(labels.min()) < 0 or int(labels.max()) >= len(materials)):
+        raise ValueError(f"material_field_from_regions: labels must lie in [0, {len(materials)})")
+    tab = torch.tensor([[float(m[1]), float(m[2]), float(m[0])] for m in materials], dtype=torch.float64,
+                       device=labels.device)
+    per_tet = tab[labels.long()]
+    return per_tet[:, 0].contiguous(), per_tet[:, 1].contiguous(), per_tet[:, 2].contiguous()
+
+
 def _gram_diag(X, Y):
     """diag(X^T Y) for (n, k) fp64 blocks, in chunks the Gram kernel accepts (<= 64 columns, multiples of 8)."""
     k = X.shape[1]
@@ -143,6 +184,20 @@ def _gram_diag(X, Y):
         c1 = min(k, c0 + 48)
         out.append(torch.diagonal(native.gram(X[:, c0:c1], Y[:, c0:c1])))
     return torch.cat(out)
+
+
+def _vals_forward(obj):
+    """lambda + (u^T K u - lambda u^T M u) of the wanted modes, (mode_num,) fp32: the value of get_vals()."""
+    X, lam = obj._Xpad, obj.eigenvalues          # all wanted columns, padded to a multiple of 16
+    KX, MX = native.spmm_k_and_m(obj.deform.pattern, obj._Kval, obj._Mblk, X)
+    lo = obj._n_rigid
+    hi = lo + obj.mode_num
+    uku = _gram_diag(X, KX)[lo:hi]
+    umu = _gram_diag(X, MX)[lo:hi]
+    predict = torch.zeros(obj.mode_num, dtype=torch.float32, device=X.device)
+    predict += lam
+    predict += uku - lam * umu
+    return predict
 
 
 class _EigvalShape(torch.autograd.Function):
@@ -154,17 +209,9 @@ class _EigvalShape(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, vertices, obj):
-        X, lam = obj._Xpad, obj.eigenvalues          # all wanted columns, padded to a multiple of 16
+        lam = obj.eigenvalues
         d = obj.deform
-        pat = d.pattern
-        KX, MX = native.spmm_k_and_m(pat, obj._Kval, obj._Mblk, X)
-        lo = obj._n_rigid
-        hi = lo + obj.mode_num
-        uku = _gram_diag(X, KX)[lo:hi]
-        umu = _gram_diag(X, MX)[lo:hi]
-        predict = torch.zeros(obj.mode_num, dtype=torch.float32, device=X.device)
-        predict += lam
-        predict += uku - lam * umu
+        predict = _vals_forward(obj)
         ctx.order = obj.tetmesh.order
         ctx.lame = obj._lame_used
         ctx.vdtype = obj.tetmesh.vertices.dtype
@@ -180,6 +227,49 @@ class _EigvalShape(torch.autograd.Function):
         gv = g.reshape(-1).to(torch.float64).contiguous()
         grad = native.eigval_grad_shape(verts32, tets, ctx.order, mu, lam_l, ctab, mtab, ctx.U, lam, gv, inc_ptr, inc)
         return grad.to(ctx.vdtype), None
+
+
+class _EigvalField(torch.autograd.Function):
+    """get_vals() of an object with a material field: the value of _EigvalShape, gradients u^T (dK - lambda dM) u to the
+    vertices (native.eigval_grad_shape_field) and to the per-tet (E, nu, rho) (native.material_field_grad for (mu_t, lam_t,
+    rho_t), then the chain rule of _lame elementwise).  The field values, eigenpairs and geometry the assembly used are
+    pinned at forward time, as in _EigvalShape."""
+
+    @staticmethod
+    def forward(ctx, vertices, youngs, poisson, density, obj):
+        lam = obj.eigenvalues
+        d = obj.deform
+        predict = _vals_forward(obj)
+        f = obj._field_used
+        ctx.order, ctx.wsum = obj.tetmesh.order, d.wsum
+        ctx.vdtype = obj.tetmesh.vertices.dtype
+        ctx.dtypes = tuple(None if t is None else t.dtype for t in (youngs, poisson, density))
+        ctx.U = obj.U_hat
+        inc_ptr, inc = d.incidence
+        ctx.save_for_backward(obj._verts32, d.tets_i32, d.ctab, d.mtab(1.0), d.m32(), lam, inc_ptr, inc, f["mu"], f["lam"],
+                              f["rho"], f["youngs"], f["poisson"])
+        return predict.unsqueeze(1)
+
+    @staticmethod
+    def backward(ctx, g):
+        verts32, tets, ctab, mtab1, m32, lam, inc_ptr, inc, mu_t, lam_t, rho_t, E, nu = ctx.saved_tensors
+        gv = g.reshape(-1).to(torch.float64).contiguous()
+        gverts = gE = gnu = grho = None
+        if ctx.needs_input_grad[0]:
+            gverts = native.eigval_grad_shape_field(verts32, tets, ctx.order, (mu_t, lam_t, rho_t), ctab, mtab1, ctx.U, lam,
+                                                    gv, inc_ptr, inc).to(ctx.vdtype)
+        if any(ctx.needs_input_grad[1:4]):
+            G = native.material_field_grad(verts32, tets, ctx.order, m32, ctx.wsum, ctx.U, lam, gv)
+            if ctx.needs_input_grad[1] or ctx.needs_input_grad[2]:
+                with torch.enable_grad():
+                    E_, nu_ = E.detach().requires_grad_(True), nu.detach().requires_grad_(True)
+                    mu_, la_ = _lame(E_, nu_)
+                    gE, gnu = torch.autograd.grad((mu_ * G[:, 0] + la_ * G[:, 1]).sum(), (E_, nu_))
+                gE = gE.to(ctx.dtypes[0]) if ctx.needs_input_grad[1] else None
+                gnu = gnu.to(ctx.dtypes[1]) if ctx.needs_input_grad[2] else None
+            if ctx.needs_input_grad[3]:
+                grho = G[:, 2].to(ctx.dtypes[2])
+        return gverts, gE, gnu, grho, None
 
 
 class _StiffFunc(torch.autograd.Function):
@@ -299,6 +389,8 @@ class DiffSoundObj:
         self.last_strike_points = None
         self.fixed_nodes = None
         self._fixed_u8 = None
+        self.material_field = None      # (youngs, poisson, density) of set_material_field, None: one material
+        self._field_used = None
 
     # ------------------------------------------------------------------ parameters
     def parameters(self):
@@ -324,6 +416,24 @@ class DiffSoundObj:
         self.scale = torch.eye(3, dtype=torch.float64, device=self.tetmesh.device)
 
     # ------------------------------------------------------------------ assembly
+    def _field_snapshot(self, density):
+        """The field the next assembly uses, validated again (optimisers change the tensors in place): fp64 E, nu and the
+        Lame parameters of _lame, fp32 rho; a part left None is the material's scalar (density: `density`)."""
+        youngs, poisson, dens = self.material_field
+        d = self.deform
+        check_material_field(d.num_tets, d.device, youngs, poisson, dens)
+        mat = self.material_model.mat
+        f64 = dict(dtype=torch.float64, device=d.device)
+
+        def part(t, scalar):
+            return torch.full((d.num_tets,), float(scalar), **f64) if t is None else t.detach().to(torch.float64).clone()
+
+        E, nu = part(youngs, mat.youngs), part(poisson, mat.poisson)
+        mu_t, lam_t = _lame(E, nu)
+        rho = (torch.full((d.num_tets,), float(density), dtype=torch.float32, device=d.device) if dens is None
+               else dens.detach().to(torch.float32).clone())
+        return dict(youngs=E, poisson=nu, mu=mu_t.contiguous(), lam=lam_t.contiguous(), rho=rho.contiguous())
+
     def _assemble(self, density):
         d = self.deform
         mu, lam = self.material_model.lame()
@@ -332,8 +442,16 @@ class DiffSoundObj:
         pat = d.pattern
         if "_geom" not in self.__dict__:
             self._geom = torch.empty(d.num_tets * 14, dtype=torch.float64, device=d.device)
-        self._Kval, self._Mblk = native.assemble_km(self._verts32, d.tets_i32, self.tetmesh.order, pat, mu, lam, d.ctab,
-                                                    d.mtab(density), Kval=self._Kval, Mblk=self._Mblk, geom=self._geom)
+        if self.material_field is None:
+            self._field_used = None
+            self._Kval, self._Mblk = native.assemble_km(self._verts32, d.tets_i32, self.tetmesh.order, pat, mu, lam, d.ctab,
+                                                        d.mtab(density), Kval=self._Kval, Mblk=self._Mblk, geom=self._geom)
+        else:
+            f = self._field_snapshot(density)
+            self._field_used = f
+            self._Kval, self._Mblk = native.assemble_km(self._verts32, d.tets_i32, self.tetmesh.order, pat, 0.0, 0.0, d.ctab,
+                                                        d.m32(), Kval=self._Kval, Mblk=self._Mblk, geom=self._geom,
+                                                        field=(f["mu"], f["lam"], f["rho"]))
         if self._fixed_u8 is not None:
             native.fix_nodes_km(pat, self._fixed_u8, self._Kval, self._Mblk)
         self._density_used = float(density)
@@ -373,6 +491,9 @@ class DiffSoundObj:
     def stiff_func(self, x_in: torch.Tensor):
         """K(theta) x, differentiable in (E, nu) and in x: K = mu K_mu + lam K_lam (diff_model.py:314-328).
         Accepts (n,) or (n, k) like the reference, any number of columns."""
+        if self.material_field is not None:
+            raise NotImplementedError("stiff_func: K = mu K_mu + lam K_lam with one (mu, lam) for the whole object; it is not "
+                                      "defined for a material field (set_material_field(None) first)")
         x = x_in.unsqueeze(1) if x_in.dim() == 1 else x_in
         mu, lam = self.material_model.lame()
         mu = torch.as_tensor(mu, dtype=torch.float32).to(x.device)
@@ -414,6 +535,50 @@ class DiffSoundObj:
             self.__dict__.pop(key, None)
         if self._Kval is not None:
             self._assemble(self._density_used)
+
+    # ------------------------------------------------------------------ material fields
+    def set_material_field(self, youngs=None, poisson=None, density=None):
+        """Give every tet its own material: (T,) fp32 / fp64 CUDA tensors on the mesh's device, indexed by the rows of
+        `tetmesh.tets` (the input tets, in order), of Young's modulus, Poisson's ratio and density.  A part left None is
+        the material's scalar; all three None clears the field (one material again).  The tensors are kept by reference
+        and read (and validated) at every assembly, so an optimiser may update them in place; set the field again each
+        step otherwise.  With a field, K = sum_t (mu_t K_mu,t + lam_t K_lam,t) with (mu_t, lam_t) = _lame(E_t, nu_t) in
+        fp64, and the mass entry of tet t is double(float32(m_ab) * float32(rho_t)): a constant field gives K and M
+        bitwise equal to the homogeneous object.  get_vals() is then differentiable in the three tensors too.  Rayleigh
+        damping stays global (impulse_response's alpha, beta).
+
+        The warm start is kept: a new field on the same mesh is a small perturbation of the previous solve.  Raises
+        ValueError on a TrainableLinear material model (its global E, nu logits and a field would both define E)."""
+        if youngs is None and poisson is None and density is None:
+            self.material_field = None
+        else:
+            if isinstance(self.material_model, TrainableLinear):
+                raise ValueError("set_material_field: the material model is TrainableLinear, whose global (E, nu) logits "
+                                 "would compete with a per-tet field; build the object with FixedLinear")
+            check_material_field(self.deform.num_tets, self.deform.device, youngs, poisson, density)
+            self.material_field = (youngs, poisson, density)
+        self._q = None
+        for key in ("_stiff_coo", "_mass_coo"):
+            self.__dict__.pop(key, None)
+        if self._Kval is not None:
+            self._assemble(self._density_used)
+
+    def element_energies(self):
+        """(strain, kinetic), each (T, mode_num) fp64, no gradient: u_i^T K_t u_i and u_i^T M_t u_i of every tet t and
+        solved mode i (U_hat, M-normalised), for the material of the last assembly (field or not).  Summed over the tets
+        they give u_i^T K u_i = lambda_i and u_i^T M u_i = 1."""
+        if getattr(self, "U_hat", None) is None:
+            raise RuntimeError("element_energies: run eigen_decomposition() first")
+        d = self.deform
+        f = self._field_used
+        if f is None:
+            mu, lam = self._lame_used
+            T = d.num_tets
+            f = dict(mu=torch.full((T,), mu, dtype=torch.float64, device=d.device),
+                     lam=torch.full((T,), lam, dtype=torch.float64, device=d.device),
+                     rho=torch.full((T,), self._density_used, dtype=torch.float32, device=d.device))
+        return native.element_energies(self._verts32, d.tets_i32, self.tetmesh.order, d.m32(), d.wsum, self.U_hat,
+                                       (f["mu"], f["lam"], f["rho"]))
 
     @property
     def _n_rigid(self):
@@ -492,7 +657,11 @@ class DiffSoundObj:
             # two-level p-multigrid preconditioner: P1 operator of the same mesh, same material
             mu, la = self._lame_used
             coarse.fixed = None if self._fixed_u8 is None else self._fixed_u8[coarse.corner_nodes].contiguous()
-            coarse.assemble(self._verts32, mu, la, coarse.ctab, self.deform.coarse_mtab(self._density_used))
+            if self._field_used is None:
+                coarse.assemble(self._verts32, mu, la, coarse.ctab, self.deform.coarse_mtab(self._density_used))
+            else:       # coarse tet t is fine tet t: the same per-tet arrays
+                f = self._field_used
+                coarse.assemble(self._verts32, 0.0, 0.0, coarse.ctab, self.deform.m32(1), field=(f["mu"], f["lam"], f["rho"]))
             # n_c^(1/3) scaling fits compact bodies; thin shells (the bowl fixture) need the floor: 37 -> 28 outer iterations
             cdeg = int(self.coarse_degree) or int(min(64, max(32, round((3 * coarse.n_nodes) ** (1.0 / 3.0) / 1.2))))
             cratio = float(self.coarse_ratio) or 0.4 * cdeg * cdeg
@@ -587,7 +756,8 @@ class DiffSoundObj:
         dev = self.deform.device
         predict = torch.zeros(self.mode_num, dtype=torch.float32, device=dev)
         predict += self.eigenvalues
-        if self.task != "gt":
+        # with a material field the global (E, nu) are not parameters of K (and TrainableLinear is refused): no term to add
+        if self.task != "gt" and self._field_used is None:
             q_mu, q_la, q_m = self._material_forms()
             mu, lam = self.material_model.lame()
             mu, lam = torch.as_tensor(mu).to(dev), torch.as_tensor(lam).to(dev)
@@ -598,7 +768,10 @@ class DiffSoundObj:
 
     def get_vals(self):
         """(mode_num, 1) fp32 eigenvalues, differentiable w.r.t. the vertex positions
-        (diff_model.py:390-399)."""
+        (diff_model.py:390-399) and, with a material field, w.r.t. its tensors."""
+        if self._field_used is not None:
+            youngs, poisson, density = self.material_field if self.material_field is not None else (None, None, None)
+            return _EigvalField.apply(self.tetmesh.vertices, youngs, poisson, density, self)
         return _EigvalShape.apply(self.tetmesh.vertices, self)
 
     # ------------------------------------------------------------------ striking the object

@@ -62,3 +62,9 @@ def mass_density_table(fem_order, density):
     """mtab[a, b] = double(float32(m_ab) * float32(density)), fp64 (nodes, nodes):
     the factor the reference multiplies |6V| with (diff_model.py:299-303)."""
     return (_mass_table_cpu(fem_order, fem_order + 2) * density).double().contiguous()
+
+
+def unit_mass_table32(fem_order):
+    """m_ab fp32 (nodes, nodes): the unit-density table that the material-field kernels round against float32(rho_t) per tet,
+    exactly as mass_density_table rounds against one density."""
+    return _mass_table_cpu(fem_order, fem_order + 2).clone()

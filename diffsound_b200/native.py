@@ -148,10 +148,21 @@ class Pattern:
         return torch.stack([rows, col], dim=0)
 
 
-def assemble_km(verts_f32, tets_i32, order, pattern, mu, lam, ctab, mtab, Kval=None, Mblk=None, geom=None, kernel=None):
+def _check_field(field, T, dev):
+    mu_t, lam_t, rho_t = field
+    for name, t, dt in (("mu", mu_t, torch.float64), ("lam", lam_t, torch.float64), ("rho", rho_t, torch.float32)):
+        if t.dtype != dt or t.shape != (T,) or t.device != dev or not t.is_contiguous():
+            raise ValueError(f"material field: {name} must be a contiguous ({T},) {dt} tensor on {dev}")
+    return _p(mu_t), _p(lam_t), _p(rho_t)
+
+
+def assemble_km(verts_f32, tets_i32, order, pattern, mu, lam, ctab, mtab, Kval=None, Mblk=None, geom=None, kernel=None,
+                field=None):
     """K (scalar-CSR value order of the reference) and M (one scalar per block) into the fixed pattern.  kernel: 'tets'
     (tet-sequential rows: quadratic meshes whose pattern carries the slot map and whose rows have <= 256 blocks), 'rows'
-    (balanced contributor lists: everything else) or None = pick."""
+    (balanced contributor lists: everything else) or None = pick.
+    field: (mu_t (T,) fp64, lam_t (T,) fp64, rho_t (T,) fp32) one material per tet (ds_assemble_km_field /
+    ds_assemble_km_tets_field); mu and lam are then ignored and mtab is the fp32 unit-density mass table (npe, npe)."""
     lib = _lib.load()
     dev = verts_f32.device
     assert verts_f32.dtype == torch.float32 and tets_i32.dtype == torch.int32
@@ -169,6 +180,22 @@ def assemble_km(verts_f32, tets_i32, order, pattern, mu, lam, ctab, mtab, Kval=N
     if kernel == "tets":
         if not can_tets:
             raise ValueError("assemble_km(kernel='tets') needs a quadratic mesh, Pattern(want_slot=True) and rows of <= 256 blocks")
+    if field is not None:
+        assert mtab.dtype == torch.float32
+        fp = _check_field(field, T, dev)
+        with torch.cuda.device(dev):
+            if kernel == "tets":
+                _lib.check(lib.ds_assemble_km_tets_field(_p(verts_f32), _p(tets_i32), T, order, pattern.n_nodes, *fp, _p(ctab),
+                                                         _p(mtab), _p(pattern.brow), _p(pattern.bcol), _p(pattern.contrib_ptr),
+                                                         _p(pattern.contrib), _p(pattern.slot), pattern.max_deg, pattern.nnzb,
+                                                         _p(geom), _p(Kval), _p(Mblk), _stream()), "ds_assemble_km_tets_field")
+            else:
+                _lib.check(lib.ds_assemble_km_field(_p(verts_f32), _p(tets_i32), T, order, pattern.n_nodes, *fp, _p(ctab),
+                                                    _p(mtab), _p(pattern.brow), _p(pattern.bcol), _p(pattern.contrib_ptr),
+                                                    _p(pattern.contrib), pattern.nnzb, _p(geom), _p(Kval), _p(Mblk),
+                                                    _stream()), "ds_assemble_km_field")
+        return Kval, Mblk
+    if kernel == "tets":
         with torch.cuda.device(dev):
             _lib.check(lib.ds_assemble_km_tets(_p(verts_f32), _p(tets_i32), T, order, pattern.n_nodes, float(mu), float(lam),
                                                _p(ctab), _p(mtab), _p(pattern.brow), _p(pattern.bcol), _p(pattern.contrib_ptr),
@@ -357,13 +384,15 @@ class CoarseLevel:
         self.use_coords = True
         self.fixed = None           # uint8 (n_nodes,) clamped corner nodes, applied after every assemble()
 
-    def assemble(self, verts_f32, mu, lam, ctab1, mtab1):
-        """P1 stiffness (and mass) on the corner nodes at the current vertex positions, clamped at `fixed` when set."""
+    def assemble(self, verts_f32, mu, lam, ctab1, mtab1, field=None):
+        """P1 stiffness (and mass) on the corner nodes at the current vertex positions, clamped at `fixed` when set.
+        field: the fine level's (mu_t, lam_t, rho_t) unchanged (coarse tet t is fine tet t; mtab1 then the fp32 unit
+        table), see assemble_km."""
         self.verts = verts_f32[self.corner_nodes].contiguous()
         if self.geom is None:
             self.geom = torch.empty(self.tets.shape[0] * 14, dtype=torch.float64, device=self.tets.device)
         self.Kval, self.Mblk = assemble_km(self.verts, self.tets, 1, self.pattern, mu, lam, ctab1, mtab1,
-                                           Kval=self.Kval, Mblk=self.Mblk, geom=self.geom)
+                                           Kval=self.Kval, Mblk=self.Mblk, geom=self.geom, field=field)
         if self.fixed is not None:
             fix_nodes_km(self.pattern, self.fixed, self.Kval, self.Mblk)
 
@@ -528,6 +557,64 @@ def eigval_grad_shape(verts_f32, tets_i32, order, mu, lam_lame, ctab, mtab, U, l
                                             _p(inc_ptr), _p(inc), _p(tet_grad), _p(out), _stream()),
                    "ds_eigval_grad_shape")
     return out
+
+
+def eigval_grad_shape_field(verts_f32, tets_i32, order, field, ctab, mtab1, U, lam, g, inc_ptr, inc, tet_grad=None):
+    """eigval_grad_shape with one material per tet (ds_eigval_grad_shape_field): field = (mu_t, lam_t, rho_t) as in
+    assemble_km, mtab1 the unit-density table promoted to fp64.  -> (n_nodes, 3) fp32."""
+    lib = _lib.load()
+    dev = verts_f32.device
+    T = tets_i32.shape[0]
+    n_nodes = verts_f32.shape[0]
+    up, ldu = _pv(U)
+    k = U.shape[1]
+    assert lam.dtype == torch.float64 and g.dtype == torch.float64 and lam.numel() == k and g.numel() == k
+    fp = _check_field(field, T, dev)
+    if tet_grad is None:
+        tet_grad = torch.empty(T * 12, dtype=torch.float64, device=dev)
+    out = torch.empty(n_nodes, 3, dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.ds_eigval_grad_shape_field(_p(verts_f32), _p(tets_i32), T, order, n_nodes, *fp, _p(ctab), _p(mtab1),
+                                                  up, ldu, k, _p(lam.contiguous()), _p(g.contiguous()), _p(inc_ptr), _p(inc),
+                                                  _p(tet_grad), _p(out), _stream()), "ds_eigval_grad_shape_field")
+    return out
+
+
+def material_field_grad(verts_f32, tets_i32, order, m32, wsum, U, lam, g):
+    """(T, 3) fp64 per-tet (sum_i g_i u_i^T K_mu,t u_i, sum_i g_i u_i^T K_lam,t u_i, -sum_i g_i lam_i u_i^T Mhat_t u_i)
+    (ds_material_field_grad): the gradient of sum_i g_i lambda_i w.r.t. (mu_t, lam_t, rho_t).  m32: fp32 unit-density
+    mass table; U (n, k) fp64 row-major view, read in place; lam, g (k,) fp64."""
+    lib = _lib.load()
+    dev = verts_f32.device
+    T = tets_i32.shape[0]
+    up, ldu = _pv(U)
+    k = U.shape[1]
+    assert m32.dtype == torch.float32 and lam.dtype == torch.float64 and g.dtype == torch.float64
+    assert lam.numel() == k and g.numel() == k
+    out = torch.empty(T, 3, dtype=torch.float64, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.ds_material_field_grad(_p(verts_f32), _p(tets_i32), T, order, _p(m32), float(wsum), up, ldu, k,
+                                              _p(lam.contiguous()), _p(g.contiguous()), _p(out), _stream()),
+                   "ds_material_field_grad")
+    return out
+
+
+def element_energies(verts_f32, tets_i32, order, m32, wsum, U, field):
+    """(strain, kinetic), each (T, k) fp64: u_i^T K_t u_i and u_i^T M_t u_i of every tet t and mode i (ds_element_energies);
+    field = (mu_t, lam_t, rho_t) as in assemble_km."""
+    lib = _lib.load()
+    dev = verts_f32.device
+    T = tets_i32.shape[0]
+    up, ldu = _pv(U)
+    k = U.shape[1]
+    assert m32.dtype == torch.float32
+    fp = _check_field(field, T, dev)
+    strain = torch.empty(T, k, dtype=torch.float64, device=dev)
+    kinetic = torch.empty(T, k, dtype=torch.float64, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.ds_element_energies(_p(verts_f32), _p(tets_i32), T, order, _p(m32), float(wsum), up, ldu, k, *fp,
+                                           _p(strain), _p(kinetic), _stream()), "ds_element_energies")
+    return strain, kinetic
 
 
 def eigval_quadforms_material(verts_f32, tets_i32, order, mtab, wsum, U):

@@ -89,6 +89,20 @@ int ds_assemble_km_tets(const float* verts, const int32_t* tets, int64_t T, int 
                         const int32_t* brow, const int32_t* bcol, const int32_t* contrib_ptr,
                         const int32_t* contrib, const int32_t* slot, int max_deg, int64_t nnzb, double* geom,
                         double* Kval, double* Mblk, void* stream);
+/* Material fields: the same two assemblies with one material per tet.  No reference interface: the reference models one
+ * material.  mu_t, lam_t: fp64 [T] Lame parameters, rho_t: fp32 [T] densities, indexed like tets; m32: fp32 [npe*npe]
+ * unit-density mass table.  K = sum_t (mu_t K_mu,t + lam_t K_lam,t) and the mass entry of tet t is
+ * double(float(m_ab) * rho_t), with the operation order of the scalar kernels: a constant field gives K and M bitwise
+ * equal to ds_assemble_km / ds_assemble_km_tets.  Same pattern, outputs and determinism. */
+int ds_assemble_km_field(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes,
+                         const double* mu_t, const double* lam_t, const float* rho_t, const double* ctab,
+                         const float* m32, const int32_t* brow, const int32_t* bcol, const int32_t* contrib_ptr,
+                         const int32_t* contrib, int64_t nnzb, double* geom, double* Kval, double* Mblk, void* stream);
+int ds_assemble_km_tets_field(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes,
+                              const double* mu_t, const double* lam_t, const float* rho_t, const double* ctab,
+                              const float* m32, const int32_t* brow, const int32_t* bcol, const int32_t* contrib_ptr,
+                              const int32_t* contrib, const int32_t* slot, int max_deg, int64_t nnzb, double* geom,
+                              double* Kval, double* Mblk, void* stream);
 /* Clamped nodes (csrc/fixed.cu): homogeneous Dirichlet conditions on whole nodes.  No reference interface: the reference
  * solves every object free-free.  In place on the block pattern of K (scalar-CSR order, as ds_assemble_km writes it) and M
  * (one scalar per block, may be NULL): every off-diagonal block (i, j) with fixed[i] || fixed[j] (device uint8 [n_nodes])
@@ -323,6 +337,27 @@ int ds_eigval_grad_shape(const float* verts, const int32_t* tets, int64_t T, int
                          const double* U, int64_t ldu, int k, const double* lam, const double* g,
                          const int32_t* inc_ptr, const int32_t* inc, double* tet_grad,
                          float* grad_verts, void* stream);
+/* Shape gradient with a material field: mu_t, lam_t fp64 [T], rho_t fp32 [T] as ds_assemble_km_field; mtab1: the
+ * unit-density table promoted to fp64 (double(float(m_ab))), the mass part of element t is scaled by rho_t. */
+int ds_eigval_grad_shape_field(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes,
+                               const double* mu_t, const double* lam_t, const float* rho_t, const double* ctab,
+                               const double* mtab1, const double* U, int64_t ldu, int k, const double* lam,
+                               const double* g, const int32_t* inc_ptr, const int32_t* inc, double* tet_grad,
+                               float* grad_verts, void* stream);
+/* Material-field gradient: out fp64 [T*3] = (sum_i g_i u_i^T K_mu,t u_i, sum_i g_i u_i^T K_lam,t u_i,
+ * -sum_i g_i lam_i u_i^T Mhat_t u_i) per tet t, Mhat_t the unit-density element mass (m32: fp32 [npe*npe] table).
+ * The element forms of ds_eigval_quadforms_material (exact quadrature, wsum as there); U fp64 [3*n_nodes x ldu] read in
+ * place, lam/g fp64 [k].  One warp per tet, lanes across modes, a fixed shuffle tree over the lanes: no atomics,
+ * bitwise reproducible. */
+int ds_material_field_grad(const float* verts, const int32_t* tets, int64_t T, int order, const float* m32,
+                           double wsum, const double* U, int64_t ldu, int k, const double* lam, const double* g,
+                           double* out, void* stream);
+/* Element energies of k modes: strain fp64 [T*k] = u_i^T K_t u_i = mu_t q_mu + lam_t q_lam, kinetic fp64 [T*k] =
+ * u_i^T M_t u_i with the mass entries double(float(m_ab) * rho_t) of ds_assemble_km_field.  Same kernel as
+ * ds_material_field_grad without the weighted reduction. */
+int ds_element_energies(const float* verts, const int32_t* tets, int64_t T, int order, const float* m32, double wsum,
+                        const double* U, int64_t ldu, int k, const double* mu_t, const double* lam_t, const float* rho_t,
+                        double* strain, double* kinetic, void* stream);
 /* Material: q_mu[i] = u_i^T K(mu=1,lam=0) u_i, q_lam[i] = u_i^T K(0,1) u_i,
  * q_m[i] = u_i^T M u_i; replaces the matrix-free stiff_func path
  * (diff_model.py:314-328, 371-388; deform.py:70-87, 149-165).  wsum = sum of the
