@@ -54,6 +54,10 @@ SIGNATURES = {
                                     f64p, f64p, f64p, ptr]),
     "ds_assemble_km_tets_field": (cint, [f32p, i32p, i64, cint, i64, f64p, f64p, f32p, f64p, f32p, i32p, i32p, i32p, i32p,
                                          i32p, cint, i64, f64p, f64p, f64p, ptr]),
+    "ds_assemble_km_tensor": (cint, [f32p, i32p, i64, cint, i64, f64p, f32p, f64p, f32p, i32p, i32p, i32p, i32p, i64,
+                                     f64p, f64p, f64p, ptr]),
+    "ds_assemble_km_tets_tensor": (cint, [f32p, i32p, i64, cint, i64, f64p, f32p, f64p, f32p, i32p, i32p, i32p, i32p, i32p,
+                                          cint, i64, f64p, f64p, f64p, ptr]),
     "ds_mass_expand": (cint, [i32p, i64, i64, f64p, f64p, ptr]),
     "ds_fix_nodes_km": (cint, [i32p, i32p, i64, i64, ptr, f64p, f64p, ptr]),
     "ds_assemble_mass_coo": (cint, [f64p, i32p, i64, cint, f64p, dbl, f64p, i32p, i32p, ptr]),
@@ -95,6 +99,10 @@ SIGNATURES = {
                                           f64p, i32p, i32p, f64p, f32p, ptr]),
     "ds_material_field_grad": (cint, [f32p, i32p, i64, cint, f32p, dbl, f64p, i64, cint, f64p, f64p, f64p, ptr]),
     "ds_element_energies": (cint, [f32p, i32p, i64, cint, f32p, dbl, f64p, i64, cint, f64p, f64p, f32p, f64p, f64p, ptr]),
+    "ds_eigval_grad_shape_tensor": (cint, [f32p, i32p, i64, cint, i64, f64p, f32p, f64p, f64p, f64p, i64, cint, f64p, f64p,
+                                           i32p, i32p, f64p, f32p, ptr]),
+    "ds_elasticity_field_grad": (cint, [f32p, i32p, i64, cint, f32p, dbl, f64p, i64, cint, f64p, f64p, f64p, f64p, ptr]),
+    "ds_element_energies_tensor": (cint, [f32p, i32p, i64, cint, f32p, dbl, f64p, i64, cint, f64p, f32p, f64p, f64p, ptr]),
     "ds_quadform_scratch_elems": (i64, [cint]),
     "ds_eigval_quadforms_material": (cint, [f32p, i32p, i64, cint, f64p, dbl, f64p, i64, cint, f64p, f64p, ptr]),
     "ds_synth_scratch_elems": (i64, [i64, cint, i64]),

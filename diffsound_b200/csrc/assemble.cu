@@ -16,8 +16,12 @@
 //   M_ab = mtab[a][b] |det6V| I3.
 // Owner-computes: the warp that owns node row i sums all element contributions of its blocks
 // (i, bcol[brow[i]+p]) in ascending element order, the work split evenly over its lanes (k_assemble_rows).
-// Material fields (FIELD = true): mu, lam and the mass table entry come from tet e's own (mu_e, lam_e, rho_e) with the
+// Material fields (MODE = MAT_LAME): mu, lam and the mass table entry come from tet e's own (mu_e, lam_e, rho_e) with the
 // scalar kernels' operation order, so a constant field reproduces the homogeneous K and M bit for bit.
+// Elasticity-tensor fields (MODE = MAT_TENSOR): tet e's own 6x6 Voigt matrix C_e (order 11, 22, 33, 23, 13, 12, engineering
+// shear strains, sigma_V = C eps_V) in the global frame, packed as its 21-entry upper triangle row by row, and
+//   K_ab[c][d] = |det A| sum_{k,l} C_{ckdl} S_ab[k][l]      (C_{ckdl}: the rank-4 form of C_e).
+// An isotropic C = lam 11^T + mu diag(2, 2, 2, 1, 1, 1) gives the Lame expression above (in another summation order).
 #include "common.cuh"
 #include "../../include/diffsound_sm100.h"
 #include <algorithm>
@@ -103,13 +107,15 @@ __global__ void k_tet_geometry(const float* __restrict__ verts, const int32_t* _
     g[13] = fabs(__dadd_rn(__dadd_rn(t1, t2), t3));
 }
 
-// Per-tet material of the field variants (ds_assemble_km_field): Lame parameters (fp64) and density (fp32) of tet e, and
-// the fp32 unit-density mass table.  The scalar kernels are the FIELD = false instantiations and never read it.
+// Per-tet material of the field variants (ds_assemble_km_field, ds_assemble_km_tensor): Lame parameters (fp64) or the
+// packed elasticity tensor (fp64 [T][21]), the density (fp32) of tet e, and the fp32 unit-density mass table.  The scalar
+// kernels are the MAT_SCALAR instantiations and never read it.
 struct FieldArgs {
     const double* __restrict__ mu;
     const double* __restrict__ lam;
     const float* __restrict__ rho;
     const float* __restrict__ m32;
+    const double* __restrict__ C;
 };
 
 // mass table entry of one element: s_mtab holds double(float32(m_ab) * float32(rho)) for one material, double(m_ab) for a
@@ -126,16 +132,17 @@ __device__ __forceinline__ void stage_mtab(double* s_mtab, const double* __restr
 }
 
 // one element contribution (tet e, local nodes a, b) added to a 3x3 accumulator and the mass scalar
-template <int ORDER, bool FIELD>
+template <int ORDER, int MODE>
 __device__ __forceinline__ void add_contribution(int pair, const double* __restrict__ geom, const double* s_ctab,
                                                  const double* s_mtab, double mu_s, double lam_s, const FieldArgs& f,
                                                  double (&acc)[3][3], double& macc) {
     constexpr int NPE = ORDER == 1 ? 4 : 10;
     constexpr int NPE2 = NPE * NPE;
+    constexpr bool FIELD = MODE != MAT_SCALAR;
     const int e = pair / NPE2;
     const int ab = pair - e * NPE2;
-    const double mu = FIELD ? __ldg(f.mu + e) : mu_s;
-    const double lam = FIELD ? __ldg(f.lam + e) : lam_s;
+    const double mu = MODE == MAT_LAME ? __ldg(f.mu + e) : mu_s;
+    const double lam = MODE == MAT_LAME ? __ldg(f.lam + e) : lam_s;
     const int a = ab / NPE, b = ab - a * NPE;
     const double* g = geom + (int64_t)e * GEOM_STRIDE;
     double S[3][3] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}};
@@ -163,15 +170,33 @@ __device__ __forceinline__ void add_contribution(int pair, const double* __restr
         }
     }
     const double detK = g[12], detM = g[13];
-    const double tr = mu * (S[0][0] + S[1][1] + S[2][2]);
+    if constexpr (MODE == MAT_TENSOR) {
+        const double* __restrict__ Ce = f.C + (int64_t)e * 21;
+        double Cv[21];
 #pragma unroll
-    for (int c = 0; c < 3; ++c)
+        for (int t = 0; t < 21; ++t) Cv[t] = __ldg(Ce + t);
 #pragma unroll
-        for (int d = 0; d < 3; ++d) {
-            double v = mu * S[d][c] + lam * S[c][d];
-            if (c == d) v += tr;
-            acc[c][d] += detK * v;
-        }
+        for (int c = 0; c < 3; ++c)
+#pragma unroll
+            for (int d = 0; d < 3; ++d) {
+                double v = 0.0;
+#pragma unroll
+                for (int k = 0; k < 3; ++k)
+#pragma unroll
+                    for (int l = 0; l < 3; ++l) v = fma(Cv[voigt_packed(voigt(c, k), voigt(d, l))], S[k][l], v);
+                acc[c][d] += detK * v;
+            }
+    } else {
+        const double tr = mu * (S[0][0] + S[1][1] + S[2][2]);
+#pragma unroll
+        for (int c = 0; c < 3; ++c)
+#pragma unroll
+            for (int d = 0; d < 3; ++d) {
+                double v = mu * S[d][c] + lam * S[c][d];
+                if (c == d) v += tr;
+                acc[c][d] += detK * v;
+            }
+    }
     macc += mass_entry<FIELD>(s_mtab[ab], FIELD ? __ldg(f.rho + e) : 0.0f) * detM;
 }
 
@@ -184,7 +209,7 @@ __device__ __forceinline__ void add_contribution(int pair, const double* __restr
 // (The lane-per-slot version spent 7x the instructions of a balanced warp waiting for the longest slot.)
 constexpr int AS_WARPS = 4;
 
-template <int ORDER, bool FIELD>
+template <int ORDER, int MODE>
 __global__ void __launch_bounds__(32 * AS_WARPS)
 k_assemble_rows(const double* __restrict__ geom, const double* __restrict__ ctab_g,
                 const double* __restrict__ mtab_g, const int32_t* __restrict__ brow,
@@ -197,7 +222,7 @@ k_assemble_rows(const double* __restrict__ geom, const double* __restrict__ ctab
     __shared__ double s_part[AS_WARPS][32][2][10];     // [lane][head / tail][9 stiffness entries + mass]
     __shared__ int s_head[AS_WARPS][32];               // slot of the lane's head partial, -1: none
     for (int t = threadIdx.x; t < NPE2 * 16; t += blockDim.x) s_ctab[t] = ctab_g[t];
-    stage_mtab<FIELD>(s_mtab, mtab_g, f, NPE2);
+    stage_mtab<MODE != MAT_SCALAR>(s_mtab, mtab_g, f, NPE2);
     __syncthreads();
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     double (*part)[2][10] = s_part[warp];
@@ -251,7 +276,7 @@ k_assemble_rows(const double* __restrict__ geom, const double* __restrict__ ctab
                     s_begin = s_end;
                     s_end = contrib_ptr[cur + 1];
                 }
-                add_contribution<ORDER, FIELD>(contrib[q], geom, s_ctab, s_mtab, mu, lam, f, acc, macc);
+                add_contribution<ORDER, MODE>(contrib[q], geom, s_ctab, s_mtab, mu, lam, f, acc, macc);
             }
             // the slot in progress at the end of the chunk
             const bool began_here = s_begin >= qa, ends_here = s_end == qb;
@@ -305,7 +330,7 @@ constexpr int AT_WARPS = 8;
 constexpr int AT_SLOT = 11;                       // doubles per slot of the row image: 9 + 1 + one of padding (an odd pitch
                                                   // spreads the 64-bit accesses over all bank pairs; 10 gave 5-way conflicts)
 
-template <bool FIELD>
+template <int MODE>
 __global__ void __launch_bounds__(32 * AT_WARPS)
 k_assemble_rows_tets2(const double* __restrict__ geom, const double* __restrict__ ctab_g, const double* __restrict__ mtab_g,
                       const int32_t* __restrict__ brow, const int32_t* __restrict__ bcol,
@@ -313,6 +338,7 @@ k_assemble_rows_tets2(const double* __restrict__ geom, const double* __restrict_
                       const int32_t* __restrict__ slot, int64_t n_nodes, int cap, double mu_s, double lam_s, FieldArgs f,
                       double* __restrict__ Kval, double* __restrict__ Mblk) {
     constexpr int NPE = 10, NPE2 = 100;
+    constexpr bool FIELD = MODE != MAT_SCALAR;
     extern __shared__ __align__(16) double s_dyn[];
     double* s_ct4 = s_dyn;                        // [a][b][li][mi]: the <= 2 x 2 support products of ctab, zero where absent
     double* s_mtab = s_ct4 + NPE2 * 4;            // [a][b]
@@ -351,8 +377,8 @@ k_assemble_rows_tets2(const double* __restrict__ geom, const double* __restrict_
             const int e = pair / NPE2;
             const int a = (pair - e * NPE2) / NPE;                       // the entry is (e, a, a)
             const double* __restrict__ g = geom + (int64_t)e * GEOM_STRIDE;
-            const double mu = FIELD ? __ldg(f.mu + e) : mu_s;                 // warp-uniform: broadcast loads
-            const double lam = FIELD ? __ldg(f.lam + e) : lam_s;
+            const double mu = MODE == MAT_LAME ? __ldg(f.mu + e) : mu_s;      // warp-uniform: broadcast loads
+            const double lam = MODE == MAT_LAME ? __ldg(f.lam + e) : lam_s;
             const float rho = FIELD ? __ldg(f.rho + e) : 0.0f;
             const int la0 = 3 * c_sup2[a][0], la1 = 3 * c_sup2[a][1];    // warp-uniform
             const int so = lane_on ? __ldg(slot + (int64_t)e * NPE2 + a * NPE + bb) - b0 : 0;
@@ -378,21 +404,53 @@ k_assemble_rows_tets2(const double* __restrict__ geom, const double* __restrict_
             const double glc1 = c == 0 ? gl1[0] : (c == 1 ? gl1[1] : gl1[2]);
             const double wc0 = c == 0 ? w0[0] : (c == 1 ? w0[1] : w0[2]);
             const double wc1 = c == 0 ? w1[0] : (c == 1 ? w1[1] : w1[2]);
-            const double tr = mu * (fma(gl0[0], w0[0], fma(gl0[1], w0[1], gl0[2] * w0[2])) +
-                                    fma(gl1[0], w1[0], fma(gl1[1], w1[1], gl1[2] * w1[2])));
-            if (lane_on) {
-                double* out = acc + so * AT_SLOT + 3 * c;
-                double v[3];
+            if constexpr (MODE == MAT_TENSOR) {
+                // row c of the block: v[d] = sum_{k,l} C_{ckdl} S[k][l] with all nine S[k][l] = sum_li G_li[k] w_li[l];
+                // C is warp-uniform (broadcast loads), lane c picks its three Voigt rows voigt(c, k)
+                const double* __restrict__ Ce = f.C + (int64_t)e * 21;
+                double Cv[21];
 #pragma unroll
-                for (int d = 0; d < 3; ++d) {
-                    const double Scd = fma(glc0, w0[d], glc1 * w1[d]);          // S[c][d]
-                    const double Sdc = fma(gl0[d], wc0, gl1[d] * wc1);          // S[d][c]
-                    v[d] = fma(mu, Sdc, lam * Scd);
+                for (int t = 0; t < 21; ++t) Cv[t] = __ldg(Ce + t);
+                if (lane_on) {
+                    double* out = acc + so * AT_SLOT + 3 * c;
+                    double v[3] = {0.0, 0.0, 0.0};
+#pragma unroll
+                    for (int k = 0; k < 3; ++k) {
+                        const int r0 = voigt(0, k), r1 = voigt(1, k), r2 = voigt(2, k);
+#pragma unroll
+                        for (int l = 0; l < 3; ++l) {
+                            const double Skl = fma(gl0[k], w0[l], gl1[k] * w1[l]);
+#pragma unroll
+                            for (int d = 0; d < 3; ++d) {
+                                const int J = voigt(d, l);
+                                const double ck = c == 0 ? Cv[voigt_packed(r0, J)]
+                                                         : (c == 1 ? Cv[voigt_packed(r1, J)] : Cv[voigt_packed(r2, J)]);
+                                v[d] = fma(ck, Skl, v[d]);
+                            }
+                        }
+                    }
+                    out[0] += detK * v[0];
+                    out[1] += detK * v[1];
+                    out[2] += detK * v[2];
+                    if (c == 0) acc[so * AT_SLOT + 9] += mass_entry<FIELD>(s_mtab[a * NPE + bb], rho) * detM;
                 }
-                out[0] += detK * (c == 0 ? v[0] + tr : v[0]);
-                out[1] += detK * (c == 1 ? v[1] + tr : v[1]);
-                out[2] += detK * (c == 2 ? v[2] + tr : v[2]);
-                if (c == 0) acc[so * AT_SLOT + 9] += mass_entry<FIELD>(s_mtab[a * NPE + bb], rho) * detM;
+            } else {
+                const double tr = mu * (fma(gl0[0], w0[0], fma(gl0[1], w0[1], gl0[2] * w0[2])) +
+                                        fma(gl1[0], w1[0], fma(gl1[1], w1[1], gl1[2] * w1[2])));
+                if (lane_on) {
+                    double* out = acc + so * AT_SLOT + 3 * c;
+                    double v[3];
+#pragma unroll
+                    for (int d = 0; d < 3; ++d) {
+                        const double Scd = fma(glc0, w0[d], glc1 * w1[d]);          // S[c][d]
+                        const double Sdc = fma(gl0[d], wc0, gl1[d] * wc1);          // S[d][c]
+                        v[d] = fma(mu, Sdc, lam * Scd);
+                    }
+                    out[0] += detK * (c == 0 ? v[0] + tr : v[0]);
+                    out[1] += detK * (c == 1 ? v[1] + tr : v[1]);
+                    out[2] += detK * (c == 2 ? v[2] + tr : v[2]);
+                    if (c == 0) acc[so * AT_SLOT + 9] += mass_entry<FIELD>(s_mtab[a * NPE + bb], rho) * detM;
+                }
             }
             __syncwarp();
             pair = pair_next;
@@ -467,53 +525,53 @@ __global__ void k_mass_coo(const double* __restrict__ vertices, const int32_t* _
 
 using namespace ds;
 
-static void assemble_account(int64_t T, int npe, int64_t n_nodes, int64_t nnzb, bool field) {
+static void assemble_account(int64_t T, int npe, int64_t n_nodes, int64_t nnzb, int mode) {
     prof_account(PROF_ASSEMBLE, 2.0 * 9.0 * (double)nnzb * 8.0 + (double)T * npe * 4.0 + (double)n_nodes * 12.0 + (double)T * npe * npe * 4.0 +
-                 (field ? (double)T * 20.0 : 0.0), 0.0);
+                 (mode == MAT_LAME ? (double)T * 20.0 : mode == MAT_TENSOR ? (double)T * (21.0 * 8.0 + 4.0) : 0.0), 0.0);
 }
 
-template <bool FIELD>
+template <int MODE>
 static int assemble_rows(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes, double mu,
                          double lam, const FieldArgs& f, const double* ctab, const double* mtab, const int32_t* brow,
                          const int32_t* contrib_ptr, const int32_t* contrib, int64_t nnzb, double* geom, double* Kval,
                          double* Mblk, cudaStream_t stream) {
     int npe = order == 1 ? 4 : 10;
     ProfScope prof(PROF_ASSEMBLE, stream);
-    assemble_account(T, npe, n_nodes, nnzb, FIELD);
+    assemble_account(T, npe, n_nodes, nnzb, MODE);
     k_tet_geometry<<<(unsigned)ceil_div(T, 128), 128, 0, stream>>>(verts, tets, T, npe, order, geom);
     DS_LAUNCH_CHECK();
     // grid-stride over rows: the per-order tables are staged into shared memory once per CTA
     unsigned blocks = (unsigned)std::min<int64_t>(ceil_div(n_nodes, AS_WARPS), 148 * 12);
     if (order == 1)
-        k_assemble_rows<1, FIELD><<<blocks, 32 * AS_WARPS, 0, stream>>>(geom, ctab, mtab, brow, contrib_ptr, contrib, n_nodes,
+        k_assemble_rows<1, MODE><<<blocks, 32 * AS_WARPS, 0, stream>>>(geom, ctab, mtab, brow, contrib_ptr, contrib, n_nodes,
                                                                         mu, lam, f, Kval, Mblk);
     else
-        k_assemble_rows<2, FIELD><<<blocks, 32 * AS_WARPS, 0, stream>>>(geom, ctab, mtab, brow, contrib_ptr, contrib, n_nodes,
+        k_assemble_rows<2, MODE><<<blocks, 32 * AS_WARPS, 0, stream>>>(geom, ctab, mtab, brow, contrib_ptr, contrib, n_nodes,
                                                                         mu, lam, f, Kval, Mblk);
     DS_LAUNCH_CHECK();
     return DS_OK;
 }
 
-template <bool FIELD>
+template <int MODE>
 static int assemble_tets(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes, double mu,
                          double lam, const FieldArgs& f, const double* ctab, const double* mtab, const int32_t* brow,
                          const int32_t* bcol, const int32_t* contrib_ptr, const int32_t* contrib, const int32_t* slot,
                          int max_deg, int64_t nnzb, double* geom, double* Kval, double* Mblk, cudaStream_t stream) {
     const int npe = 10;
     ProfScope prof(PROF_ASSEMBLE, stream);
-    assemble_account(T, npe, n_nodes, nnzb, FIELD);
+    assemble_account(T, npe, n_nodes, nnzb, MODE);
     k_tet_geometry<<<(unsigned)ceil_div(T, 128), 128, 0, stream>>>(verts, tets, T, npe, order, geom);
     DS_LAUNCH_CHECK();
     const int cap = (max_deg + 3) & ~3;
     const size_t smem = (size_t)(100 * 4 + 100 + (size_t)AT_WARPS * cap * AT_SLOT) * sizeof(double);
-    DS_CUDA(cudaFuncSetAttribute(k_assemble_rows_tets2<FIELD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    DS_CUDA(cudaFuncSetAttribute(k_assemble_rows_tets2<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 1;
-    DS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_assemble_rows_tets2<FIELD>, 32 * AT_WARPS, smem));
+    DS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_assemble_rows_tets2<MODE>, 32 * AT_WARPS, smem));
     int dev = 0, sms = 148;
     DS_CUDA(cudaGetDevice(&dev));
     DS_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     const unsigned blocks = (unsigned)std::min<int64_t>(ceil_div(n_nodes, AT_WARPS), (int64_t)sms * std::max(per_sm, 1));
-    k_assemble_rows_tets2<FIELD><<<blocks, 32 * AT_WARPS, smem, stream>>>(geom, ctab, mtab, brow, bcol, contrib_ptr, contrib,
+    k_assemble_rows_tets2<MODE><<<blocks, 32 * AT_WARPS, smem, stream>>>(geom, ctab, mtab, brow, bcol, contrib_ptr, contrib,
                                                                           slot, n_nodes, cap, mu, lam, f, Kval, Mblk);
     DS_LAUNCH_CHECK();
     return DS_OK;
@@ -529,7 +587,7 @@ extern "C" int ds_assemble_km(const float* verts, const int32_t* tets, int64_t T
     DS_REQUIRE(verts && tets && ctab && mtab && brow && contrib_ptr && contrib && geom && Kval && Mblk,
                "ds_assemble_km: null argument");
     DS_REQUIRE(T > 0 && n_nodes > 0, "ds_assemble_km: empty mesh");
-    return assemble_rows<false>(verts, tets, T, order, n_nodes, mu, lam, FieldArgs{}, ctab, mtab, brow, contrib_ptr, contrib,
+    return assemble_rows<MAT_SCALAR>(verts, tets, T, order, n_nodes, mu, lam, FieldArgs{}, ctab, mtab, brow, contrib_ptr, contrib,
                                 nnzb, geom, Kval, Mblk, (cudaStream_t)stream_);
 }
 
@@ -543,7 +601,7 @@ extern "C" int ds_assemble_km_field(const float* verts, const int32_t* tets, int
     DS_REQUIRE(verts && tets && mu_t && lam_t && rho_t && ctab && m32 && brow && contrib_ptr && contrib && geom && Kval && Mblk,
                "ds_assemble_km_field: null argument");
     DS_REQUIRE(T > 0 && n_nodes > 0, "ds_assemble_km_field: empty mesh");
-    return assemble_rows<true>(verts, tets, T, order, n_nodes, 0.0, 0.0, FieldArgs{mu_t, lam_t, rho_t, m32}, ctab, nullptr,
+    return assemble_rows<MAT_LAME>(verts, tets, T, order, n_nodes, 0.0, 0.0, FieldArgs{mu_t, lam_t, rho_t, m32, nullptr}, ctab, nullptr,
                                brow, contrib_ptr, contrib, nnzb, geom, Kval, Mblk, (cudaStream_t)stream_);
 }
 
@@ -560,7 +618,7 @@ extern "C" int ds_assemble_km_tets(const float* verts, const int32_t* tets, int6
     DS_REQUIRE(T > 0 && n_nodes > 0, "ds_assemble_km_tets: empty mesh");
     DS_REQUIRE(max_deg >= 1 && max_deg <= 256, "ds_assemble_km_tets: max_deg=%d must be in [1, 256] (longer rows: ds_assemble_km)",
                max_deg);
-    return assemble_tets<false>(verts, tets, T, order, n_nodes, mu, lam, FieldArgs{}, ctab, mtab, brow, bcol, contrib_ptr,
+    return assemble_tets<MAT_SCALAR>(verts, tets, T, order, n_nodes, mu, lam, FieldArgs{}, ctab, mtab, brow, bcol, contrib_ptr,
                                 contrib, slot, max_deg, nnzb, geom, Kval, Mblk, (cudaStream_t)stream_);
 }
 
@@ -575,8 +633,38 @@ extern "C" int ds_assemble_km_tets_field(const float* verts, const int32_t* tets
     DS_REQUIRE(T > 0 && n_nodes > 0, "ds_assemble_km_tets_field: empty mesh");
     DS_REQUIRE(max_deg >= 1 && max_deg <= 256,
                "ds_assemble_km_tets_field: max_deg=%d must be in [1, 256] (longer rows: ds_assemble_km_field)", max_deg);
-    return assemble_tets<true>(verts, tets, T, order, n_nodes, 0.0, 0.0, FieldArgs{mu_t, lam_t, rho_t, m32}, ctab, nullptr,
+    return assemble_tets<MAT_LAME>(verts, tets, T, order, n_nodes, 0.0, 0.0, FieldArgs{mu_t, lam_t, rho_t, m32, nullptr}, ctab, nullptr,
                                brow, bcol, contrib_ptr, contrib, slot, max_deg, nnzb, geom, Kval, Mblk, (cudaStream_t)stream_);
+}
+
+extern "C" int ds_assemble_km_tensor(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes,
+                                     const double* C21, const float* rho_t, const double* ctab, const float* m32,
+                                     const int32_t* brow, const int32_t* bcol, const int32_t* contrib_ptr,
+                                     const int32_t* contrib, int64_t nnzb, double* geom, double* Kval, double* Mblk,
+                                     void* stream_) {
+    (void)bcol;
+    DS_REQUIRE(order == 1 || order == 2, "ds_assemble_km_tensor: order must be 1 or 2 (got %d)", order);
+    DS_REQUIRE(verts && tets && C21 && rho_t && ctab && m32 && brow && contrib_ptr && contrib && geom && Kval && Mblk,
+               "ds_assemble_km_tensor: null argument");
+    DS_REQUIRE(T > 0 && n_nodes > 0, "ds_assemble_km_tensor: empty mesh");
+    return assemble_rows<MAT_TENSOR>(verts, tets, T, order, n_nodes, 0.0, 0.0, FieldArgs{nullptr, nullptr, rho_t, m32, C21},
+                                     ctab, nullptr, brow, contrib_ptr, contrib, nnzb, geom, Kval, Mblk, (cudaStream_t)stream_);
+}
+
+extern "C" int ds_assemble_km_tets_tensor(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes,
+                                          const double* C21, const float* rho_t, const double* ctab, const float* m32,
+                                          const int32_t* brow, const int32_t* bcol, const int32_t* contrib_ptr,
+                                          const int32_t* contrib, const int32_t* slot, int max_deg, int64_t nnzb,
+                                          double* geom, double* Kval, double* Mblk, void* stream_) {
+    DS_REQUIRE(order == 2, "ds_assemble_km_tets_tensor: quadratic tets only (order 1 goes through ds_assemble_km_tensor)");
+    DS_REQUIRE(verts && tets && C21 && rho_t && ctab && m32 && brow && bcol && contrib_ptr && contrib && slot && geom && Kval &&
+               Mblk, "ds_assemble_km_tets_tensor: null argument");
+    DS_REQUIRE(T > 0 && n_nodes > 0, "ds_assemble_km_tets_tensor: empty mesh");
+    DS_REQUIRE(max_deg >= 1 && max_deg <= 256,
+               "ds_assemble_km_tets_tensor: max_deg=%d must be in [1, 256] (longer rows: ds_assemble_km_tensor)", max_deg);
+    return assemble_tets<MAT_TENSOR>(verts, tets, T, order, n_nodes, 0.0, 0.0, FieldArgs{nullptr, nullptr, rho_t, m32, C21},
+                                     ctab, nullptr, brow, bcol, contrib_ptr, contrib, slot, max_deg, nnzb, geom, Kval, Mblk,
+                                     (cudaStream_t)stream_);
 }
 
 extern "C" int ds_mass_expand(const int32_t* brow, int64_t n_nodes, int64_t nnzb, const double* Mblk,

@@ -51,6 +51,17 @@ inline int check_cuda(cudaError_t e, const char* what, const char* file, int lin
 
 inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
+// Material of the assembly and shape-gradient kernels: one (mu, lam) for the object, one (mu_t, lam_t) per tet, or one
+// elasticity tensor C_t per tet.
+enum MatMode { MAT_SCALAR = 0, MAT_LAME = 1, MAT_TENSOR = 2 };
+
+// Voigt index of the symmetric pair (i, j): 11 22 33 23 13 12 -> 0 .. 5
+__host__ __device__ constexpr int voigt(int i, int j) { return i == j ? i : 6 - i - j; }
+// position of Voigt entry (I, J) in the 21-entry upper triangle, row by row
+__host__ __device__ constexpr int voigt_packed(int I, int J) {
+    return I <= J ? I * (11 - I) / 2 + J : J * (11 - J) / 2 + I;
+}
+
 // Growable device scratch arena owned by a ds_workspace (the only allocation
 // the library performs; everything else is caller-owned torch memory).
 struct Arena {

@@ -21,11 +21,18 @@
 // m, so the exact integral of a quadratic form phi is |det A|/120 (phi(sum_m F_m) + sum_m phi(F_m)).
 //
 // Material fields.  The same element forms per (tet, mode) give d lambda_i / d(mu_t, lam_t, rho_t) and the element
-// energies (k_material_field); the shape gradient reads (mu_t, lam_t, rho_t) per element (k_eigval_grad_shape<_, true>).
+// energies (k_material_field); the shape gradient reads (mu_t, lam_t, rho_t) per element (k_eigval_grad_shape<_, MAT_LAME>).
+//
+// Elasticity-tensor fields (Voigt convention of csrc/assemble.cu, C_t packed as 21 upper-triangle entries).  With
+// C_{ckdl} the rank-4 form of C_t, e(G) = sum_{p,m} Q_pm[c][d] C_{ckdl} G_p[k] G_m[l], and by the major symmetry of C
+//     de/dG_p[j] = 2 sum_m sum_{c,d,k} Q_pm[c][d] C_{cjdk} G_m[k]                (k_eigval_grad_shape<_, MAT_TENSOR>).
+// d lambda_i / dC_t is the strain Gram E_t,i = int_t eps_V(u_i) eps_V(u_i)^T dV, integrated exactly like the material
+// forms (k_elasticity_field); lambda_i = sum_t <C_t, E_t,i> because the strain energy is quadratic in eps.
 #include "common.cuh"
 #include "../../include/diffsound_sm100.h"
 #include "kernels.cuh"
 #include <cub/cub.cuh>
+#include <type_traits>
 
 namespace ds {
 
@@ -129,22 +136,34 @@ struct GradSmem {
     double Q[GS_WARPS][192];                             // 144 Q entries, 12 dE/dG, 12 G (at 160), 12 dD (at 172)
 };
 
-// Per-tet material of the field variant (ds_eigval_grad_shape_field); unused by the scalar instantiation.
+// tensor fields: one packed elasticity tensor per warp in addition
+template <int ORDER>
+struct GradSmemTensor : GradSmem<ORDER> {
+    double C[GS_WARPS][24];
+};
+
+template <int ORDER, int MODE>
+using GradSmemOf = std::conditional_t<MODE == MAT_TENSOR, GradSmemTensor<ORDER>, GradSmem<ORDER>>;
+
+// Per-tet material of the field variants (ds_eigval_grad_shape_field, ds_eigval_grad_shape_tensor); unused by the
+// scalar instantiation.
 struct GradField {
     const double* __restrict__ mu;
     const double* __restrict__ lam;
     const float* __restrict__ rho;
+    const double* __restrict__ C;   // [T][21]
 };
 
-// FIELD: mu, lam of element e from the field, mtab_g the unit-density table (promoted fp32) and the mass part of the
-// element scaled by rho_e.
-template <int ORDER, bool FIELD>
+// MAT_LAME: mu, lam of element e from the field; MAT_TENSOR: its elasticity tensor.  Both: mtab_g the unit-density table
+// (promoted fp32) and the mass part of the element scaled by rho_e.
+template <int ORDER, int MODE>
 __global__ void __launch_bounds__(GS_WARPS * 32)
 k_eigval_grad_shape(const float* __restrict__ verts, const int32_t* __restrict__ tets, int64_t T, double mu_s,
                     double lam_s, GradField f, const double* __restrict__ ctab_g, const double* __restrict__ mtab_g,
                     const double* __restrict__ U, int64_t ldu, int k, const double* __restrict__ lamv,
                     const double* __restrict__ gv, double* __restrict__ tet_grad) {
-    using SM = GradSmem<ORDER>;
+    using SM = GradSmemOf<ORDER, MODE>;
+    constexpr bool FIELD = MODE != MAT_SCALAR;
     constexpr int NPE = SM::NPE, ROWS = SM::ROWS, RT = SM::RT, RP = SM::RP;
     constexpr int NL = ORDER == 1 ? 1 : 4;
     constexpr int NTILE = RT * (RT + 1) / 2;
@@ -170,8 +189,11 @@ k_eigval_grad_shape(const float* __restrict__ verts, const int32_t* __restrict__
     const int64_t wstride = (int64_t)gridDim.x * GS_WARPS;
     for (int64_t e = (int64_t)blockIdx.x * GS_WARPS + warp; e < T; e += wstride) {
         const int32_t* tp = tets + e * NPE;
-        const double mu = FIELD ? __ldg(f.mu + e) : mu_s;
-        const double lam = FIELD ? __ldg(f.lam + e) : lam_s;
+        const double mu = MODE == MAT_LAME ? __ldg(f.mu + e) : mu_s;
+        const double lam = MODE == MAT_LAME ? __ldg(f.lam + e) : lam_s;
+        if constexpr (MODE == MAT_TENSOR) {
+            if (lane < 21) sm.C[warp][lane] = __ldg(f.C + e * 21 + lane);
+        }
         int32_t cn[4];
         load_corners(tp, ORDER, cn);
         TetGeom geo;
@@ -269,7 +291,31 @@ k_eigval_grad_shape(const float* __restrict__ verts, const int32_t* __restrict__
         __syncwarp();
         // ---- dE/dG (lanes 0..11 = (p, j)) and e = 1/2 G : dE/dG
         double dG = 0.0;
-        if (lane < 12) {
+        if constexpr (MODE == MAT_TENSOR) {
+            if (lane < 12) {
+                const int p = lane / 3, j = lane - 3 * p;
+                const double* Cs = sm.C[warp];
+                double Cj[3][3][3];     // C_{cjdk} of this lane's j
+#pragma unroll
+                for (int c = 0; c < 3; ++c)
+#pragma unroll
+                    for (int d = 0; d < 3; ++d)
+#pragma unroll
+                        for (int k = 0; k < 3; ++k) Cj[c][d][k] = Cs[voigt_packed(voigt(c, j), voigt(d, k))];
+#pragma unroll
+                for (int m = 0; m < 4; ++m) {
+                    const double* Qpm = Qs + (p * 4 + m) * 9;
+                    double s = 0.0;
+#pragma unroll
+                    for (int c = 0; c < 3; ++c)
+#pragma unroll
+                        for (int d = 0; d < 3; ++d)
+                            s = fma(Qpm[3 * c + d],
+                                    fma(Cj[c][d][0], geo.G[m][0], fma(Cj[c][d][1], geo.G[m][1], Cj[c][d][2] * geo.G[m][2])), s);
+                    dG = fma(2.0, s, dG);
+                }
+            }
+        } else if (lane < 12) {
             int p = lane / 3, j = lane - 3 * p;
 #pragma unroll
             for (int m = 0; m < 4; ++m) {
@@ -491,6 +537,49 @@ __global__ void k_quadform_reduce(const double* __restrict__ partial, int nparts
 //         field assembly rounds them (float32(m_ab) * float32(rho_t)).
 constexpr int MF_WARPS = 4;
 
+// u^T Mhat u of one element (the mass form of k_quadforms) with the table entries rounded as the field assembly rounds
+// them, float32(m_ab) * float32(rho), when SCALED
+template <int NPE, bool SCALED>
+__device__ __forceinline__ double elem_mass_form(const float* s_m32, float rho, const double (&u)[NPE][3]) {
+    double ms = 0.0;
+#pragma unroll
+    for (int a = 0; a < NPE; ++a) {
+        double ta[3] = {0.0, 0.0, 0.0};
+#pragma unroll
+        for (int b = a + 1; b < NPE; ++b) {
+            const double mab = SCALED ? (double)__fmul_rn(s_m32[a * NPE + b], rho) : (double)s_m32[a * NPE + b];
+            ta[0] = fma(mab, u[b][0], ta[0]);
+            ta[1] = fma(mab, u[b][1], ta[1]);
+            ta[2] = fma(mab, u[b][2], ta[2]);
+        }
+        const double maa = SCALED ? (double)__fmul_rn(s_m32[a * NPE + a], rho) : (double)s_m32[a * NPE + a];
+#pragma unroll
+        for (int c = 0; c < 3; ++c) ms = fma(u[a][c], fma(maa, u[a][c], 2.0 * ta[c]), ms);
+    }
+    return ms;
+}
+
+// displacement gradient F[r][j] = du_r / dx_j of a quadratic tet at corner m (F is linear in the barycentric coordinates)
+__device__ __forceinline__ void p2_corner_grad(const double (&u)[10][3], const TetGeom& geo, int m, double (&F)[3][3]) {
+    constexpr int CORNER[4] = {0, 2, 4, 9};
+    constexpr int EDGE[4][4] = {{-1, 1, 5, 6}, {1, -1, 3, 7}, {5, 3, -1, 8}, {6, 7, 8, -1}};
+#pragma unroll
+    for (int r = 0; r < 3; ++r)
+#pragma unroll
+        for (int j = 0; j < 3; ++j) F[r][j] = 0.0;
+#pragma unroll
+    for (int l = 0; l < 4; ++l) {
+        double h[3];
+#pragma unroll
+        for (int r = 0; r < 3; ++r)
+            h[r] = (l == m) ? 3.0 * u[CORNER[l]][r] : 4.0 * u[EDGE[l][m] < 0 ? 0 : EDGE[l][m]][r] - u[CORNER[l]][r];
+#pragma unroll
+        for (int r = 0; r < 3; ++r)
+#pragma unroll
+            for (int j = 0; j < 3; ++j) F[r][j] = fma(h[r], geo.G[l][j], F[r][j]);
+    }
+}
+
 template <int ORDER, bool ENERGY>
 __global__ void __launch_bounds__(MF_WARPS * 32)
 k_material_field(const float* __restrict__ verts, const int32_t* __restrict__ tets, int64_t T, const float* __restrict__ m32,
@@ -523,24 +612,9 @@ k_material_field(const float* __restrict__ verts, const int32_t* __restrict__ te
                 for (int c = 0; c < 3; ++c) u[a][c] = on ? __ldg(U + (3 * node + c) * ldu + i) : 0.0;
             }
             // mass form, as k_quadforms
-            double ms = 0.0;
-#pragma unroll
-            for (int a = 0; a < NPE; ++a) {
-                double ta[3] = {0.0, 0.0, 0.0};
-#pragma unroll
-                for (int b = a + 1; b < NPE; ++b) {
-                    const double mab = ENERGY ? (double)__fmul_rn(s_m32[a * NPE + b], rho) : (double)s_m32[a * NPE + b];
-                    ta[0] = fma(mab, u[b][0], ta[0]);
-                    ta[1] = fma(mab, u[b][1], ta[1]);
-                    ta[2] = fma(mab, u[b][2], ta[2]);
-                }
-                const double maa = ENERGY ? (double)__fmul_rn(s_m32[a * NPE + a], rho) : (double)s_m32[a * NPE + a];
-#pragma unroll
-                for (int c = 0; c < 3; ++c) ms = fma(u[a][c], fma(maa, u[a][c], 2.0 * ta[c]), ms);
-            }
-            const double q_m = geo.detM * ms;
+            const double q_m = geo.detM * elem_mass_form<NPE, ENERGY>(s_m32, rho, u);
             double q_mu, q_la;
-            if (ORDER == 1) {
+            if constexpr (ORDER == 1) {
                 double F[3][3];
 #pragma unroll
                 for (int r = 0; r < 3; ++r)
@@ -553,24 +627,12 @@ k_material_field(const float* __restrict__ verts, const int32_t* __restrict__ te
                 q_mu = geo.detK * wsum * pm;
                 q_la = geo.detK * wsum * pl;
             } else {
-                constexpr int CORNER[4] = {0, 2, 4, 9};
-                constexpr int EDGE[4][4] = {{-1, 1, 5, 6}, {1, -1, 3, 7}, {5, 3, -1, 8}, {6, 7, 8, -1}};
                 double S[3][3] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}};
                 double smu = 0.0, sla = 0.0;
 #pragma unroll
                 for (int m = 0; m < 4; ++m) {
-                    double F[3][3] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}};
-#pragma unroll
-                    for (int l = 0; l < 4; ++l) {
-                        double h[3];
-#pragma unroll
-                        for (int r = 0; r < 3; ++r)
-                            h[r] = (l == m) ? 3.0 * u[CORNER[l]][r] : 4.0 * u[EDGE[l][m] < 0 ? 0 : EDGE[l][m]][r] - u[CORNER[l]][r];
-#pragma unroll
-                        for (int r = 0; r < 3; ++r)
-#pragma unroll
-                            for (int j = 0; j < 3; ++j) F[r][j] = fma(h[r], geo.G[l][j], F[r][j]);
-                    }
+                    double F[3][3];
+                    p2_corner_grad(u, geo, m, F);
                     double pm, pl;
                     phi_pair(F, pm, pl);
                     smu += pm;
@@ -609,6 +671,129 @@ k_material_field(const float* __restrict__ verts, const int32_t* __restrict__ te
                 out[3 * e + 0] = a_mu;
                 out[3 * e + 1] = a_la;
                 out[3 * e + 2] = a_m;
+            }
+        }
+    }
+}
+
+// ---------------------------------------------------------------------------
+// elasticity-tensor gradient and element energies
+// ---------------------------------------------------------------------------
+// The sibling of k_material_field for tensor fields: one warp per tet, lane = mode (chunks of 32 modes).  Per (tet, mode)
+// the strain Gram E = int_t eps_V eps_V^T dV (21 packed entries): |det A| wsum phi(F) for linear tets, the vertex rule
+// |det A| / 120 (phi(sum_m F_m) + sum_m phi(F_m)) for quadratic ones, phi(F) = eps_V(F) eps_V(F)^T.
+// GRAD:   outC[t] = sum_i g_i E_t,i (21 entries), out2[t] = -sum_i g_i lam_i q_m, summed over the lanes by a fixed
+//         xor-shuffle tree -- no atomics, bitwise reproducible.
+// ENERGY: outC[t, i] = <C_t, E_t,i> (strain), out2[t, i] = u^T M_t u (kinetic, mass entries float32(m_ab) * float32(rho_t)).
+
+// e += phi(F): the packed upper triangle of eps_V eps_V^T, eps_V = (F00, F11, F22, F12 + F21, F02 + F20, F01 + F10)
+__device__ __forceinline__ void add_strain_gram(const double (&F)[3][3], double (&e)[21]) {
+    const double v[6] = {F[0][0], F[1][1], F[2][2], F[1][2] + F[2][1], F[0][2] + F[2][0], F[0][1] + F[1][0]};
+#pragma unroll
+    for (int I = 0; I < 6; ++I)
+#pragma unroll
+        for (int J = I; J < 6; ++J) e[voigt_packed(I, J)] = fma(v[I], v[J], e[voigt_packed(I, J)]);
+}
+
+template <int ORDER, bool ENERGY>
+__global__ void __launch_bounds__(MF_WARPS * 32)
+k_elasticity_field(const float* __restrict__ verts, const int32_t* __restrict__ tets, int64_t T, const float* __restrict__ m32,
+                   double wsum, const double* __restrict__ U, int64_t ldu, int k, const double* __restrict__ lamv,
+                   const double* __restrict__ gv, const double* __restrict__ C21, const float* __restrict__ rho_t,
+                   double* __restrict__ outC, double* __restrict__ out2) {
+    constexpr int NPE = ORDER == 1 ? 4 : 10;
+    __shared__ float s_m32[NPE * NPE];
+    for (int t = threadIdx.x; t < NPE * NPE; t += blockDim.x) s_m32[t] = m32[t];
+    __syncthreads();
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int64_t wstride = (int64_t)gridDim.x * MF_WARPS;
+    const int kpad = (k + 31) & ~31;
+    for (int64_t e = (int64_t)blockIdx.x * MF_WARPS + warp; e < T; e += wstride) {
+        const int32_t* tp = tets + e * NPE;
+        int32_t cn[4];
+        load_corners(tp, ORDER, cn);
+        TetGeom geo;
+        tet_geometry<false>(verts, cn, geo);
+        const float rho = ENERGY ? __ldg(rho_t + e) : 1.0f;
+        double Cw[21];          // ENERGY: C_t with the off-diagonal entries doubled, so that <C, E> = sum_p Cw[p] E[p]
+        if (ENERGY) {
+#pragma unroll
+            for (int I = 0; I < 6; ++I)
+#pragma unroll
+                for (int J = I; J < 6; ++J) {
+                    const int p = voigt_packed(I, J);
+                    Cw[p] = (I == J ? 1.0 : 2.0) * __ldg(C21 + e * 21 + p);
+                }
+        }
+        double acc[21], a_m = 0.0;
+#pragma unroll
+        for (int p = 0; p < 21; ++p) acc[p] = 0.0;
+        for (int i0 = 0; i0 < kpad; i0 += 32) {
+            const int i = i0 + lane;
+            const bool on = i < k;
+            double u[NPE][3];
+#pragma unroll
+            for (int a = 0; a < NPE; ++a) {
+                const int64_t node = __ldg(tp + a);
+#pragma unroll
+                for (int c = 0; c < 3; ++c) u[a][c] = on ? __ldg(U + (3 * node + c) * ldu + i) : 0.0;
+            }
+            const double q_m = geo.detM * elem_mass_form<NPE, ENERGY>(s_m32, rho, u);
+            double E[21];
+#pragma unroll
+            for (int p = 0; p < 21; ++p) E[p] = 0.0;
+            double w;
+            if constexpr (ORDER == 1) {
+                double F[3][3];
+#pragma unroll
+                for (int r = 0; r < 3; ++r)
+#pragma unroll
+                    for (int j = 0; j < 3; ++j)
+                        F[r][j] = u[0][r] * geo.G[0][j] + u[1][r] * geo.G[1][j] + u[2][r] * geo.G[2][j] +
+                                  u[3][r] * geo.G[3][j];
+                add_strain_gram(F, E);
+                w = geo.detK * wsum;
+            } else {
+                double S[3][3] = {{0, 0, 0}, {0, 0, 0}, {0, 0, 0}};
+#pragma unroll
+                for (int m = 0; m < 4; ++m) {
+                    double F[3][3];
+                    p2_corner_grad(u, geo, m, F);
+                    add_strain_gram(F, E);
+#pragma unroll
+                    for (int r = 0; r < 3; ++r)
+#pragma unroll
+                        for (int j = 0; j < 3; ++j) S[r][j] += F[r][j];
+                }
+                add_strain_gram(S, E);
+                w = geo.detK * (1.0 / 120.0);
+            }
+            if (ENERGY) {
+                if (on) {
+                    double en = 0.0;
+#pragma unroll
+                    for (int p = 0; p < 21; ++p) en = fma(Cw[p], E[p], en);
+                    __stcs(outC + e * k + i, w * en);
+                    __stcs(out2 + e * k + i, q_m);
+                }
+            } else if (on) {
+                const double gw = __ldg(gv + i) * w;
+#pragma unroll
+                for (int p = 0; p < 21; ++p) acc[p] = fma(gw, E[p], acc[p]);
+                a_m = fma(-__ldg(gv + i) * __ldg(lamv + i), q_m, a_m);
+            }
+        }
+        if (!ENERGY) {
+#pragma unroll
+            for (int off = 16; off > 0; off >>= 1) {
+#pragma unroll
+                for (int p = 0; p < 21; ++p) acc[p] += __shfl_xor_sync(0xffffffffu, acc[p], off);
+                a_m += __shfl_xor_sync(0xffffffffu, a_m, off);
+            }
+            if (lane == 0) {
+#pragma unroll
+                for (int p = 0; p < 21; ++p) outC[21 * e + p] = acc[p];
+                out2[e] = a_m;
             }
         }
     }
@@ -653,7 +838,7 @@ extern "C" int ds_corner_incidence(ds_workspace* ws, const int32_t* tets, int64_
     return DS_OK;
 }
 
-template <bool FIELD>
+template <int MODE>
 static int grad_shape(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes, double mu,
                       double lam_lame, const GradField& f, const double* ctab, const double* mtab, const double* U,
                       int64_t ldu, int k, const double* lam, const double* g, const int32_t* inc_ptr, const int32_t* inc,
@@ -664,19 +849,19 @@ static int grad_shape(const float* verts, const int32_t* tets, int64_t T, int or
         // derivatives, ~ 2 (3 npe)^2 x 12 / 4 (counted from the kernel's DMMA tiles in DESIGN.md)
         const int npe_ = order == 1 ? 4 : 10;
         prof_account(PROF_GRAD, (double)n_nodes * 3.0 * k * 8.0 + (double)T * npe_ * 4.0 + (double)n_nodes * 36.0 +
-                     (FIELD ? (double)T * 20.0 : 0.0), 0.0);
+                     (MODE == MAT_LAME ? (double)T * 20.0 : MODE == MAT_TENSOR ? (double)T * (21.0 * 8.0 + 4.0) : 0.0), 0.0);
     }
     int64_t ctas64 = ceil_div(T, GS_WARPS);
     int ctas = (int)(ctas64 < 148 * 8 ? ctas64 : 148 * 8);
     if (order == 1) {
-        size_t smem = sizeof(GradSmem<1>) + 2 * kpad * sizeof(double);
-        DS_CUDA(cudaFuncSetAttribute(k_eigval_grad_shape<1, FIELD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_eigval_grad_shape<1, FIELD><<<ctas, GS_WARPS * 32, smem, stream>>>(verts, tets, T, mu, lam_lame, f, ctab, mtab, U, ldu,
+        size_t smem = sizeof(GradSmemOf<1, MODE>) + 2 * kpad * sizeof(double);
+        DS_CUDA(cudaFuncSetAttribute(k_eigval_grad_shape<1, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        k_eigval_grad_shape<1, MODE><<<ctas, GS_WARPS * 32, smem, stream>>>(verts, tets, T, mu, lam_lame, f, ctab, mtab, U, ldu,
                                                                              k, lam, g, tet_grad);
     } else {
-        size_t smem = sizeof(GradSmem<2>) + 2 * kpad * sizeof(double);
-        DS_CUDA(cudaFuncSetAttribute(k_eigval_grad_shape<2, FIELD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_eigval_grad_shape<2, FIELD><<<ctas, GS_WARPS * 32, smem, stream>>>(verts, tets, T, mu, lam_lame, f, ctab, mtab, U, ldu,
+        size_t smem = sizeof(GradSmemOf<2, MODE>) + 2 * kpad * sizeof(double);
+        DS_CUDA(cudaFuncSetAttribute(k_eigval_grad_shape<2, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        k_eigval_grad_shape<2, MODE><<<ctas, GS_WARPS * 32, smem, stream>>>(verts, tets, T, mu, lam_lame, f, ctab, mtab, U, ldu,
                                                                              k, lam, g, tet_grad);
     }
     DS_LAUNCH_CHECK();
@@ -695,7 +880,7 @@ extern "C" int ds_eigval_grad_shape(const float* verts, const int32_t* tets, int
     DS_REQUIRE(verts && tets && ctab && mtab && U && lam && g && inc_ptr && inc && tet_grad && grad_verts,
                "ds_eigval_grad_shape: null argument");
     DS_REQUIRE(T > 0 && n_nodes > 0 && k > 0 && k <= 1024 && ldu >= k, "ds_eigval_grad_shape: bad sizes");
-    return grad_shape<false>(verts, tets, T, order, n_nodes, mu, lam_lame, GradField{}, ctab, mtab, U, ldu, k, lam, g, inc_ptr,
+    return grad_shape<MAT_SCALAR>(verts, tets, T, order, n_nodes, mu, lam_lame, GradField{}, ctab, mtab, U, ldu, k, lam, g, inc_ptr,
                              inc, tet_grad, grad_verts, (cudaStream_t)stream_);
 }
 
@@ -708,7 +893,7 @@ extern "C" int ds_eigval_grad_shape_field(const float* verts, const int32_t* tet
     DS_REQUIRE(verts && tets && mu_t && lam_t && rho_t && ctab && mtab1 && U && lam && g && inc_ptr && inc && tet_grad &&
                grad_verts, "ds_eigval_grad_shape_field: null argument");
     DS_REQUIRE(T > 0 && n_nodes > 0 && k > 0 && k <= 1024 && ldu >= k, "ds_eigval_grad_shape_field: bad sizes");
-    return grad_shape<true>(verts, tets, T, order, n_nodes, 0.0, 0.0, GradField{mu_t, lam_t, rho_t}, ctab, mtab1, U, ldu, k, lam,
+    return grad_shape<MAT_LAME>(verts, tets, T, order, n_nodes, 0.0, 0.0, GradField{mu_t, lam_t, rho_t, nullptr}, ctab, mtab1, U, ldu, k, lam,
                             g, inc_ptr, inc, tet_grad, grad_verts, (cudaStream_t)stream_);
 }
 
@@ -753,6 +938,61 @@ extern "C" int ds_element_energies(const float* verts, const int32_t* tets, int6
     DS_REQUIRE(T > 0 && k > 0 && ldu >= k, "ds_element_energies: bad sizes");
     return material_field<true>(verts, tets, T, order, m32, wsum, U, ldu, k, nullptr, nullptr, mu_t,
                                 lam_t, rho_t, strain, kinetic, (cudaStream_t)stream_);
+}
+
+template <bool ENERGY>
+static int elasticity_field(const float* verts, const int32_t* tets, int64_t T, int order, const float* m32, double wsum,
+                            const double* U, int64_t ldu, int k, const double* lam, const double* g, const double* C21,
+                            const float* rho_t, double* outC, double* out2, cudaStream_t stream) {
+    ProfScope prof(PROF_MATERIAL_FIELD, stream);
+    {   // U rows of every tet (re-read per tet: L2), geometry, per-tet tensor / outputs
+        const int npe = order == 1 ? 4 : 10;
+        prof_account(PROF_MATERIAL_FIELD, (double)T * (npe * 3.0 * k * 8.0 + npe * 4.0 + 48.0) +
+                     (ENERGY ? (double)T * (21.0 * 8.0 + 4.0 + 16.0 * k) : (double)T * 22.0 * 8.0), 0.0);
+    }
+    const int64_t ctas64 = ceil_div(T, MF_WARPS);
+    const unsigned ctas = (unsigned)(ctas64 < 148 * 16 ? ctas64 : 148 * 16);
+    if (order == 1)
+        k_elasticity_field<1, ENERGY><<<ctas, MF_WARPS * 32, 0, stream>>>(verts, tets, T, m32, wsum, U, ldu, k, lam, g, C21,
+                                                                          rho_t, outC, out2);
+    else
+        k_elasticity_field<2, ENERGY><<<ctas, MF_WARPS * 32, 0, stream>>>(verts, tets, T, m32, wsum, U, ldu, k, lam, g, C21,
+                                                                          rho_t, outC, out2);
+    DS_LAUNCH_CHECK();
+    return DS_OK;
+}
+
+extern "C" int ds_eigval_grad_shape_tensor(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes,
+                                           const double* C21, const float* rho_t, const double* ctab, const double* mtab1,
+                                           const double* U, int64_t ldu, int k, const double* lam, const double* g,
+                                           const int32_t* inc_ptr, const int32_t* inc, double* tet_grad, float* grad_verts,
+                                           void* stream_) {
+    DS_REQUIRE(order == 1 || order == 2, "ds_eigval_grad_shape_tensor: order must be 1 or 2 (got %d)", order);
+    DS_REQUIRE(verts && tets && C21 && rho_t && ctab && mtab1 && U && lam && g && inc_ptr && inc && tet_grad && grad_verts,
+               "ds_eigval_grad_shape_tensor: null argument");
+    DS_REQUIRE(T > 0 && n_nodes > 0 && k > 0 && k <= 1024 && ldu >= k, "ds_eigval_grad_shape_tensor: bad sizes");
+    return grad_shape<MAT_TENSOR>(verts, tets, T, order, n_nodes, 0.0, 0.0, GradField{nullptr, nullptr, rho_t, C21}, ctab, mtab1,
+                                  U, ldu, k, lam, g, inc_ptr, inc, tet_grad, grad_verts, (cudaStream_t)stream_);
+}
+
+extern "C" int ds_elasticity_field_grad(const float* verts, const int32_t* tets, int64_t T, int order, const float* m32,
+                                        double wsum, const double* U, int64_t ldu, int k, const double* lam, const double* g,
+                                        double* outC, double* out_rho, void* stream_) {
+    DS_REQUIRE(order == 1 || order == 2, "ds_elasticity_field_grad: order must be 1 or 2 (got %d)", order);
+    DS_REQUIRE(verts && tets && m32 && U && lam && g && outC && out_rho, "ds_elasticity_field_grad: null argument");
+    DS_REQUIRE(T > 0 && k > 0 && ldu >= k, "ds_elasticity_field_grad: bad sizes");
+    return elasticity_field<false>(verts, tets, T, order, m32, wsum, U, ldu, k, lam, g, nullptr, nullptr, outC, out_rho,
+                                   (cudaStream_t)stream_);
+}
+
+extern "C" int ds_element_energies_tensor(const float* verts, const int32_t* tets, int64_t T, int order, const float* m32,
+                                          double wsum, const double* U, int64_t ldu, int k, const double* C21,
+                                          const float* rho_t, double* strain, double* kinetic, void* stream_) {
+    DS_REQUIRE(order == 1 || order == 2, "ds_element_energies_tensor: order must be 1 or 2 (got %d)", order);
+    DS_REQUIRE(verts && tets && m32 && U && C21 && rho_t && strain && kinetic, "ds_element_energies_tensor: null argument");
+    DS_REQUIRE(T > 0 && k > 0 && ldu >= k, "ds_element_energies_tensor: bad sizes");
+    return elasticity_field<true>(verts, tets, T, order, m32, wsum, U, ldu, k, nullptr, nullptr, C21, rho_t, strain, kinetic,
+                                  (cudaStream_t)stream_);
 }
 
 extern "C" int64_t ds_quadform_scratch_elems(int k) { return (int64_t)QF_MAX_CTAS * QF_WARPS * 3 * k; }

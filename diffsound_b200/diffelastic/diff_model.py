@@ -35,6 +35,11 @@ def _lame(youngs, poisson):
     return lame_mu, lame_lambda
 
 
+# packed upper triangle of a 6x6 Voigt matrix, row by row (the 21 values per tet the tensor kernels read), and back
+_IU = torch.triu_indices(6, 6)
+_VOIGT_UNPACK = torch.tensor([[min(i, j) * (11 - min(i, j)) // 2 + max(i, j) for j in range(6)] for i in range(6)])
+
+
 def _stress(F, lame_mu, lame_lambda):
     """P = mu (F + F^T) + lambda tr(F) I   (diff_model.py:39-41)."""
     tr = F.diagonal(dim1=-2, dim2=-1).sum(-1)
@@ -161,6 +166,31 @@ def check_material_field(num_tets, device, youngs=None, poisson=None, density=No
             raise ValueError(f"set_material_field: {name} violates {cond}")
 
 
+def check_elasticity_field(num_tets, device, C, density=None):
+    """Host validation of an elasticity-tensor field (DiffSoundObj.set_elasticity_field): C a finite fp32 / fp64
+    (num_tets, 6, 6) tensor on `device`, symmetric to 1e-10 max|C| and positive definite in every tet (a Cholesky
+    factorisation on the device); density None or a finite positive fp32 / fp64 (num_tets,) tensor on `device`.  Raises
+    ValueError otherwise."""
+    if not torch.is_tensor(C) or C.dtype not in (torch.float32, torch.float64):
+        raise ValueError("set_elasticity_field: C must be a float32 or float64 tensor")
+    if C.shape != (num_tets, 6, 6):
+        raise ValueError(f"set_elasticity_field: C has shape {tuple(C.shape)}, expected ({num_tets}, 6, 6): one Voigt matrix "
+                         "per row of tetmesh.tets")
+    if C.device != torch.device(device):
+        raise ValueError(f"set_elasticity_field: C is on {C.device}, the mesh on {device}")
+    x = C.detach().to(torch.float64)
+    if not bool(torch.isfinite(x).all()):
+        raise ValueError("set_elasticity_field: C has non-finite values")
+    if not bool(((x - x.transpose(1, 2)).abs().amax() <= 1e-10 * x.abs().amax())):
+        raise ValueError("set_elasticity_field: C is not symmetric (to 1e-10 max|C|)")
+    _, info = torch.linalg.cholesky_ex(0.5 * (x + x.transpose(1, 2)))
+    bad = torch.nonzero(info).flatten()
+    if bad.numel():
+        raise ValueError(f"set_elasticity_field: C is not positive definite in {bad.numel()} tets (first: tet {int(bad[0])})")
+    if density is not None:
+        check_material_field(num_tets, device, density=density)
+
+
 def material_field_from_regions(labels, materials):
     """(youngs, poisson, density), each (T,) fp64 on the device of `labels`: the material `materials[labels[t]]` (MatSet
     tuples) of every tet, for DiffSoundObj.set_material_field."""
@@ -270,6 +300,43 @@ class _EigvalField(torch.autograd.Function):
             if ctx.needs_input_grad[3]:
                 grho = G[:, 2].to(ctx.dtypes[2])
         return gverts, gE, gnu, grho, None
+
+
+class _EigvalTensor(torch.autograd.Function):
+    """get_vals() of an object with an elasticity-tensor field: the value of _EigvalShape, gradients u^T (dK - lambda dM) u
+    to the vertices (native.eigval_grad_shape_tensor, C fixed in world axes), to C (the symmetric strain Gram
+    sum_i g_i E_t,i of native.elasticity_field_grad, unpacked to (T, 6, 6)) and to the density.  The tensors, eigenpairs
+    and geometry the assembly used are pinned at forward time, as in _EigvalShape."""
+
+    @staticmethod
+    def forward(ctx, vertices, C, density, obj):
+        lam = obj.eigenvalues
+        d = obj.deform
+        predict = _vals_forward(obj)
+        f = obj._tensor_used
+        ctx.order, ctx.wsum = obj.tetmesh.order, d.wsum
+        ctx.vdtype = obj.tetmesh.vertices.dtype
+        ctx.dtypes = (C.dtype, None if density is None else density.dtype)
+        ctx.U = obj.U_hat
+        inc_ptr, inc = d.incidence
+        ctx.save_for_backward(obj._verts32, d.tets_i32, d.ctab, d.mtab(1.0), d.m32(), lam, inc_ptr, inc, f["C21"], f["rho"])
+        return predict.unsqueeze(1)
+
+    @staticmethod
+    def backward(ctx, g):
+        verts32, tets, ctab, mtab1, m32, lam, inc_ptr, inc, C21, rho_t = ctx.saved_tensors
+        gv = g.reshape(-1).to(torch.float64).contiguous()
+        gverts = gC = grho = None
+        if ctx.needs_input_grad[0]:
+            gverts = native.eigval_grad_shape_tensor(verts32, tets, ctx.order, (C21, rho_t), ctab, mtab1, ctx.U, lam, gv,
+                                                     inc_ptr, inc).to(ctx.vdtype)
+        if ctx.needs_input_grad[1] or ctx.needs_input_grad[2]:
+            G21, G_rho = native.elasticity_field_grad(verts32, tets, ctx.order, m32, ctx.wsum, ctx.U, lam, gv)
+            if ctx.needs_input_grad[1]:
+                gC = G21[:, _VOIGT_UNPACK].to(ctx.dtypes[0])
+            if ctx.needs_input_grad[2]:
+                grho = G_rho.to(ctx.dtypes[1])
+        return gverts, gC, grho, None
 
 
 class _StiffFunc(torch.autograd.Function):
@@ -391,6 +458,8 @@ class DiffSoundObj:
         self._fixed_u8 = None
         self.material_field = None      # (youngs, poisson, density) of set_material_field, None: one material
         self._field_used = None
+        self.elasticity_field = None    # (C, density) of set_elasticity_field, None: isotropic
+        self._tensor_used = None
 
     # ------------------------------------------------------------------ parameters
     def parameters(self):
@@ -434,6 +503,18 @@ class DiffSoundObj:
                else dens.detach().to(torch.float32).clone())
         return dict(youngs=E, poisson=nu, mu=mu_t.contiguous(), lam=lam_t.contiguous(), rho=rho.contiguous())
 
+    def _tensor_snapshot(self, density):
+        """The elasticity-tensor field the next assembly uses, validated again: C symmetrised in fp64 (T, 6, 6), its packed
+        upper triangle C21 (T, 21) and fp32 rho (density None: `density`)."""
+        C, dens = self.elasticity_field
+        d = self.deform
+        check_elasticity_field(d.num_tets, d.device, C, dens)
+        x = C.detach().to(torch.float64)
+        Cs = 0.5 * (x + x.transpose(1, 2))
+        rho = (torch.full((d.num_tets,), float(density), dtype=torch.float32, device=d.device) if dens is None
+               else dens.detach().to(torch.float32).clone())
+        return dict(C=Cs, C21=Cs[:, _IU[0], _IU[1]].contiguous(), rho=rho.contiguous())
+
     def _assemble(self, density):
         d = self.deform
         mu, lam = self.material_model.lame()
@@ -442,7 +523,15 @@ class DiffSoundObj:
         pat = d.pattern
         if "_geom" not in self.__dict__:
             self._geom = torch.empty(d.num_tets * 14, dtype=torch.float64, device=d.device)
-        if self.material_field is None:
+        self._tensor_used = None
+        if self.elasticity_field is not None:
+            self._field_used = None
+            t = self._tensor_snapshot(density)
+            self._tensor_used = t
+            self._Kval, self._Mblk = native.assemble_km(self._verts32, d.tets_i32, self.tetmesh.order, pat, 0.0, 0.0, d.ctab,
+                                                        d.m32(), Kval=self._Kval, Mblk=self._Mblk, geom=self._geom,
+                                                        tensor=(t["C21"], t["rho"]))
+        elif self.material_field is None:
             self._field_used = None
             self._Kval, self._Mblk = native.assemble_km(self._verts32, d.tets_i32, self.tetmesh.order, pat, mu, lam, d.ctab,
                                                         d.mtab(density), Kval=self._Kval, Mblk=self._Mblk, geom=self._geom)
@@ -494,6 +583,9 @@ class DiffSoundObj:
         if self.material_field is not None:
             raise NotImplementedError("stiff_func: K = mu K_mu + lam K_lam with one (mu, lam) for the whole object; it is not "
                                       "defined for a material field (set_material_field(None) first)")
+        if self.elasticity_field is not None:
+            raise NotImplementedError("stiff_func: K = mu K_mu + lam K_lam with one (mu, lam) for the whole object; it is not "
+                                      "defined for an elasticity-tensor field (set_elasticity_field(None) first)")
         x = x_in.unsqueeze(1) if x_in.dim() == 1 else x_in
         mu, lam = self.material_model.lame()
         mu = torch.as_tensor(mu, dtype=torch.float32).to(x.device)
@@ -555,8 +647,43 @@ class DiffSoundObj:
             if isinstance(self.material_model, TrainableLinear):
                 raise ValueError("set_material_field: the material model is TrainableLinear, whose global (E, nu) logits "
                                  "would compete with a per-tet field; build the object with FixedLinear")
+            if self.elasticity_field is not None:
+                raise ValueError("set_material_field: an elasticity-tensor field is set and both define the stiffness; "
+                                 "clear it first (set_elasticity_field(None))")
             check_material_field(self.deform.num_tets, self.deform.device, youngs, poisson, density)
             self.material_field = (youngs, poisson, density)
+        self._q = None
+        for key in ("_stiff_coo", "_mass_coo"):
+            self.__dict__.pop(key, None)
+        if self._Kval is not None:
+            self._assemble(self._density_used)
+
+    def set_elasticity_field(self, C, density=None):
+        """Give every tet its own anisotropic material: C (T, 6, 6) fp32 / fp64 CUDA tensor of elasticity matrices over the
+        rows of `tetmesh.tets`, and optionally density (T,) (None: the material's scalar).  Voigt order (11, 22, 33, 23, 13,
+        12) with engineering shear strains, eps_V = (e11, e22, e33, 2 e23, 2 e13, 2 e12), sigma_V = C eps_V, strain energy
+        1/2 int eps_V^T C_t eps_V dV; C is in the global (mesh) frame and does not turn with the vertices.  One material
+        everywhere is C0.expand(T, 6, 6); diffelastic.anisotropic builds isotropic, orthotropic and rotated tensors.
+        `set_elasticity_field(None)` clears the field (and drops the warm start, so the object then solves exactly as the
+        isotropic one).
+
+        The tensors are kept by reference and validated at every assembly (shape, dtype, device, finite, symmetric to
+        1e-10 max|C|, positive definite per tet); C is symmetrised before use.  get_vals() is then differentiable in the
+        vertices, C (d lambda_i / dC_t is the symmetric strain Gram int_t eps_V eps_V^T of mode i) and density.  The mass
+        entries round as with set_material_field.  Raises ValueError on a TrainableLinear material model or while a
+        set_material_field field is set: both would define the stiffness."""
+        if C is None:
+            self.elasticity_field = None
+            self._warm = []
+        else:
+            if isinstance(self.material_model, TrainableLinear):
+                raise ValueError("set_elasticity_field: the material model is TrainableLinear, whose global (E, nu) logits "
+                                 "would compete with a per-tet tensor; build the object with FixedLinear")
+            if self.material_field is not None:
+                raise ValueError("set_elasticity_field: a material field is set and both define the stiffness; clear it "
+                                 "first (set_material_field(None))")
+            check_elasticity_field(self.deform.num_tets, self.deform.device, C, density)
+            self.elasticity_field = (C, density)
         self._q = None
         for key in ("_stiff_coo", "_mass_coo"):
             self.__dict__.pop(key, None)
@@ -570,6 +697,10 @@ class DiffSoundObj:
         if getattr(self, "U_hat", None) is None:
             raise RuntimeError("element_energies: run eigen_decomposition() first")
         d = self.deform
+        if self._tensor_used is not None:
+            t = self._tensor_used
+            return native.element_energies_tensor(self._verts32, d.tets_i32, self.tetmesh.order, d.m32(), d.wsum, self.U_hat,
+                                                  (t["C21"], t["rho"]))
         f = self._field_used
         if f is None:
             mu, lam = self._lame_used
@@ -657,7 +788,10 @@ class DiffSoundObj:
             # two-level p-multigrid preconditioner: P1 operator of the same mesh, same material
             mu, la = self._lame_used
             coarse.fixed = None if self._fixed_u8 is None else self._fixed_u8[coarse.corner_nodes].contiguous()
-            if self._field_used is None:
+            if self._tensor_used is not None:       # coarse tet t is fine tet t: the same per-tet arrays
+                t = self._tensor_used
+                coarse.assemble(self._verts32, 0.0, 0.0, coarse.ctab, self.deform.m32(1), tensor=(t["C21"], t["rho"]))
+            elif self._field_used is None:
                 coarse.assemble(self._verts32, mu, la, coarse.ctab, self.deform.coarse_mtab(self._density_used))
             else:       # coarse tet t is fine tet t: the same per-tet arrays
                 f = self._field_used
@@ -756,8 +890,9 @@ class DiffSoundObj:
         dev = self.deform.device
         predict = torch.zeros(self.mode_num, dtype=torch.float32, device=dev)
         predict += self.eigenvalues
-        # with a material field the global (E, nu) are not parameters of K (and TrainableLinear is refused): no term to add
-        if self.task != "gt" and self._field_used is None:
+        # with a material or tensor field the global (E, nu) are not parameters of K (and TrainableLinear is refused): no
+        # term to add
+        if self.task != "gt" and self._field_used is None and self._tensor_used is None:
             q_mu, q_la, q_m = self._material_forms()
             mu, lam = self.material_model.lame()
             mu, lam = torch.as_tensor(mu).to(dev), torch.as_tensor(lam).to(dev)
@@ -768,7 +903,10 @@ class DiffSoundObj:
 
     def get_vals(self):
         """(mode_num, 1) fp32 eigenvalues, differentiable w.r.t. the vertex positions
-        (diff_model.py:390-399) and, with a material field, w.r.t. its tensors."""
+        (diff_model.py:390-399) and, with a material or elasticity-tensor field, w.r.t. its tensors."""
+        if self._tensor_used is not None:
+            C, density = self.elasticity_field if self.elasticity_field is not None else (self._tensor_used["C"], None)
+            return _EigvalTensor.apply(self.tetmesh.vertices, C, density, self)
         if self._field_used is not None:
             youngs, poisson, density = self.material_field if self.material_field is not None else (None, None, None)
             return _EigvalField.apply(self.tetmesh.vertices, youngs, poisson, density, self)

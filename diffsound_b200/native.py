@@ -156,13 +156,23 @@ def _check_field(field, T, dev):
     return _p(mu_t), _p(lam_t), _p(rho_t)
 
 
+def _check_tensor(tensor, T, dev):
+    C21, rho_t = tensor
+    for name, t, shape, dt in (("C21", C21, (T, 21), torch.float64), ("rho", rho_t, (T,), torch.float32)):
+        if t.dtype != dt or t.shape != shape or t.device != dev or not t.is_contiguous():
+            raise ValueError(f"elasticity field: {name} must be a contiguous {shape} {dt} tensor on {dev}")
+    return _p(C21), _p(rho_t)
+
+
 def assemble_km(verts_f32, tets_i32, order, pattern, mu, lam, ctab, mtab, Kval=None, Mblk=None, geom=None, kernel=None,
-                field=None):
+                field=None, tensor=None):
     """K (scalar-CSR value order of the reference) and M (one scalar per block) into the fixed pattern.  kernel: 'tets'
     (tet-sequential rows: quadratic meshes whose pattern carries the slot map and whose rows have <= 256 blocks), 'rows'
     (balanced contributor lists: everything else) or None = pick.
     field: (mu_t (T,) fp64, lam_t (T,) fp64, rho_t (T,) fp32) one material per tet (ds_assemble_km_field /
-    ds_assemble_km_tets_field); mu and lam are then ignored and mtab is the fp32 unit-density mass table (npe, npe)."""
+    ds_assemble_km_tets_field); mu and lam are then ignored and mtab is the fp32 unit-density mass table (npe, npe).
+    tensor: (C21 (T, 21) fp64 packed Voigt elasticity matrices, rho_t (T,) fp32) one anisotropic material per tet
+    (ds_assemble_km_tensor / ds_assemble_km_tets_tensor); mu, lam and mtab as for `field`."""
     lib = _lib.load()
     dev = verts_f32.device
     assert verts_f32.dtype == torch.float32 and tets_i32.dtype == torch.int32
@@ -180,6 +190,21 @@ def assemble_km(verts_f32, tets_i32, order, pattern, mu, lam, ctab, mtab, Kval=N
     if kernel == "tets":
         if not can_tets:
             raise ValueError("assemble_km(kernel='tets') needs a quadratic mesh, Pattern(want_slot=True) and rows of <= 256 blocks")
+    if tensor is not None:
+        assert field is None and mtab.dtype == torch.float32
+        tp = _check_tensor(tensor, T, dev)
+        with torch.cuda.device(dev):
+            if kernel == "tets":
+                _lib.check(lib.ds_assemble_km_tets_tensor(_p(verts_f32), _p(tets_i32), T, order, pattern.n_nodes, *tp, _p(ctab),
+                                                          _p(mtab), _p(pattern.brow), _p(pattern.bcol), _p(pattern.contrib_ptr),
+                                                          _p(pattern.contrib), _p(pattern.slot), pattern.max_deg, pattern.nnzb,
+                                                          _p(geom), _p(Kval), _p(Mblk), _stream()), "ds_assemble_km_tets_tensor")
+            else:
+                _lib.check(lib.ds_assemble_km_tensor(_p(verts_f32), _p(tets_i32), T, order, pattern.n_nodes, *tp, _p(ctab),
+                                                     _p(mtab), _p(pattern.brow), _p(pattern.bcol), _p(pattern.contrib_ptr),
+                                                     _p(pattern.contrib), pattern.nnzb, _p(geom), _p(Kval), _p(Mblk),
+                                                     _stream()), "ds_assemble_km_tensor")
+        return Kval, Mblk
     if field is not None:
         assert mtab.dtype == torch.float32
         fp = _check_field(field, T, dev)
@@ -384,15 +409,15 @@ class CoarseLevel:
         self.use_coords = True
         self.fixed = None           # uint8 (n_nodes,) clamped corner nodes, applied after every assemble()
 
-    def assemble(self, verts_f32, mu, lam, ctab1, mtab1, field=None):
+    def assemble(self, verts_f32, mu, lam, ctab1, mtab1, field=None, tensor=None):
         """P1 stiffness (and mass) on the corner nodes at the current vertex positions, clamped at `fixed` when set.
-        field: the fine level's (mu_t, lam_t, rho_t) unchanged (coarse tet t is fine tet t; mtab1 then the fp32 unit
-        table), see assemble_km."""
+        field / tensor: the fine level's (mu_t, lam_t, rho_t) / (C21, rho_t) unchanged (coarse tet t is fine tet t; mtab1
+        then the fp32 unit table), see assemble_km."""
         self.verts = verts_f32[self.corner_nodes].contiguous()
         if self.geom is None:
             self.geom = torch.empty(self.tets.shape[0] * 14, dtype=torch.float64, device=self.tets.device)
         self.Kval, self.Mblk = assemble_km(self.verts, self.tets, 1, self.pattern, mu, lam, ctab1, mtab1,
-                                           Kval=self.Kval, Mblk=self.Mblk, geom=self.geom, field=field)
+                                           Kval=self.Kval, Mblk=self.Mblk, geom=self.geom, field=field, tensor=tensor)
         if self.fixed is not None:
             fix_nodes_km(self.pattern, self.fixed, self.Kval, self.Mblk)
 
@@ -614,6 +639,65 @@ def element_energies(verts_f32, tets_i32, order, m32, wsum, U, field):
     with torch.cuda.device(dev):
         _lib.check(lib.ds_element_energies(_p(verts_f32), _p(tets_i32), T, order, _p(m32), float(wsum), up, ldu, k, *fp,
                                            _p(strain), _p(kinetic), _stream()), "ds_element_energies")
+    return strain, kinetic
+
+
+def eigval_grad_shape_tensor(verts_f32, tets_i32, order, tensor, ctab, mtab1, U, lam, g, inc_ptr, inc, tet_grad=None):
+    """eigval_grad_shape with one elasticity tensor per tet (ds_eigval_grad_shape_tensor): tensor = (C21, rho_t) as in
+    assemble_km, mtab1 the unit-density table promoted to fp64.  -> (n_nodes, 3) fp32."""
+    lib = _lib.load()
+    dev = verts_f32.device
+    T = tets_i32.shape[0]
+    n_nodes = verts_f32.shape[0]
+    up, ldu = _pv(U)
+    k = U.shape[1]
+    assert lam.dtype == torch.float64 and g.dtype == torch.float64 and lam.numel() == k and g.numel() == k
+    tp = _check_tensor(tensor, T, dev)
+    if tet_grad is None:
+        tet_grad = torch.empty(T * 12, dtype=torch.float64, device=dev)
+    out = torch.empty(n_nodes, 3, dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.ds_eigval_grad_shape_tensor(_p(verts_f32), _p(tets_i32), T, order, n_nodes, *tp, _p(ctab), _p(mtab1),
+                                                   up, ldu, k, _p(lam.contiguous()), _p(g.contiguous()), _p(inc_ptr), _p(inc),
+                                                   _p(tet_grad), _p(out), _stream()), "ds_eigval_grad_shape_tensor")
+    return out
+
+
+def elasticity_field_grad(verts_f32, tets_i32, order, m32, wsum, U, lam, g):
+    """(gC (T, 21), grho (T,)) fp64 (ds_elasticity_field_grad): gC the packed upper triangle of sum_i g_i E_t,i, with
+    E_t,i = int_t eps_V(u_i) eps_V(u_i)^T dV the strain Gram of mode i on tet t (d lambda_i / dC_t for a symmetric C), and
+    grho = -sum_i g_i lam_i u_i^T Mhat_t u_i.  m32, U, lam, g as in material_field_grad."""
+    lib = _lib.load()
+    dev = verts_f32.device
+    T = tets_i32.shape[0]
+    up, ldu = _pv(U)
+    k = U.shape[1]
+    assert m32.dtype == torch.float32 and lam.dtype == torch.float64 and g.dtype == torch.float64
+    assert lam.numel() == k and g.numel() == k
+    gC = torch.empty(T, 21, dtype=torch.float64, device=dev)
+    grho = torch.empty(T, dtype=torch.float64, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.ds_elasticity_field_grad(_p(verts_f32), _p(tets_i32), T, order, _p(m32), float(wsum), up, ldu, k,
+                                                _p(lam.contiguous()), _p(g.contiguous()), _p(gC), _p(grho), _stream()),
+                   "ds_elasticity_field_grad")
+    return gC, grho
+
+
+def element_energies_tensor(verts_f32, tets_i32, order, m32, wsum, U, tensor):
+    """(strain, kinetic), each (T, k) fp64 (ds_element_energies_tensor): <C_t, E_t,i> and u_i^T M_t u_i; tensor = (C21,
+    rho_t) as in assemble_km."""
+    lib = _lib.load()
+    dev = verts_f32.device
+    T = tets_i32.shape[0]
+    up, ldu = _pv(U)
+    k = U.shape[1]
+    assert m32.dtype == torch.float32
+    tp = _check_tensor(tensor, T, dev)
+    strain = torch.empty(T, k, dtype=torch.float64, device=dev)
+    kinetic = torch.empty(T, k, dtype=torch.float64, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.ds_element_energies_tensor(_p(verts_f32), _p(tets_i32), T, order, _p(m32), float(wsum), up, ldu, k, *tp,
+                                                  _p(strain), _p(kinetic), _stream()), "ds_element_energies_tensor")
     return strain, kinetic
 
 

@@ -103,6 +103,21 @@ int ds_assemble_km_tets_field(const float* verts, const int32_t* tets, int64_t T
                               const float* m32, const int32_t* brow, const int32_t* bcol, const int32_t* contrib_ptr,
                               const int32_t* contrib, const int32_t* slot, int max_deg, int64_t nnzb, double* geom,
                               double* Kval, double* Mblk, void* stream);
+/* Elasticity-tensor fields: the same two assemblies with one anisotropic material per tet.  C21: fp64 [T*21], the 6x6
+ * elasticity matrix of tet t in Voigt order (11, 22, 33, 23, 13, 12) with engineering shear strains
+ * (eps_V = (e11, e22, e33, 2 e23, 2 e13, 2 e12), sigma_V = C eps_V), in the global (mesh) frame, packed as its upper triangle
+ * row by row; the strain energy of tet t is 1/2 int eps_V^T C_t eps_V dV, so K_ab[c][d] = |det A| sum_{k,l} C_{ckdl} S_ab[k][l].
+ * rho_t, m32 and the mass entries as ds_assemble_km_field.  An isotropic C reproduces the Lame assembly up to rounding (the
+ * summation order differs).  Same pattern, outputs and determinism. */
+int ds_assemble_km_tensor(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes,
+                          const double* C21, const float* rho_t, const double* ctab, const float* m32,
+                          const int32_t* brow, const int32_t* bcol, const int32_t* contrib_ptr, const int32_t* contrib,
+                          int64_t nnzb, double* geom, double* Kval, double* Mblk, void* stream);
+int ds_assemble_km_tets_tensor(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes,
+                               const double* C21, const float* rho_t, const double* ctab, const float* m32,
+                               const int32_t* brow, const int32_t* bcol, const int32_t* contrib_ptr, const int32_t* contrib,
+                               const int32_t* slot, int max_deg, int64_t nnzb, double* geom, double* Kval, double* Mblk,
+                               void* stream);
 /* Clamped nodes (csrc/fixed.cu): homogeneous Dirichlet conditions on whole nodes.  No reference interface: the reference
  * solves every object free-free.  In place on the block pattern of K (scalar-CSR order, as ds_assemble_km writes it) and M
  * (one scalar per block, may be NULL): every off-diagonal block (i, j) with fixed[i] || fixed[j] (device uint8 [n_nodes])
@@ -358,6 +373,25 @@ int ds_material_field_grad(const float* verts, const int32_t* tets, int64_t T, i
 int ds_element_energies(const float* verts, const int32_t* tets, int64_t T, int order, const float* m32, double wsum,
                         const double* U, int64_t ldu, int k, const double* mu_t, const double* lam_t, const float* rho_t,
                         double* strain, double* kinetic, void* stream);
+/* Shape gradient with an elasticity-tensor field: C21 fp64 [T*21], rho_t fp32 [T] as ds_assemble_km_tensor, mtab1 as
+ * ds_eigval_grad_shape_field.  C stays fixed in world axes when the vertices move. */
+int ds_eigval_grad_shape_tensor(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes,
+                                const double* C21, const float* rho_t, const double* ctab, const double* mtab1,
+                                const double* U, int64_t ldu, int k, const double* lam, const double* g,
+                                const int32_t* inc_ptr, const int32_t* inc, double* tet_grad, float* grad_verts,
+                                void* stream);
+/* Elasticity-tensor gradient: outC fp64 [T*21] = sum_i g_i E_t,i (packed upper triangle), E_t,i = int_t eps_V(u_i)
+ * eps_V(u_i)^T dV the strain Gram of mode i on tet t (exact quadrature, wsum as ds_eigval_quadforms_material), which is
+ * d lambda_i / dC_t for a symmetric C; out_rho fp64 [T] = -sum_i g_i lam_i u_i^T Mhat_t u_i.  One warp per tet, lanes
+ * across modes, a fixed shuffle tree: no atomics, bitwise reproducible. */
+int ds_elasticity_field_grad(const float* verts, const int32_t* tets, int64_t T, int order, const float* m32,
+                             double wsum, const double* U, int64_t ldu, int k, const double* lam, const double* g,
+                             double* outC, double* out_rho, void* stream);
+/* Element energies with an elasticity-tensor field: strain fp64 [T*k] = <C_t, E_t,i>, kinetic fp64 [T*k] as
+ * ds_element_energies. */
+int ds_element_energies_tensor(const float* verts, const int32_t* tets, int64_t T, int order, const float* m32,
+                               double wsum, const double* U, int64_t ldu, int k, const double* C21, const float* rho_t,
+                               double* strain, double* kinetic, void* stream);
 /* Material: q_mu[i] = u_i^T K(mu=1,lam=0) u_i, q_lam[i] = u_i^T K(0,1) u_i,
  * q_m[i] = u_i^T M u_i; replaces the matrix-free stiff_func path
  * (diff_model.py:314-328, 371-388; deform.py:70-87, 149-165).  wsum = sum of the

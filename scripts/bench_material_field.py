@@ -92,7 +92,7 @@ def ptxas_records():
         text = open(path).read()
         for m in re.finditer(r"Function properties for (\S+)\n(.*?)ptxas info\s+: Used (\d+) registers", text, re.S):
             name, body, regs = m.group(1), m.group(2), int(m.group(3))
-            if "k_material_field" in name or re.search(r"k_(assemble_rows|assemble_rows_tets2|eigval_grad_shape)I.*Lb1E", name):
+            if "k_material_field" in name or re.search(r"k_(assemble_rows|assemble_rows_tets2|eigval_grad_shape)I(Li\dE)?Li1EE", name):
                 spill = re.search(r"(\d+) bytes spill stores, (\d+) bytes spill loads", body)
                 out.append(dict(case="ptxas", kernel=name, registers=regs,
                                 spill_stores=int(spill.group(1)) if spill else None,
