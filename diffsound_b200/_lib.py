@@ -60,6 +60,11 @@ SIGNATURES = {
                                           cint, i64, f64p, f64p, f64p, ptr]),
     "ds_mass_expand": (cint, [i32p, i64, i64, f64p, f64p, ptr]),
     "ds_fix_nodes_km": (cint, [i32p, i32p, i64, i64, ptr, f64p, f64p, ptr]),
+    "ds_support_km": (cint, [f32p, i32p, i64, cint, i64, i32p, i32p, i64, f64p, f64p, i32p, i32p, i32p, i64, i32p, i32p,
+                             i32p, i64, f64p, ptr]),
+    "ds_support_grad": (cint, [f32p, i32p, i64, cint, i64, i32p, i32p, i64, f64p, f64p, f64p, i64, cint, f64p, i32p, i32p,
+                               i32p, i64, f64p, f64p, f64p, ptr]),
+    "ds_support_energies": (cint, [f32p, i32p, i64, cint, i64, i32p, i32p, i64, f64p, f64p, f64p, i64, cint, f64p, ptr]),
     "ds_assemble_mass_coo": (cint, [f64p, i32p, i64, cint, f64p, dbl, f64p, i32p, i32p, ptr]),
     "ds_spmm_km": (cint, [i32p, i32p, i64, f64p, f64p, dbl, f64p, i64, cint, dbl, dbl, f64p, i64, f64p, i64, ptr]),
     "ds_spmm_k_and_m": (cint, [i32p, i32p, i64, f64p, f64p, f64p, i64, cint, f64p, i64, f64p, i64, ptr]),

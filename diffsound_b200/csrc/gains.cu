@@ -19,6 +19,7 @@
 #include "common.cuh"
 #include "../../include/diffsound_sm100.h"
 #include "closest.cuh"
+#include "tet_faces.cuh"
 #include <cub/cub.cuh>
 #include <climits>
 
@@ -27,13 +28,6 @@ namespace ds {
 namespace {
 
 constexpr int GAINS_WARPS = 8;     // points per CTA (one warp each)
-
-// local node of tet corner j (shape_func.CORNER_LOCAL)
-__device__ __forceinline__ int corner_local(int order, int j) { return order == 1 ? j : (j == 3 ? 9 : 2 * j); }
-
-// the (l, m) barycentric pair of P2 node a (shape_func.P2_NODES): l == m a corner, else the mid-edge node of (l, m)
-__constant__ signed char c_p2_l[10] = {0, 0, 1, 1, 2, 2, 0, 1, 2, 3};
-__constant__ signed char c_p2_m[10] = {0, 1, 1, 2, 2, 0, 3, 3, 3, 3};
 
 // corner ids of face f (opposite corner f) of tet t, sorted ascending
 __device__ __forceinline__ void face_triple(const int32_t* __restrict__ tets, int npe, int order, int64_t i, uint32_t (&v)[3]) {

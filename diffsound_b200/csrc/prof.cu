@@ -78,7 +78,8 @@ static void drain() {
 static const char* kNames[PROF_NCLASS] = {"pattern", "geometry", "assemble", "spmm", "cheb_step", "gram", "block_gemm",
                                           "eigh", "residual", "copy", "grad_shape", "quadforms", "synth", "other",
                                           "coarse_step", "transfer", "jacobi_scale", "sdf_build", "sdf_query",
-                                          "sdf_winding", "tet_stuff", "gains", "fix_nodes", "material_field"};
+                                          "sdf_winding", "tet_stuff", "gains", "fix_nodes", "material_field",
+                                          "support"};
 
 }  // namespace ds
 

@@ -191,6 +191,61 @@ def check_elasticity_field(num_tets, device, C, density=None):
         check_material_field(num_tets, device, density=density)
 
 
+#: supports must hold every rigid motion: the smallest eigenvalue of the 6 x 6 R^T K_s R over the rigid fields (unit
+#: translations, rotations scaled by the object's extent) must exceed this fraction of the largest.  Roundoff leaves an
+#: unsupported direction near 1e-16; a genuinely soft direction (k_t = 1e-6 k_n) is far above the margin.
+SUPPORT_RIGID_MARGIN = 1e-10
+
+
+def check_support_stiffness(S, device, normal, tangential):
+    """Host validation of support stiffnesses (DiffSoundObj.set_supports): each a Python float or a finite fp32 / fp64 (S,)
+    tensor on `device`, all >= 0.  Returns (k_n, k_t) as contiguous fp64 (S,) tensors (copies).  Raises ValueError."""
+    out = []
+    for name, k in (("normal", normal), ("tangential", tangential)):
+        if torch.is_tensor(k):
+            if k.dtype not in (torch.float32, torch.float64):
+                raise ValueError(f"set_supports: {name} must be a float or a float32 / float64 tensor")
+            if k.shape != (S,):
+                raise ValueError(f"set_supports: {name} has shape {tuple(k.shape)}, expected ({S},): one value per support "
+                                 "face in ascending face order")
+            if k.device != torch.device(device):
+                raise ValueError(f"set_supports: {name} is on {k.device}, the mesh on {device}")
+            x = k.detach().to(torch.float64).clone().contiguous()
+        elif isinstance(k, (int, float)) and not isinstance(k, bool):
+            x = torch.full((S,), float(k), dtype=torch.float64, device=device)
+        else:
+            raise ValueError(f"set_supports: {name} must be a float or a (S,) tensor")
+        if not bool(torch.isfinite(x).all()):
+            raise ValueError(f"set_supports: {name} has non-finite values")
+        if not bool((x >= 0).all()):
+            raise ValueError(f"set_supports: {name} must be >= 0")
+        out.append(x)
+    return out[0], out[1]
+
+
+def support_rigid_matrix(p0, p1, p2, kn, kt):
+    """The 6 x 6 R^T K_s R of a spring bed over the rigid fields R = [translations, rotations / L] about the centroid of
+    the support corners (L their extent), from the exact edge-midpoint rule (rigid fields are linear, the integrand
+    quadratic).  p0, p1, p2 (S, 3) fp64 face corners; kn, kt (S,) fp64."""
+    c = torch.cat([p0, p1, p2]).mean(0)
+    L = float(torch.cat([p0, p1, p2]).sub(c).norm(dim=1).max().clamp_min(1e-30))
+    a = 0.5 * torch.cross(p1 - p0, p2 - p0, dim=1)
+    A = a.norm(dim=1)
+    n = a / A.clamp_min(1e-300)[:, None]
+    Sm = (kn - kt)[:, None, None] * n[:, :, None] * n[:, None, :] + kt[:, None, None] * torch.eye(3, dtype=a.dtype,
+                                                                                                    device=a.device)
+    G = torch.zeros(6, 6, dtype=a.dtype, device=a.device)
+    eye = torch.eye(3, dtype=a.dtype, device=a.device).expand(p0.shape[0], 3, 3)
+    for x in (0.5 * (p0 + p1), 0.5 * (p1 + p2), 0.5 * (p2 + p0)):
+        y = (x - c) / L
+        z = torch.zeros_like(y[:, 0])
+        rot = torch.stack([torch.stack([-y[:, 1], y[:, 0], z], 1), torch.stack([z, -y[:, 2], y[:, 1]], 1),
+                           torch.stack([y[:, 2], z, -y[:, 0]], 1)], dim=2)          # (S, 3, 3): columns are the fields
+        R = torch.cat([eye, rot], dim=2)                                             # (S, 3, 6)
+        G += torch.einsum("s,sci,scd,sdj->ij", A / 3, R, Sm, R)
+    return G
+
+
 def material_field_from_regions(labels, materials):
     """(youngs, poisson, density), each (T,) fp64 on the device of `labels`: the material `materials[labels[t]]` (MatSet
     tuples) of every tet, for DiffSoundObj.set_material_field."""
@@ -339,6 +394,31 @@ class _EigvalTensor(torch.autograd.Function):
         return gverts, gC, grho, None
 
 
+class _SupportTerm(torch.autograd.Function):
+    """Zero-valued term of get_vals() for an object on elastic supports: the eigenvalues already include K_s (the value is
+    read from Kval), and the backward adds the support part sum_i g_i u_i^T dK_s u_i of the gradient, to the vertices
+    (through the area vectors of the support faces) and to the per-face normal / tangential stiffnesses
+    (native.support_grad).  The stiffnesses, eigenvectors and geometry the assembly used are pinned at forward time."""
+
+    @staticmethod
+    def forward(ctx, vertices, normal, tangential, obj):
+        sup = obj._sup_used
+        ctx.vdtype = obj.tetmesh.vertices.dtype
+        ctx.dtypes = tuple(k.dtype if torch.is_tensor(k) else None for k in (normal, tangential))
+        ctx.faces, ctx.U = obj._sup["fine"], obj.U_hat
+        ctx.save_for_backward(obj._verts32, obj.deform.tets_i32, sup["kn"], sup["kt"])
+        return torch.zeros(obj.mode_num, 1, dtype=torch.float32, device=obj.deform.device)
+
+    @staticmethod
+    def backward(ctx, g):
+        verts32, tets, kn, kt = ctx.saved_tensors
+        gv = g.reshape(-1).to(torch.float64).contiguous()
+        gk, gverts = native.support_grad(verts32, tets, ctx.faces, kn, kt, ctx.U, gv, want_verts=ctx.needs_input_grad[0])
+        gn = gk[:, 0].to(ctx.dtypes[0]) if ctx.needs_input_grad[1] else None
+        gt = gk[:, 1].to(ctx.dtypes[1]) if ctx.needs_input_grad[2] else None
+        return (None if gverts is None else gverts.to(ctx.vdtype)), gn, gt, None
+
+
 class _StiffFunc(torch.autograd.Function):
     """y = (mu K_mu + lam K_lam) x with gradients to x (K is symmetric: K^T g) and to the two Lame
     scalars (<g, K_mu x>, <g, K_lam x>) -- stiff_func of the reference is differentiable in both
@@ -460,6 +540,9 @@ class DiffSoundObj:
         self._field_used = None
         self.elasticity_field = None    # (C, density) of set_elasticity_field, None: isotropic
         self._tensor_used = None
+        self.supports = None            # (faces mask, normal, tangential) of set_supports, None: no supports
+        self._sup = None                # native.SupportFaces of the fine (and coarse) level
+        self._sup_used = None           # the (k_n, k_t) fp64 (S,) the last assembly used
 
     # ------------------------------------------------------------------ parameters
     def parameters(self):
@@ -541,6 +624,11 @@ class DiffSoundObj:
             self._Kval, self._Mblk = native.assemble_km(self._verts32, d.tets_i32, self.tetmesh.order, pat, 0.0, 0.0, d.ctab,
                                                         d.m32(), Kval=self._Kval, Mblk=self._Mblk, geom=self._geom,
                                                         field=(f["mu"], f["lam"], f["rho"]))
+        self._sup_used = None
+        if self.supports is not None:
+            kn, kt = self._support_snapshot()
+            self._sup_used = dict(kn=kn, kt=kt)
+            native.support_km(self._verts32, d.tets_i32, pat, self._sup["fine"], kn, kt, self._Kval)
         if self._fixed_u8 is not None:
             native.fix_nodes_km(pat, self._fixed_u8, self._Kval, self._Mblk)
         self._density_used = float(density)
@@ -586,6 +674,9 @@ class DiffSoundObj:
         if self.elasticity_field is not None:
             raise NotImplementedError("stiff_func: K = mu K_mu + lam K_lam with one (mu, lam) for the whole object; it is not "
                                       "defined for an elasticity-tensor field (set_elasticity_field(None) first)")
+        if self.supports is not None:
+            raise NotImplementedError("stiff_func: K = mu K_mu + lam K_lam has no support term; it is not defined for an "
+                                      "object on elastic supports (set_supports(None) first)")
         x = x_in.unsqueeze(1) if x_in.dim() == 1 else x_in
         mu, lam = self.material_model.lame()
         mu = torch.as_tensor(mu, dtype=torch.float32).to(x.device)
@@ -690,6 +781,79 @@ class DiffSoundObj:
         if self._Kval is not None:
             self._assemble(self._density_used)
 
+    # ------------------------------------------------------------------ elastic supports
+    def set_supports(self, faces, normal=None, tangential=None):
+        """Rest the object on elastic supports: a Winkler spring bed on the boundary faces of the boolean mask `faces` over
+        the rows of surface(), with normal and tangential stiffness per unit area (N/m^3; see supports.pad_stiffness for a
+        pad of given material and thickness).  normal / tangential are floats or (S,) fp32 / fp64 CUDA tensors, one value
+        per support face in ascending face order; tensors are kept by reference and validated again at every assembly
+        (shape, device, finite, >= 0), so an optimiser may update them in place.  Face f adds int_f N_a N_b dA ((k_n - k_t)
+        n n^T + k_t I) to K (native.support_km, fine and coarse level); M is unchanged.
+
+        The object then has no rigid modes: `eigenvalues` / `U_hat` are the lowest mode_num pairs, the support's bounce and
+        rock modes included, and get_vals() is differentiable in the two stiffness tensors as well.  Unless nodes are also
+        clamped, the supports must hold every rigid motion (R^T K_s R positive definite, SUPPORT_RIGID_MARGIN); a flat face
+        with k_t = 0, for instance, leaves the object free to slide and raises ValueError.  `set_supports(None)` removes
+        them.  Either way the warm start and the cached operators are dropped."""
+        if faces is None:
+            self.supports = None
+            self._sup = None
+        else:
+            srf, owner, local = self.surface()
+            if not torch.is_tensor(faces) or faces.dtype != torch.bool or faces.shape != (srf.shape[0],):
+                raise ValueError(f"set_supports: faces must be a boolean ({srf.shape[0]},) mask over the rows of surface()")
+            if faces.device != srf.device:
+                raise ValueError(f"set_supports: faces is on {faces.device}, the mesh on {srf.device}")
+            sel = torch.nonzero(faces).squeeze(1)
+            if sel.numel() == 0:
+                raise ValueError("set_supports: no face selected; pass None to remove the supports")
+            if normal is None or tangential is None:
+                raise ValueError("set_supports: normal and tangential stiffnesses are required")
+            prev = (self.supports, self._sup)
+            self.supports = (faces, normal, tangential)
+            self._sup = dict(fine=native.SupportFaces(self.deform.tets_i32, self.tetmesh.order, owner[sel], local[sel]),
+                             corners=srf[sel])
+            try:
+                self._support_snapshot()
+            except ValueError:
+                self.supports, self._sup = prev
+                raise
+        self._warm = []
+        self._q = None
+        for key in ("_Kunit", "_stiff_coo", "_mass_coo"):
+            self.__dict__.pop(key, None)
+        if self._Kval is not None:
+            self._assemble(self._density_used)
+
+    def _support_faces_coarse(self):
+        if "coarse" not in self._sup:
+            fine = self._sup["fine"]
+            self._sup["coarse"] = native.SupportFaces(self.deform.coarse.tets, 1, fine.owner, fine.local)
+        return self._sup["coarse"]
+
+    def _support_snapshot(self):
+        """(k_n, k_t) fp64 (S,) of the supports, validated again; unless clamps are set, the rigid-motion check too."""
+        _, normal, tangential = self.supports
+        kn, kt = check_support_stiffness(self._sup["fine"].S, self.deform.device, normal, tangential)
+        if self._fixed_u8 is None:
+            p = self.tetmesh.vertices.detach().to(torch.float64)[self._sup["corners"]]
+            ev = torch.linalg.eigvalsh(support_rigid_matrix(p[:, 0], p[:, 1], p[:, 2], kn, kt))
+            if not bool(ev[0] > SUPPORT_RIGID_MARGIN * ev[-1]):
+                raise ValueError("set_supports: the supports do not hold every rigid motion (the smallest eigenvalue of "
+                                 f"R^T K_s R is {float(ev[0]):.3e}, the largest {float(ev[-1]):.3e}); support more faces, "
+                                 "give them tangential stiffness, or clamp nodes")
+        return kn, kt
+
+    def support_energies(self):
+        """(S, mode_num) fp64, no gradient: u_i^T K_s,f u_i of every support face f (ascending) and solved mode i for the
+        stiffnesses of the last assembly; with element_energies()'s strain they sum to lambda_i."""
+        if getattr(self, "U_hat", None) is None:
+            raise RuntimeError("support_energies: run eigen_decomposition() first")
+        if self._sup_used is None:
+            raise RuntimeError("support_energies: the object has no supports (set_supports)")
+        return native.support_energies(self._verts32, self.deform.tets_i32, self._sup["fine"], self._sup_used["kn"],
+                                       self._sup_used["kt"], self.U_hat)
+
     def element_energies(self):
         """(strain, kinetic), each (T, mode_num) fp64, no gradient: u_i^T K_t u_i and u_i^T M_t u_i of every tet t and
         solved mode i (U_hat, M-normalised), for the material of the last assembly (field or not).  Summed over the tets
@@ -713,8 +877,8 @@ class DiffSoundObj:
 
     @property
     def _n_rigid(self):
-        """Rigid-body modes at the bottom of the spectrum: six free-free, none when clamped."""
-        return 6 if self._fixed_u8 is None else 0
+        """Rigid-body modes at the bottom of the spectrum: six free-free, none when clamped or on supports."""
+        return 6 if self._fixed_u8 is None and self.supports is None else 0
 
     # ------------------------------------------------------------------ eigen-solve
     def eigen_decomposition(self):
@@ -724,7 +888,7 @@ class DiffSoundObj:
     def _start_block(self, m, batch=0):
         """Start block of batch `batch` (n, m): the previous decomposition's Ritz block of this mesh when there is
         one (warm start; COPIED -- ds_lobpcg overwrites its block in place and earlier U_hat views / pending
-        backward passes keep the old storage), else the six analytic rigid-body modes (free objects only) + seeded random
+        backward passes keep the old storage), else the six analytic rigid-body fields (unclamped objects) + seeded random
         columns."""
         n = self.deform.pattern.n
         dev = self.deform.device
@@ -733,7 +897,7 @@ class DiffSoundObj:
             return prev.clone(), True
         g = torch.Generator(device=dev).manual_seed(batch)
         X = torch.randn(n, m, dtype=torch.float64, device=dev, generator=g)
-        if batch == 0 and self._n_rigid:
+        if batch == 0 and self._fixed_u8 is None:      # free or on supports: the rigid fields start the lowest modes
             p = self._verts32.double()
             p = p - p.mean(0, keepdim=True)
             X[:, :6] = 0
@@ -768,8 +932,8 @@ class DiffSoundObj:
         return next((c for c in (16, 32, 48) if c >= need + min(4, c // 8)), None)
 
     def eigen_decomposition_arpack(self):
-        """Lowest mode_num + 6 eigenpairs of K u = lambda M u, rigid six dropped (a clamped object: the lowest mode_num
-        pairs, see fix_nodes).  The name is the
+        """Lowest mode_num + 6 eigenpairs of K u = lambda M u, rigid six dropped (a clamped object or one on supports: the
+        lowest mode_num pairs, see fix_nodes and set_supports).  The name is the
         reference's (diff_model.py:335-369: SciPy ARPACK shift-invert on the CPU); the solver is the
         device-resident LOBPCG of csrc/lobpcg.cu.  More pairs than one 48-column block holds are found in
         batches: every batch runs M-orthogonal to the pairs already converged (ds_lobpcg_opts.locked) and
@@ -788,14 +952,18 @@ class DiffSoundObj:
             # two-level p-multigrid preconditioner: P1 operator of the same mesh, same material
             mu, la = self._lame_used
             coarse.fixed = None if self._fixed_u8 is None else self._fixed_u8[coarse.corner_nodes].contiguous()
+            sup = None if self._sup_used is None else (self._support_faces_coarse(), self._sup_used["kn"],
+                                                       self._sup_used["kt"])
             if self._tensor_used is not None:       # coarse tet t is fine tet t: the same per-tet arrays
                 t = self._tensor_used
-                coarse.assemble(self._verts32, 0.0, 0.0, coarse.ctab, self.deform.m32(1), tensor=(t["C21"], t["rho"]))
+                coarse.assemble(self._verts32, 0.0, 0.0, coarse.ctab, self.deform.m32(1), tensor=(t["C21"], t["rho"]),
+                                supports=sup)
             elif self._field_used is None:
-                coarse.assemble(self._verts32, mu, la, coarse.ctab, self.deform.coarse_mtab(self._density_used))
+                coarse.assemble(self._verts32, mu, la, coarse.ctab, self.deform.coarse_mtab(self._density_used), supports=sup)
             else:       # coarse tet t is fine tet t: the same per-tet arrays
                 f = self._field_used
-                coarse.assemble(self._verts32, 0.0, 0.0, coarse.ctab, self.deform.m32(1), field=(f["mu"], f["lam"], f["rho"]))
+                coarse.assemble(self._verts32, 0.0, 0.0, coarse.ctab, self.deform.m32(1), field=(f["mu"], f["lam"], f["rho"]),
+                                supports=sup)
             # n_c^(1/3) scaling fits compact bodies; thin shells (the bowl fixture) need the floor: 37 -> 28 outer iterations
             cdeg = int(self.coarse_degree) or int(min(64, max(32, round((3 * coarse.n_nodes) ** (1.0 / 3.0) / 1.2))))
             cratio = float(self.coarse_ratio) or 0.4 * cdeg * cdeg
@@ -898,12 +1066,24 @@ class DiffSoundObj:
             mu, lam = torch.as_tensor(mu).to(dev), torch.as_tensor(lam).to(dev)
             # fp64 until the final cast (the reference does this sum in fp32, diff_model.py:382-386)
             add_term = (mu.double() * q_mu + lam.double() * q_la) - self.eigenvalues * q_m
+            if self._sup_used is not None:      # lambda = u^T K u includes the spring bed
+                add_term = add_term + self.support_energies().sum(0)
             predict = predict + add_term.float()
         return (torch.sqrt(predict) / 2 / np.pi).unsqueeze(1)
 
     def get_vals(self):
         """(mode_num, 1) fp32 eigenvalues, differentiable w.r.t. the vertex positions
-        (diff_model.py:390-399) and, with a material or elasticity-tensor field, w.r.t. its tensors."""
+        (diff_model.py:390-399), with a material or elasticity-tensor field w.r.t. its tensors, and on supports w.r.t. the
+        normal and tangential stiffness tensors of set_supports."""
+        vals = self._get_vals_volume()
+        if self._sup_used is None:
+            return vals
+        _, normal, tangential = self.supports if self.supports is not None else (None, None, None)
+        normal = normal if torch.is_tensor(normal) else None
+        tangential = tangential if torch.is_tensor(tangential) else None
+        return vals + _SupportTerm.apply(self.tetmesh.vertices, normal, tangential, self)
+
+    def _get_vals_volume(self):
         if self._tensor_used is not None:
             C, density = self.elasticity_field if self.elasticity_field is not None else (self._tensor_used["C"], None)
             return _EigvalTensor.apply(self.tetmesh.vertices, C, density, self)

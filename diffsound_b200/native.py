@@ -247,6 +247,97 @@ def fix_nodes_km(pattern, fixed, Kval, Mblk=None):
     return Kval, Mblk
 
 
+class SupportFaces:
+    """Support faces of one mesh level for the ds_support_* kernels: owner / local int32 (S,) (the face opposite corner
+    local[s] of tet owner[s]) and the node -> (face, face-local node) incidence of ds_support_km, built from `tets_i32`."""
+
+    def __init__(self, tets_i32, order, owner, local):
+        from .diffelastic.shape_func import CORNER_LOCAL, P2_NODES
+        dev = tets_i32.device
+        self.order = int(order)
+        self.owner = owner.to(device=dev, dtype=torch.int32).contiguous()
+        self.local = local.to(device=dev, dtype=torch.int32).contiguous()
+        self.S = int(self.owner.numel())
+        # face-local nodes of the face opposite corner f: corners j != f, then (P2) the mid-edge nodes off corner f
+        rows = []
+        for f in range(4):
+            r = [CORNER_LOCAL[self.order][j] for j in range(4) if j != f]
+            if self.order == 2:
+                r += [a for a, (l, m) in enumerate(P2_NODES) if l != m and f not in (l, m)]
+            rows.append(r)
+        tab = torch.tensor(rows, dtype=torch.int64, device=dev)
+        nodes = tets_i32.long()[self.owner.long()[:, None], tab[self.local.long()]]          # (S, nf)
+        nf = nodes.shape[1]
+        ent = torch.arange(self.S * nf, device=dev)
+        code = (ent // nf) * 8 + ent % nf
+        order_ = torch.argsort(nodes.reshape(-1) * (8 * self.S) + code)
+        flat = nodes.reshape(-1)[order_]
+        self.inc_node, counts = torch.unique_consecutive(flat, return_counts=True)
+        self.inc_node = self.inc_node.to(torch.int32).contiguous()
+        self.inc_ptr = torch.zeros(counts.numel() + 1, dtype=torch.int32, device=dev)
+        self.inc_ptr[1:] = torch.cumsum(counts, 0).to(torch.int32)
+        self.inc = code[order_].to(torch.int32).contiguous()
+        self.R = int(self.inc_node.numel())
+        self.nodes = nodes
+
+
+def _check_stiffness(k, S, dev):
+    if k.dtype != torch.float64 or k.shape != (S,) or k.device != dev or not k.is_contiguous():
+        raise ValueError(f"supports: stiffness must be a contiguous ({S},) float64 tensor on {dev}")
+    return _p(k)
+
+
+def support_km(verts_f32, tets_i32, pattern, faces, kn, kt, Kval):
+    """Add the spring bed of SupportFaces `faces` with per-face stiffnesses kn, kt (S,) fp64 to Kval in place
+    (ds_support_km)."""
+    lib = _lib.load()
+    dev = Kval.device
+    assert Kval.numel() == pattern.nnz and faces.order in (1, 2)
+    with torch.cuda.device(dev):
+        _lib.check(lib.ds_support_km(_p(verts_f32), _p(tets_i32), tets_i32.shape[0], faces.order, pattern.n_nodes,
+                                     _p(faces.owner), _p(faces.local), faces.S, _check_stiffness(kn, faces.S, dev),
+                                     _check_stiffness(kt, faces.S, dev), _p(faces.inc_node), _p(faces.inc_ptr),
+                                     _p(faces.inc), faces.R, _p(pattern.brow), _p(pattern.bcol),
+                                     _p(getattr(pattern, "slot", None)), pattern.nnzb, _p(Kval), _stream()), "ds_support_km")
+    return Kval
+
+
+def support_grad(verts_f32, tets_i32, faces, kn, kt, U, g, want_verts=True):
+    """Gradient of sum_i g_i u_i^T K_s u_i (ds_support_grad): ((S, 2) fp64 to (kn, kt), (n_nodes, 3) fp64 to the node
+    positions or None).  U (n, k) fp64 row-major view; g (k,) fp64."""
+    lib = _lib.load()
+    dev = verts_f32.device
+    up, ldu = _pv(U)
+    k = U.shape[1]
+    assert g.dtype == torch.float64 and g.numel() == k
+    n_nodes = verts_f32.shape[0]
+    scratch = torch.empty(faces.S * 9, dtype=torch.float64, device=dev)
+    gk = torch.empty(faces.S, 2, dtype=torch.float64, device=dev)
+    gv = torch.empty(n_nodes, 3, dtype=torch.float64, device=dev) if want_verts else None
+    with torch.cuda.device(dev):
+        _lib.check(lib.ds_support_grad(_p(verts_f32), _p(tets_i32), tets_i32.shape[0], faces.order, n_nodes, _p(faces.owner),
+                                       _p(faces.local), faces.S, _check_stiffness(kn, faces.S, dev),
+                                       _check_stiffness(kt, faces.S, dev), up, ldu, k, _p(g.contiguous()),
+                                       _p(faces.inc_node), _p(faces.inc_ptr), _p(faces.inc), faces.R, _p(scratch), _p(gk),
+                                       _p(gv), _stream()), "ds_support_grad")
+    return gk, gv
+
+
+def support_energies(verts_f32, tets_i32, faces, kn, kt, U):
+    """(S, k) fp64 u_i^T K_s,f u_i of every support face and mode (ds_support_energies)."""
+    lib = _lib.load()
+    dev = verts_f32.device
+    up, ldu = _pv(U)
+    k = U.shape[1]
+    out = torch.empty(faces.S, k, dtype=torch.float64, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(lib.ds_support_energies(_p(verts_f32), _p(tets_i32), tets_i32.shape[0], faces.order, verts_f32.shape[0],
+                                           _p(faces.owner), _p(faces.local), faces.S, _check_stiffness(kn, faces.S, dev),
+                                           _check_stiffness(kt, faces.S, dev), up, ldu, k, _p(out), _stream()),
+                   "ds_support_energies")
+    return out
+
+
 def mass_expand(pattern, Mblk):
     lib = _lib.load()
     Mval = torch.empty(pattern.nnz, dtype=torch.float64, device=Mblk.device)
@@ -409,15 +500,19 @@ class CoarseLevel:
         self.use_coords = True
         self.fixed = None           # uint8 (n_nodes,) clamped corner nodes, applied after every assemble()
 
-    def assemble(self, verts_f32, mu, lam, ctab1, mtab1, field=None, tensor=None):
+    def assemble(self, verts_f32, mu, lam, ctab1, mtab1, field=None, tensor=None, supports=None):
         """P1 stiffness (and mass) on the corner nodes at the current vertex positions, clamped at `fixed` when set.
         field / tensor: the fine level's (mu_t, lam_t, rho_t) / (C21, rho_t) unchanged (coarse tet t is fine tet t; mtab1
-        then the fp32 unit table), see assemble_km."""
+        then the fp32 unit table), see assemble_km.  supports: (SupportFaces over self.tets, kn, kt), the spring bed added
+        before the clamps (coarse tet t is fine tet t, so the fine level's owner / local name the same faces)."""
         self.verts = verts_f32[self.corner_nodes].contiguous()
         if self.geom is None:
             self.geom = torch.empty(self.tets.shape[0] * 14, dtype=torch.float64, device=self.tets.device)
         self.Kval, self.Mblk = assemble_km(self.verts, self.tets, 1, self.pattern, mu, lam, ctab1, mtab1,
                                            Kval=self.Kval, Mblk=self.Mblk, geom=self.geom, field=field, tensor=tensor)
+        if supports is not None:
+            faces, kn, kt = supports
+            support_km(self.verts, self.tets, self.pattern, faces, kn, kt, self.Kval)
         if self.fixed is not None:
             fix_nodes_km(self.pattern, self.fixed, self.Kval, self.Mblk)
 

@@ -603,6 +603,9 @@ def eigen_decomposition_rowpart(obj, group=None, verbose=False, solver=None, kee
     if obj.elasticity_field is not None:
         raise NotImplementedError("row-partitioned eigen-solve: elasticity-tensor fields (DiffSoundObj.set_elasticity_field) "
                                   "are not supported; use eigen_decomposition() on one GPU")
+    if obj.supports is not None:
+        raise NotImplementedError("row-partitioned eigen-solve: elastic supports (DiffSoundObj.set_supports) are not "
+                                  "supported; use eigen_decomposition() on one GPU")
     obj._assemble(obj.material_model.mat.density)
     if obj.tetmesh.order != 2 or obj.deform.coarse is None:
         raise NotImplementedError("row-partitioned eigen-solve: quadratic meshes only (two-level preconditioner)")

@@ -125,6 +125,32 @@ int ds_assemble_km_tets_tensor(const float* verts, const int32_t* tets, int64_t 
  * warp per node row, no atomics, deterministic. */
 int ds_fix_nodes_km(const int32_t* brow, const int32_t* bcol, int64_t n_nodes, int64_t nnzb, const uint8_t* fixed,
                     double* Kval, double* Mblk, void* stream);
+/* Elastic supports (csrc/support.cu): a Winkler spring bed on S boundary faces, each named by its owning tet owner[s] and
+ * the local index local[s] of the corner opposite it (ds_tet_boundary_fill's owner / local), with normal and tangential
+ * stiffness per unit area kn[s], kt[s] (fp64, N/m^3).  Face s adds K_s,f[a, b] = int_f N_a N_b dA ((kn - kt) n n^T +
+ * kt I) over its P1 (3) or P2 (6) nodes, the face affine from its corners; M is unchanged.
+ * The incidence lists every (face, face-local node) of a support node: rows r < R of node inc_node[r] (ascending, each node
+ * once), entries inc[inc_ptr[r] .. inc_ptr[r+1]) = 8 s + q in ascending s, with q < 3 the corners (ascending tet corner
+ * index, skipping local[s]) and 3 <= q < 6 the P2 mid-edge nodes (ascending tet-local index) of face s.
+ * ds_support_km adds K_s into Kval in place (scalar-CSR order of ds_assemble_km, any block pattern; slot: the element ->
+ * slot map of ds_pattern_fill or NULL for a binary search of bcol).  One thread per incidence row; each slot is summed in
+ * fp64 in ascending face order, no atomics, bitwise reproducible, and a bitwise symmetric Kval stays so. */
+int ds_support_km(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes, const int32_t* owner,
+                  const int32_t* local, int64_t S, const double* kn, const double* kt, const int32_t* inc_node,
+                  const int32_t* inc_ptr, const int32_t* inc, int64_t R, const int32_t* brow, const int32_t* bcol,
+                  const int32_t* slot, int64_t nnzb, double* Kval, void* stream);
+/* Gradient of sum_i g_i u_i^T K_s u_i (U fp64 row-major [n x ldu], k modes; g fp64 [k]): grad_k fp64 [S*2] to (kn[s],
+ * kt[s]) and, when grad_verts is not NULL, fp64 [n_nodes*3] to the node positions (zero off the support corners), reduced
+ * through the incidence of ds_support_km.  face_scratch fp64 [S*9].  One warp per face, lanes across modes, fixed
+ * shuffle tree: bitwise reproducible. */
+int ds_support_grad(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes, const int32_t* owner,
+                    const int32_t* local, int64_t S, const double* kn, const double* kt, const double* U, int64_t ldu, int k,
+                    const double* g, const int32_t* inc_node, const int32_t* inc_ptr, const int32_t* inc, int64_t R,
+                    double* face_scratch, double* grad_k, double* grad_verts, void* stream);
+/* out fp64 [S*k] = u_i^T K_s,f u_i per support face and mode: the kernel of ds_support_grad without the reduction. */
+int ds_support_energies(const float* verts, const int32_t* tets, int64_t T, int order, int64_t n_nodes,
+                        const int32_t* owner, const int32_t* local, int64_t S, const double* kn, const double* kt,
+                        const double* U, int64_t ldu, int k, double* out, void* stream);
 int ds_mass_expand(const int32_t* brow, int64_t n_nodes, int64_t nnzb, const double* Mblk,
                    double* Mval, void* stream);
 /* Legacy twin of the reference export `assemble_mass_matrix` (massMatrixDouble.cu:138-158):
