@@ -63,17 +63,21 @@ __device__ void load_twiddles(Cplx* tw, int n) {
     }
 }
 
-// s[bitrev(i)] = hann[i] * (a[i] + i b[i]) for the frame starting at padded position fr * hop
-__device__ void load_frame(Cplx* s, const float* __restrict__ a, const float* __restrict__ b, int64_t T, int n, int logn,
+// s[bitrev(i)] = hann[i] * (a[i] + i b[i]) for the frame starting at padded position fr * hop.  Returns whether every
+// sample this thread loaded has a[i] == b[i] (false without b).
+__device__ bool load_frame(Cplx* s, const float* __restrict__ a, const float* __restrict__ b, int64_t T, int n, int logn,
                            int fr, int hop) {
+    bool same = b != nullptr;
     for (int i = threadIdx.x; i < n; i += blockDim.x) {
         const int64_t src = reflect_idx((int64_t)fr * hop + i - n / 2, T);
         const float w = 0.5f - 0.5f * cospif(2.f * (float)i / (float)n);
         Cplx v;
         v.re = w * a[src];
         v.im = b ? w * b[src] : 0.f;
+        same = same && a[src] == b[src];
         s[bitrev(i, logn)] = v;
     }
+    return same;
 }
 
 // spectra of the two real signals packed as re/im: A_f = (Z_f + conj(Z_{n-f})) / 2,  B_f = (Z_f - conj(Z_{n-f})) / (2i)
@@ -115,17 +119,20 @@ k_mss_fwd(const float* __restrict__ xp, const float* __restrict__ xt, int64_t T,
     __shared__ double red[MSS_THREADS / 32];
     const int fr = blockIdx.x, b = blockIdx.y, bins = n / 2 + 1;
     load_twiddles(tw, n);
-    load_frame(s, xp + (size_t)b * T, xt + (size_t)b * T, T, n, logn, fr, hop);
-    __syncthreads();
+    // equal frames have equal spectra, but the packed FFT rounds A and B apart: take B = A, so that pred == true
+    // gives a loss of exactly 0 (and rmse its zero gradient) instead of rounding noise
+    const bool same = __syncthreads_and(load_frame(s, xp + (size_t)b * T, xt + (size_t)b * T, T, n, logn, fr, hop));
     fft_smem(s, tw, n, logn, false);
     const float wt = time_weight(fr, frames);
     double acc = 0.0;
     for (int f = threadIdx.x + (mode == 0 ? 1 : 0); f < bins; f += blockDim.x) {     // l1: the DC bin is dropped
         Cplx A, B;
         unpack2(s, n, f, A, B);
+        if (same) B = A;
         const float Sp = A.re * A.re + A.im * A.im, St = B.re * B.re + B.im * B.im;
         const float lp = log2f(Sp + eps), lt = log2f(St + eps);
-        if (mode == 0) acc += (double)(alpha * fabsf(wt * lp - wt * lt) + fabsf(wt * Sp - wt * St));
+        // w |a - b|, not |w a - w b|: a contracted w a - w b is the rounding error of w b, not 0, when a == b
+        if (mode == 0) acc += (double)(alpha * (wt * fabsf(lp - lt)) + wt * fabsf(Sp - St));
         else acc += (double)((lp - lt) * (lp - lt));
     }
     acc = warp_sum(acc);
@@ -158,8 +165,8 @@ k_mss_bwd_frames(const float* __restrict__ xp, const float* __restrict__ xt, int
     Cplx* z = s + n;
     const int fr = blockIdx.x, b = blockIdx.y, bins = n / 2 + 1;
     load_twiddles(tw, n);
-    load_frame(s, xp + (size_t)b * T, xt + (size_t)b * T, T, n, logn, fr, hop);
-    __syncthreads();
+    // equal frames: B = A, as in k_mss_fwd
+    const bool same = __syncthreads_and(load_frame(s, xp + (size_t)b * T, xt + (size_t)b * T, T, n, logn, fr, hop));
     fft_smem(s, tw, n, logn, false);
     const float wt = time_weight(fr, frames);
     // rmse: d sqrt(m) = d m / (2 sqrt(m)), m = scale * sum
@@ -171,11 +178,12 @@ k_mss_bwd_frames(const float* __restrict__ xp, const float* __restrict__ xt, int
         if (f < bins && !(mode == 0 && f == 0)) {
             Cplx A, B;
             unpack2(s, n, f, A, B);
+            if (same) B = A;
             const float Sp = A.re * A.re + A.im * A.im, St = B.re * B.re + B.im * B.im;
             const float lp = log2f(Sp + eps), lt = log2f(St + eps);
             float g;        // d loss / d S_p[f]
             if (mode == 0) {
-                const float dl = wt * lp - wt * lt, ds_ = wt * Sp - wt * St;
+                const float dl = lp - lt, ds_ = Sp - St;         // the signs of w (a - b): w >= 0
                 const float sl = dl > 0.f ? 1.f : (dl < 0.f ? -1.f : 0.f), ss = ds_ > 0.f ? 1.f : (ds_ < 0.f ? -1.f : 0.f);
                 g = gscale * wt * (alpha * sl * inv_ln2 / (Sp + eps) + ss);
             } else {

@@ -147,7 +147,8 @@ def test_synth_forward_vs_closed_form(B, k, T, sr):
 
 
 @pytest.mark.parametrize("B,k,T,sr", [(2, 16, 4000, 32000), (5, 40, 9000, 44100), (66, 33, 700, 44100), (1, 1, 2, 44100),
-                                       (130, 131, 259, 44100), (3, 300, 4100, 44100)])
+                                       (130, 131, 259, 44100), (3, 300, 4100, 44100),
+                                       (2, 64, 88200, 44100)])   # 37 time chunks in k_synth_bwd_amp
 def test_synth_backward_vs_autograd(B, k, T, sr):
     from diffsound_b200 import native
     d, fd = _rand_modes(k, seed=3)
@@ -181,7 +182,8 @@ def test_synth_vs_reference_golden():
     assert np.linalg.norm(y - ref) / np.linalg.norm(ref) <= 1e-4
 
 
-@pytest.mark.parametrize("B,T,F", [(1, 8000, 150), (3, 1000, 1), (2, 5000, 1024), (5, 1025, 7), (2, 300, 600)])
+@pytest.mark.parametrize("B,T,F", [(1, 8000, 150), (3, 1000, 1), (2, 5000, 1024), (5, 1025, 7), (2, 300, 600),
+                                   (2, 1500, 2048)])   # F = FIR_MAXF (two FIR_TILE), T < F
 def test_force_fir_matches_reference_conv1d(B, T, F):
     """ds_force_fir against the reference's own expression, F.conv1d(signal, flipped force, groups, padding=F-1)[:, :T]
     (oscillator.py:305-309), forward and backward w.r.t. the signal."""
